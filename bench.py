@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the SS2D selective-scan hot path on B200 (contract: task statement ④).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -35,6 +35,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: importing its modules must not write __pycache__ into it
 
 import torch  # noqa: E402
 
@@ -142,6 +143,35 @@ def build_inputs(calls, device, on_device=False):
     return sets
 
 
+GRAD_NAMES = ("du", "ddelta", "dA", "dB", "dC", "dD", "ddelta_bias")
+DUMP_BUDGET_BYTES = 60_000_000      # under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, kept):
+    """Writes what fwd / bwd returned for each input set as <out_dir>/<name>.npy in float32: out, the final state
+    (x[:, :, -1, 1::2]) and the seven gradients, prefixed `call<i>_` when the step has several input sets. An array larger
+    than its equal share of the budget is replaced by a fixed sample of its flattened elements: the first `share` indices
+    of a permutation drawn from a CPU generator seeded 0, in ascending order, so that two builds run with the same
+    arguments can be compared element by element."""
+    import numpy as np
+    arrays = {}
+    for i, (out, x, grads) in enumerate(kept):
+        named = {"out": out, "last_state": x[:, :, -1, 1::2], **dict(zip(GRAD_NAMES, grads))}
+        prefix = f"call{i}_" if len(kept) > 1 else ""
+        arrays.update({prefix + k: v for k, v in named.items() if v is not None})
+    share = DUMP_BUDGET_BYTES // 4 // len(arrays)
+    os.makedirs(out_dir, exist_ok=True)
+    samples = {}
+    for name, v in arrays.items():
+        v = v.detach()
+        if v.numel() > share:
+            if v.numel() not in samples:
+                gen = torch.Generator().manual_seed(0)
+                samples[v.numel()] = torch.randperm(v.numel(), generator=gen)[:share].sort().values.to(v.device)
+            v = v.reshape(-1)[samples[v.numel()]]
+        np.save(os.path.join(out_dir, name + ".npy"), v.float().cpu().numpy())
+
+
 def run_ours(args, rank, world, local_rank):
     import ceigm_unet_b200 as pkg
     from ceigm_unet_b200 import dist as D
@@ -156,7 +186,9 @@ def run_ours(args, rank, world, local_rank):
     dev_sets = [(c, {k: v.to(device) for k, v in inp.items()}) for c, inp in host_sets]
     resident = sum(v.numel() * 4 for _, inp in dev_sets for v in inp.values())
 
-    def step(record=None):
+    def step(record=None, keep=False):
+        """One step; with keep=True returns (out, x, grads) of the last call of every input set."""
+        kept = []
         for count, t in dev_sets:
             for _ in range(count):
                 if record is not None:
@@ -164,9 +196,12 @@ def run_ours(args, rank, world, local_rank):
                 out, x = core.fwd(t["u"], t["delta"], t["A"], t["B"], t["C"], t["D"], t["delta_bias"], True, 1)
                 if record is not None:
                     record[1].record()
-                core.bwd(t["u"], t["delta"], t["A"], t["B"], t["C"], t["D"], t["delta_bias"], t["dout"], x, True, 1)
+                grads = core.bwd(t["u"], t["delta"], t["A"], t["B"], t["C"], t["D"], t["delta_bias"], t["dout"], x, True, 1)
                 if record is not None:
                     record[2].record()
+            if keep:
+                kept.append((out, x, grads))
+        return kept
 
     def barrier():
         if world > 1:
@@ -187,10 +222,13 @@ def run_ours(args, rank, world, local_rank):
     wall0 = time.time()
     e0.record()
     for i in range(args.steps):
-        step(evs[i] if evs else None)
+        last = step(evs[i] if evs else None, keep=args.dump_outputs is not None and i == args.steps - 1)
     e1.record()
     barrier()
     clocks = sampler.stop(wall0, time.time())
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     launches = pkg.launch_count()
     ms = D.max_over_ranks(e0.elapsed_time(e1), device)      # slowest rank's device time
     ms_per_step = ms / args.steps
@@ -649,7 +687,14 @@ def main():
     ap.add_argument("--e2e-streams", type=int, default=4)
     ap.add_argument("--no-extras", action="store_true", help="skip the other_workloads context block")
     ap.add_argument("--no-model", action="store_true", help="skip the model-level (GM-UNet train / inference) block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what fwd / bwd returned in the last timed step as DIR/<name>.npy (float32, at most 64 MB in "
+                         "all: larger arrays are replaced by a fixed seeded sample of their elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs dumps the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -107,10 +107,11 @@ def test_constructors_reproduce_reference_init_bit_exactly():
 
 
 def test_reference_python_picks_up_the_dropin_modules():
-    """With install_dropin(), the UNMODIFIED reference csms6s.py (build container only) binds our extension modules."""
-    ref = "/root/reference/gm-unet/model/gm/csms6s.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present (GPU box)")
+    """With install_dropin(), the UNMODIFIED reference csms6s.py (harness/install_ref.py) binds our extension modules."""
+    from harness import refmodel
+    if not refmodel.available():
+        pytest.skip("reference tree not installed (harness/install_ref.py)")
+    ref = os.path.join(refmodel.ref_root(), "model", "gm", "csms6s.py")
     import importlib.util
     import sys
     import warnings
