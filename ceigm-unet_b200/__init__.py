@@ -27,7 +27,9 @@ def graphed(module, sample_args, num_warmup_iters: int = 3):
     `sample_args`: a tuple of tensors with the shapes / dtypes / requires_grad flags of the real inputs.
     Capture BEFORE the module's first eager backward: autograd pins every parameter's gradient accumulator to the stream
     of its first use, and an accumulator created on the legacy default stream cannot be joined from a capturing stream
-    (cudaErrorStreamCaptureImplicit)."""
+    (cudaErrorStreamCaptureImplicit).
+    torch.use_deterministic_algorithms() is read when the graph is captured: the captured backward keeps the scan kernels
+    (atomic or deterministic) of that moment, whatever the switch says at replay."""
     import torch
     if not torch.cuda.is_available():
         raise RuntimeError("graphed() needs a CUDA device: there is no CPU fallback")

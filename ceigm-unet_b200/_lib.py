@@ -41,7 +41,7 @@ class ScanDesc(ctypes.Structure):
         ("B_batch_stride", ctypes.c_int64), ("B_group_stride", ctypes.c_int64), ("B_state_stride", ctypes.c_int64),
         ("C_batch_stride", ctypes.c_int64), ("C_group_stride", ctypes.c_int64), ("C_state_stride", ctypes.c_int64),
         ("u_dim_modulo", ctypes.c_int32), ("last_state_interleaved", ctypes.c_int32),
-        ("grads_prezeroed", ctypes.c_int32),
+        ("grads_prezeroed", ctypes.c_int32), ("deterministic", ctypes.c_int32),
     ]
 
 

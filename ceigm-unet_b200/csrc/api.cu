@@ -1,6 +1,7 @@
 // C ABI of libss2d_b200.so: argument validation, parameter packing, variant dispatch. No torch, no allocation.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
 
 #include <cstdio>
@@ -20,13 +21,20 @@ cudaError_t dwnhwc_stencil_launch(const void* x, const void* aux, void* y, const
 int dwnhwc_wgrad_slabs(int B, int H, int W, int nc);
 cudaError_t dwnhwc_wgrad_launch(const void* x, const void* g, int c0, int nc, int K, float* dW, float* db, int B, int H, int W,
                                 int C, int dt, float* part, cudaStream_t stream);
-cudaError_t scan_bwd_dispatch(const ScanParams& p, cudaStream_t stream);
+// backward launchers: *slabs receives the number of dB / dC partial slabs the launch wrote in deterministic mode (0 or 1:
+// dB / dC hold the result already)
+cudaError_t scan_bwd_dispatch(const ScanParams& p, cudaStream_t stream, int* slabs);
 cudaError_t scan_bwd_finalize(const ScanParams& p, float* dA, float* dD, float* dbias, cudaStream_t stream);
+cudaError_t scan_bwd_fold(const ScanParams& p, int slabs, cudaStream_t stream);
 cudaError_t scan_par_fwd_dispatch(const ScanParams& p, cudaStream_t stream);
-cudaError_t scan_par_bwd_dispatch(const ScanParams& p, cudaStream_t stream);
+cudaError_t scan_par_bwd_dispatch(const ScanParams& p, cudaStream_t stream, int* slabs);
 bool scan_n1_fwd_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err);
 bool scan_n1_bwd_try(const ScanParams& p, float* dA, float* dD, float* dbias, int grads_zeroed, cudaStream_t stream,
-                     cudaError_t* err);
+                     cudaError_t* err, int* slabs);
+// most partial slabs any backward kernel the dispatcher may pick for this pass writes in deterministic mode
+int scan_bwd_det_slabs(const ScanParams& p);
+int scan_n1_bwd_det_slabs(const ScanParams& p);
+int scan_par_bwd_det_slabs(const ScanParams& p);
 
 // d_state == 1 (the live GM-UNet regime) runs the parallel-along-L kernels (scan_par.cu)
 static bool use_par(const ScanParams& p) { return p.N == 1 && p.A_ld == 1; }
@@ -116,6 +124,7 @@ static int validate(const ss2d_scan_desc* d) {
     return SS2D_ERR_BAD_LAYOUT;
   }
   if (d->u_dim_modulo < 0) return SS2D_ERR_BAD_SHAPE;
+  if (d->deterministic != 0 && d->deterministic != 1) return SS2D_ERR_BAD_SHAPE;
   return SS2D_OK;
 }
 
@@ -135,6 +144,7 @@ static void pack(const ss2d_scan_desc* d, ScanParams& p) {
   p.out_bs = d->out_batch_stride; p.out_ds = d->out_dim_stride;
   p.B_bs = d->B_batch_stride; p.B_gs = d->B_group_stride; p.B_ns = d->B_state_stride;
   p.C_bs = d->C_batch_stride; p.C_gs = d->C_group_stride; p.C_ns = d->C_state_stride;
+  p.det = d->deterministic;
 }
 
 // TMA bulk copies need 16-byte aligned fp32 rows: every stride a multiple of 4 elements, bases 16-byte aligned
@@ -155,6 +165,30 @@ static size_t ckpt_floats_pass(const ss2d_scan_desc* d, int n) {
   return (size_t)d->batch * d->dim * nck * (size_t)n;
 }
 static size_t round4(size_t x) { return (x + 3) & ~(size_t)3; }
+
+// pass i of the backward: state count, kernel variant, whether later passes accumulate
+static void set_pass(ScanParams& p, const ss2d_scan_desc* d, int i) {
+  const int n0 = i * kStatesPerPass;
+  const int n = d->dstate - n0 < kStatesPerPass ? d->dstate - n0 : kStatesPerPass;
+  const Variant v = pick_variant(n);
+  p.N = n; p.NP = v.NS * v.R; p.accum = i > 0;
+}
+
+// Deterministic mode: one partial slab (batch, G, dstate, L) of dB and one of dC per extra CTA a group is split over, for the
+// widest split of any pass. The dispatcher launches with geometries derived from the same per-kernel functions.
+static int det_slabs(const ss2d_scan_desc* d) {
+  if (!d->deterministic) return 0;
+  ScanParams p;
+  pack(d, p);
+  int smax = 0;
+  for (int i = 0; i < n_passes(d->dstate); ++i) {
+    set_pass(p, d, i);
+    const int s = use_par(p) ? std::max(scan_n1_bwd_det_slabs(p), scan_par_bwd_det_slabs(p)) : scan_bwd_det_slabs(p);
+    smax = std::max(s, smax);
+  }
+  return smax;
+}
+static size_t slab_stride(const ss2d_scan_desc* d) { return round4((size_t)d->batch * d->n_groups * d->dstate * d->seqlen); }
 
 }  // namespace ss2d
 
@@ -177,6 +211,8 @@ size_t ss2d_scan_bwd_workspace_bytes(const ss2d_scan_desc* d, int have_ckpt) {
   const int nmax = d->dstate < kStatesPerPass ? d->dstate : kStatesPerPass;
   size_t floats = round4((size_t)d->batch * d->dim * (nmax + 2));
   if (!have_ckpt) floats += ss2d_scan_ckpt_floats(d);
+  const int slabs = det_slabs(d);
+  if (slabs > 1) floats += (size_t)2 * (slabs - 1) * slab_stride(d);
   return floats * sizeof(float);
 }
 
@@ -241,6 +277,8 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
   const int nmax = d->dstate < kStatesPerPass ? d->dstate : kStatesPerPass;
   float* part = ws;
   float* own_ckpt = ws + round4((size_t)d->batch * d->dim * (nmax + 2));
+  float* slab_base = own_ckpt + (ckpt ? 0 : ss2d_scan_ckpt_floats(d));
+  const int smax = det_slabs(d);
   if (!ckpt) {   // recompute the chunk states with a forward sweep that writes nothing else
     rc = ss2d_scan_fwd(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, nullptr, own_ckpt, nullptr, stream);
     if (rc != SS2D_OK) return rc;
@@ -252,29 +290,39 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
   p.tma_ok = tma_eligible(d, u, delta, Bmat, Cmat, dout) && d->out_dtype == SS2D_F32 && !(d->out_batch_stride & 3) &&
              !(d->out_dim_stride & 3);
   p.part = part;
+  p.slab_stride = (int64_t)slab_stride(d);
+  // dA / dD / d(delta_bias) accumulated in place only outside deterministic mode (the N = 1 kernels add per-row sums atomically)
+  const int zeroed = d->grads_prezeroed && !d->deterministic;
   size_t ck_off = 0;
   for (int i = 0; i < n_passes(d->dstate); ++i) {
     const int n0 = i * kStatesPerPass;
     const int n = d->dstate - n0 < kStatesPerPass ? d->dstate - n0 : kStatesPerPass;
-    const Variant v = pick_variant(n);
-    p.N = n; p.NP = v.NS * v.R; p.accum = i > 0;
+    set_pass(p, d, i);
     p.A = A + n0;
     p.Bm = static_cast<const char*>(Bmat) + (size_t)n0 * d->B_state_stride * esize(d->io_dtype);
     p.Cm = static_cast<const char*>(Cmat) + (size_t)n0 * d->C_state_stride * esize(d->io_dtype);
     p.ckpt_in = ckpt + ck_off;
     p.dB = dB + (size_t)n0 * d->seqlen;
     p.dC = dC + (size_t)n0 * d->seqlen;
+    p.slabB = slab_base + (size_t)n0 * d->seqlen;
+    p.slabC = slab_base + (size_t)(smax > 1 ? smax - 1 : 0) * p.slab_stride + (size_t)n0 * d->seqlen;
     ck_off += round4(ckpt_floats_pass(d, n));
     cudaError_t e;
     bool finalize = true;
+    int slabs = 0;
     if (use_par(p)) {
-      if (scan_n1_bwd_try(p, dA, dD, ddelta_bias, d->grads_prezeroed, st, &e)) finalize = !d->grads_prezeroed;
-      else e = scan_par_bwd_dispatch(p, st);
+      if (scan_n1_bwd_try(p, dA, dD, ddelta_bias, zeroed, st, &e, &slabs)) finalize = !zeroed;
+      else e = scan_par_bwd_dispatch(p, st, &slabs);
     } else {
-      e = scan_bwd_dispatch(p, st);
+      e = scan_bwd_dispatch(p, st, &slabs);
     }
     if (e != cudaSuccess) return cuda_fail(e);
     ++g_launches;
+    if (slabs > 1) {
+      e = scan_bwd_fold(p, slabs, st);
+      if (e != cudaSuccess) return cuda_fail(e);
+      ++g_launches;
+    }
     if (finalize) {
       e = scan_bwd_finalize(p, dA + n0, dD, ddelta_bias, st);
       if (e != cudaSuccess) return cuda_fail(e);
@@ -597,7 +645,7 @@ const char* ss2d_strerror(int status) {
 }
 
 const char* ss2d_last_cuda_error(void) { return g_cuda_err; }
-const char* ss2d_version(void) { return "ss2d_b200 0.1.0 sm_100a"; }
+const char* ss2d_version(void) { return "ss2d_b200 0.2.0 sm_100a"; }
 int64_t ss2d_launch_count(int reset) {
   return reset ? g_launches.exchange(0) : g_launches.load();
 }

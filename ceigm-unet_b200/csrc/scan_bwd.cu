@@ -15,8 +15,10 @@
 //     adjoint recurrence g_l = C_l dy_l + a_(l+1) g_(l+1). Nothing per-element is ever stored in HBM.
 //   * dB/dC partials are summed over the thread's rows in registers, over the warp's row lanes with a shuffle
 //     reduce-scatter, and over the CTA's warps by the producer: one vector reduction per (state, 4 positions) and
-//     CTA reaches global memory (plain stores when the CTA covers the whole group: deterministic).
+//     CTA reaches global memory (plain stores when the CTA covers the whole group: deterministic). In deterministic mode
+//     (DET) every CTA stores into its own partial slab and scan_bwd_fold_kernel sums the slabs in slab order.
 //   * dA, dD, d(delta_bias) leave through a per-batch partial buffer and a deterministic second pass.
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include <type_traits>
@@ -98,7 +100,7 @@ __device__ __forceinline__ void store_states(float* __restrict__ dst, const floa
   else dst[0] = src[0];
 }
 
-template <int NS, int R, int RPT>
+template <int NS, int R, int RPT, bool DET>
 __global__ void __launch_bounds__(kBwdThreads, RPT == 1 ? 4 : 3) scan_bwd_kernel(const ScanParams p, const __grid_constant__ TmaMaps maps) {
   using S = BwdShape<NS, R, RPT>;
   constexpr int CH = S::CH, NP = S::NP, NPB = S::NPB, RL = S::RL, RPW = S::RPW, CNT = S::CNT, NW = kBwdConsumerWarps;
@@ -163,7 +165,7 @@ __global__ void __launch_bounds__(kBwdThreads, RPT == 1 ? 4 : 3) scan_bwd_kernel
       tma_prefetch_desc(&maps.B); tma_prefetch_desc(&maps.C);
     }
     const int urow0 = p.u_mod > 0 ? d0 % p.u_mod : d0;
-    const bool single_cta_group = gridDim.x == 1;
+    const bool single_cta_group = DET || gridDim.x == 1;
     // fold the NW per-warp slabs of half tile `hc` (processing order) and send the sums to dB / dC
     auto flush_half = [&](int hc) {
       const int buf = hc & 1;
@@ -183,7 +185,7 @@ __global__ void __launch_bounds__(kBwdThreads, RPT == 1 ? 4 : 3) scan_bwd_kernel
         }
         const int l = l_base + c;
         if (n < p.N && l < L) {
-          float* dst = (which == 0 ? p.dB : p.dC) + ((int64_t)(b * p.G + g) * p.A_ld + n) * L;
+          float* dst = (DET ? det_slab(p, which, blockIdx.x) : (which == 0 ? p.dB : p.dC)) + ((int64_t)(b * p.G + g) * p.A_ld + n) * L;
           if (so.dir <= 1 && l + 3 < L && (L & 3) == 0) {
             float4* q4 = reinterpret_cast<float4*>(dst + l);
             if (single_cta_group) *q4 = acc;
@@ -534,10 +536,38 @@ __global__ void scan_bwd_finalize_kernel(const float* __restrict__ part, float* 
   else if (dbias) dbias[d] = accum ? dbias[d] + acc : acc;
 }
 
-template <int NS, int R, int RPT>
+// Deterministic mode: dB / dC (slab 0) += slabs 1 ... slabs - 1, in slab order, over this pass' states [n0, n0 + N) of every
+// (batch, group): rows of N * L floats, A_ld * L apart. HBM-bound; 128-bit accesses when L % 4 == 0.
+template <bool VEC>
+__global__ void __launch_bounds__(256) scan_bwd_fold_kernel(const ScanParams p, int slabs) {
+  constexpr int V = VEC ? 4 : 1;
+  const int which = blockIdx.y;
+  float* __restrict__ out = which ? p.dC : p.dB;
+  const float* __restrict__ src = which ? p.slabC : p.slabB;
+  const int64_t row = (int64_t)p.N * p.L, pitch = (int64_t)p.A_ld * p.L, total = (int64_t)p.batch * p.G * row;
+  for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * V; i < total; i += (int64_t)gridDim.x * blockDim.x * V) {
+    const int64_t o = i / row, off = o * pitch + (i - o * row);
+    if constexpr (VEC) {
+      float4 acc = *reinterpret_cast<const float4*>(out + off);
+#pragma unroll 4
+      for (int s = 1; s < slabs; ++s) {
+        const float4 v = __ldg(reinterpret_cast<const float4*>(src + (int64_t)(s - 1) * p.slab_stride + off));
+        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+      }
+      *reinterpret_cast<float4*>(out + off) = acc;
+    } else {
+      float acc = out[off];
+#pragma unroll 4
+      for (int s = 1; s < slabs; ++s) acc += __ldg(src + (int64_t)(s - 1) * p.slab_stride + off);
+      out[off] = acc;
+    }
+  }
+}
+
+template <int NS, int R, int RPT, bool DET>
 static cudaError_t launch_bwd(ScanParams p, cudaStream_t stream) {
   using S = BwdShape<NS, R, RPT>;
-  auto kern = scan_bwd_kernel<NS, R, RPT>;
+  auto kern = scan_bwd_kernel<NS, R, RPT, DET>;
   static PerDeviceOnce once;
   cudaError_t ea = func_attr_once(once, reinterpret_cast<const void*>(kern), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::smem_bytes);
   if (ea != cudaSuccess) return ea;
@@ -550,26 +580,65 @@ static cudaError_t launch_bwd(ScanParams p, cudaStream_t stream) {
   return cudaGetLastError();
 }
 
-bool scan_bwd2_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err);   // scan_bwd2.cu
+bool scan_bwd2_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err, int* slabs);   // scan_bwd2.cu
+int scan_bwd2_det_slabs(const ScanParams& p);
 
-cudaError_t scan_bwd_dispatch(const ScanParams& p, cudaStream_t stream) {
-  cudaError_t e2;
-  if (scan_bwd2_try(p, stream, &e2)) return e2;     // fast path: fp32 + TMA, 8 < N <= 16, contiguous traversal
+// kernel variant of this pass (0 ... 6), shared by the launcher and the slab count of deterministic mode
+static int bwd_variant(const ScanParams& p) {
   const int N = p.N;
-  if (N <= 1) return launch_bwd<1, 1, 1>(p, stream);
-  if (N <= 2) return launch_bwd<2, 1, 1>(p, stream);
-  if (N <= 4) return launch_bwd<2, 2, 1>(p, stream);
-  if (N <= 8) return launch_bwd<2, 4, 2>(p, stream);
+  if (N <= 1) return 0;
+  if (N <= 2) return 1;
+  if (N <= 4) return 2;
+  if (N <= 8) return 3;
   if (N <= 16) {
     // Two rows per thread amortise the B/C loads and the dB/dC row reduction (best on big grids); one row per thread
     // needs fewer registers / shared memory (4 CTAs per SM instead of 3) and halves the CTA size, which wins when the
     // two-row grid would not fill ~2.5 waves (measured on vm_d96 / vm_d192 / vm_d384, B200).
     const int sms = sm_count_current_device();
     const long ctas2 = (long)((p.dpg + 31) / 32) * p.G * p.batch;
-    const int rpt = ctas2 * 2 < 5L * 3 * sms ? 1 : 2;
-    return rpt == 1 ? launch_bwd<2, 8, 1>(p, stream) : launch_bwd<2, 8, 2>(p, stream);
+    return ctas2 * 2 < 5L * 3 * sms ? 4 : 5;
   }
-  return launch_bwd<4, 8, 1>(p, stream);
+  return 6;
+}
+static int bwd_rows_per_cta(int v) {
+  constexpr int ch[7] = {BwdShape<1, 1, 1>::CH, BwdShape<2, 1, 1>::CH, BwdShape<2, 2, 1>::CH, BwdShape<2, 4, 2>::CH,
+                         BwdShape<2, 8, 1>::CH, BwdShape<2, 8, 2>::CH, BwdShape<4, 8, 1>::CH};
+  return ch[v];
+}
+template <bool DET>
+static cudaError_t launch_variant(int v, const ScanParams& p, cudaStream_t stream) {
+  switch (v) {
+    case 0: return launch_bwd<1, 1, 1, DET>(p, stream);
+    case 1: return launch_bwd<2, 1, 1, DET>(p, stream);
+    case 2: return launch_bwd<2, 2, 1, DET>(p, stream);
+    case 3: return launch_bwd<2, 4, 2, DET>(p, stream);
+    case 4: return launch_bwd<2, 8, 1, DET>(p, stream);
+    case 5: return launch_bwd<2, 8, 2, DET>(p, stream);
+    default: return launch_bwd<4, 8, 1, DET>(p, stream);
+  }
+}
+
+int scan_bwd_det_slabs(const ScanParams& p) {
+  const int ch = bwd_rows_per_cta(bwd_variant(p));
+  return std::max(scan_bwd2_det_slabs(p), (p.dpg + ch - 1) / ch);
+}
+
+cudaError_t scan_bwd_dispatch(const ScanParams& p, cudaStream_t stream, int* slabs) {
+  cudaError_t e2;
+  if (scan_bwd2_try(p, stream, &e2, slabs)) return e2;     // fast path: fp32 + TMA, 8 < N <= 16, contiguous traversal
+  const int v = bwd_variant(p), ch = bwd_rows_per_cta(v);
+  *slabs = p.det ? (p.dpg + ch - 1) / ch : 0;              // = gridDim.x of launch_bwd
+  return p.det ? launch_variant<true>(v, p, stream) : launch_variant<false>(v, p, stream);
+}
+
+cudaError_t scan_bwd_fold(const ScanParams& p, int slabs, cudaStream_t stream) {
+  const bool vec = (p.L & 3) == 0;
+  const int64_t units = (int64_t)p.batch * p.G * p.N * p.L / (vec ? 4 : 1);
+  const int64_t want = (units + 255) / 256, cap = 8L * sm_count_current_device();
+  const dim3 grid((unsigned)(want < cap ? want : cap), 2);
+  if (vec) scan_bwd_fold_kernel<true><<<grid, 256, 0, stream>>>(p, slabs);
+  else scan_bwd_fold_kernel<false><<<grid, 256, 0, stream>>>(p, slabs);
+  return cudaGetLastError();
 }
 
 cudaError_t scan_bwd_finalize(const ScanParams& p, float* dA, float* dD, float* dbias, cudaStream_t stream) {

@@ -17,6 +17,8 @@
 //     straight from registers: each warp adds the totals of its 8 rows to dB / dC in L2. (A first version folded the
 //     four warps' totals through shared-memory slabs with an mbarrier hand-off per group to issue a quarter of the
 //     reductions; the hand-off coupled the warps and cost 10 % of the kernel, the extra L2 reductions cost nothing.)
+//     Deterministic mode (DET) keeps the warps uncoupled: each warp stores its totals into its own partial slab (index =
+//     the warp's position along the group), and scan_bwd_fold_kernel sums the slabs in slab order.
 #include <cstdlib>
 #include <cstring>
 #include <type_traits>
@@ -119,7 +121,7 @@ struct B2ReduceScatter {
   }
 };
 
-template <bool SOFTPLUS>
+template <bool SOFTPLUS, bool DET>
 __global__ void __launch_bounds__(B2_NW * 32, 4) scan_bwd2_kernel(const ScanParams p, const __grid_constant__ Bwd2Maps maps) {
   extern __shared__ __align__(16) unsigned char smem_rawb2[];
   unsigned char* smem = smem_rawb2 + ((1024 - (smem_u32(smem_rawb2) & 1023)) & 1023);
@@ -215,8 +217,11 @@ __global__ void __launch_bounds__(B2_NW * 32, 4) scan_bwd2_kernel(const ScanPara
   // dB / dC destination of this lane after the sum over the row-pair lanes: state n_0 = q + 8 sw, both tensors,
   // positions 2 (rp & 1), + 1 of every group. Lanes of padded states (n_0 >= N: B = C = 0 there, zero-filled by TMA, so
   // their totals are exactly 0) add their zeros to the last real state instead of being predicated off.
-  float* const red_B = p.dB + ((int64_t)(b * p.G + g) * p.A_ld + min(q + 8 * sw, p.N - 1)) * L;
-  const int64_t red_CmB = p.dC - p.dB;
+  // DET: slab wslab instead, and the padded-state lanes store nothing (a store of their zeros would overwrite state N - 1)
+  const int wslab = blockIdx.x * B2_NW + warp;
+  float* const red_B = (DET ? det_slab(p, 0, wslab) : p.dB) + ((int64_t)(b * p.G + g) * p.A_ld + min(q + 8 * sw, p.N - 1)) * L;
+  const int64_t red_CmB = DET ? det_slab(p, 1, wslab) - det_slab(p, 0, wslab) : p.dC - p.dB;
+  const bool red_lane = !DET || q + 8 * sw < p.N;
 
   auto load_ckpt = [&](int t, float2* h) {     // state before tile t = checkpoint at the end of tile t - 1
 #pragma unroll
@@ -401,10 +406,15 @@ __global__ void __launch_bounds__(B2_NW * 32, 4) scan_bwd2_kernel(const ScanPara
         }
         // this warp's totals go straight to global memory: two red.global.add.v2.f32 per lane (the branch is warp-uniform:
         // idle warps, and the groups past the end of the sequence in its last tile)
-        if (rows_valid > 0 && 4 * gi < len) {
+        if (rows_valid > 0 && 4 * gi < len && red_lane) {
           float* const dst = red_t + (REVV ? -4 * gi : 4 * gi);
-          red_add2(dst, REVV ? oB.y : oB.x, REVV ? oB.x : oB.y);
-          red_add2(dst + red_CmB, REVV ? oC.y : oC.x, REVV ? oC.x : oC.y);
+          if constexpr (DET) {
+            *reinterpret_cast<float2*>(dst) = make_float2(REVV ? oB.y : oB.x, REVV ? oB.x : oB.y);
+            *reinterpret_cast<float2*>(dst + red_CmB) = make_float2(REVV ? oC.y : oC.x, REVV ? oC.x : oC.y);
+          } else {
+            red_add2(dst, REVV ? oB.y : oB.x, REVV ? oB.x : oB.y);
+            red_add2(dst + red_CmB, REVV ? oC.y : oC.x, REVV ? oC.x : oC.y);
+          }
         }
         // ---- sum over the 8 state lanes on row-packed pairs: positions first (lane bits 0, 1), the row parity last; lane q ends
         //      up with (sB, sA) of row parity q >> 2, position q & 3 ----
@@ -508,31 +518,43 @@ static bool bwd2_maps(const ScanParams& p, Bwd2Maps* m) {
          make_tmap(&m->C, p.Cm, 4, d4, s4C, 16);
 }
 
-// Returns true when the fast path took the call (*err holds the launch status).
-bool scan_bwd2_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err) {
-  if (!p.tma_ok || p.N <= 8 || p.N > 16 || p.accum || p.io_dtype != SS2D_F32 || p.out_dtype != SS2D_F32) return false;
+// the conditions of the fast path that the descriptor alone decides (the rest are pointer alignments)
+static bool bwd2_shape_ok(const ScanParams& p) {
+  if (p.N <= 8 || p.N > 16 || p.accum || p.io_dtype != SS2D_F32 || p.out_dtype != SS2D_F32) return false;
   if (p.u_mod > 0 && p.u_mod % p.dpg != 0) return false;
-  if ((reinterpret_cast<uintptr_t>(p.du) & 15) || (reinterpret_cast<uintptr_t>(p.ddelta) & 15) ||
-      (reinterpret_cast<uintptr_t>(p.dB) & 15) || (reinterpret_cast<uintptr_t>(p.dC) & 15))
-    return false;
   for (int g = 0; g < p.G; ++g) {
     const int dir = p.layout == SS2D_LAYOUT_NATURAL ? p.dirs[g] : 0;
     if (dir == 2 || dir == 4) return false;
   }
+  return true;
+}
+
+// deterministic mode: one slab per warp that owns rows (warp index along the group)
+int scan_bwd2_det_slabs(const ScanParams& p) { return bwd2_shape_ok(p) ? (p.dpg + B2_RPW - 1) / B2_RPW : 0; }
+
+template <bool DET>
+static cudaError_t bwd2_launch(const ScanParams& p, const Bwd2Maps& maps, cudaStream_t stream) {
+  static PerDeviceOnce once, once_nosp;
+  cudaError_t e = func_attr_once(once, reinterpret_cast<const void*>(scan_bwd2_kernel<true, DET>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B2_SMEM);
+  if (e == cudaSuccess)
+    e = func_attr_once(once_nosp, reinterpret_cast<const void*>(scan_bwd2_kernel<false, DET>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B2_SMEM);
+  if (e != cudaSuccess) return e;
+  dim3 grid((p.dpg + B2_CH - 1) / B2_CH, p.G, p.batch);
+  if (p.softplus) scan_bwd2_kernel<true, DET><<<grid, B2_NW * 32, B2_SMEM, stream>>>(p, maps);
+  else scan_bwd2_kernel<false, DET><<<grid, B2_NW * 32, B2_SMEM, stream>>>(p, maps);
+  return cudaGetLastError();
+}
+
+// Returns true when the fast path took the call (*err holds the launch status).
+bool scan_bwd2_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err, int* slabs) {
+  if (!p.tma_ok || !bwd2_shape_ok(p)) return false;
+  if ((reinterpret_cast<uintptr_t>(p.du) & 15) || (reinterpret_cast<uintptr_t>(p.ddelta) & 15) ||
+      (reinterpret_cast<uintptr_t>(p.dB) & 15) || (reinterpret_cast<uintptr_t>(p.dC) & 15))
+    return false;
   Bwd2Maps maps;
   if (!bwd2_maps(p, &maps)) return false;
-
-  static PerDeviceOnce once, once_nosp;
-  {
-    cudaError_t e = func_attr_once(once, reinterpret_cast<const void*>(scan_bwd2_kernel<true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B2_SMEM);
-    if (e == cudaSuccess)
-      e = func_attr_once(once_nosp, reinterpret_cast<const void*>(scan_bwd2_kernel<false>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B2_SMEM);
-    if (e != cudaSuccess) { *err = e; return true; }
-  }
-  dim3 grid((p.dpg + B2_CH - 1) / B2_CH, p.G, p.batch);
-  if (p.softplus) scan_bwd2_kernel<true><<<grid, B2_NW * 32, B2_SMEM, stream>>>(p, maps);
-  else scan_bwd2_kernel<false><<<grid, B2_NW * 32, B2_SMEM, stream>>>(p, maps);
-  *err = cudaGetLastError();
+  *slabs = p.det ? scan_bwd2_det_slabs(p) : 0;
+  *err = p.det ? bwd2_launch<true>(p, maps, stream) : bwd2_launch<false>(p, maps, stream);
   return true;
 }
 

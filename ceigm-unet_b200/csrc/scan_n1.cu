@@ -16,11 +16,17 @@
 //   * out-of-range positions are loaded as delta = -inf: softplus gives exactly 0 there, the state freezes, and no
 //     per-position bound check is left in the arithmetic.
 //   * backward (`scan_n1_bwd_rows_kernel`): a CTA walks SEVERAL rows of its group one after the other and keeps dB / dC in
-//     registers across them — the sum over the rows of a group costs nothing and is stored once (deterministic, no atomics
-//     when one CTA covers the group). The next row's delta / u / dout are in flight meanwhile: one elected thread per row
-//     lane streams them through a 2-stage shared-memory ring with 1-D TMA bulk copies (cp.async.bulk + mbarrier); row lanes
-//     synchronise on their own named barriers, so they drift apart and overlap. dA / dD / d(delta_bias) go into
-//     caller-zeroed accumulators (`grads_prezeroed`): the call is memset + ONE kernel (scan_par: memset, kernel, finalize).
+//     registers across them — the sum over the rows of a group costs nothing and is stored once (plain stores when one CTA
+//     covers the group, red.global when several share it). The next row's delta / u / dout are in flight meanwhile: one
+//     elected thread per row lane streams them through a 2-stage shared-memory ring with 1-D TMA bulk copies
+//     (cp.async.bulk + mbarrier); row lanes synchronise on their own named barriers, so they drift apart and overlap.
+//     dA / dD / d(delta_bias) go into caller-zeroed accumulators with atomics (`grads_prezeroed`): the call is memset + ONE
+//     kernel (scan_par: memset, kernel, finalize). Neither sum is reproducible bit for bit from call to call.
+//   * deterministic mode (DET; ss2d_scan_desc.deterministic): every CTA stores dB / dC into its own partial slab (summed in
+//     slab order by scan_bwd_fold_kernel) and the per-row sums of dA / dD / d(delta_bias) go to the partial buffer of the
+//     fixed-order finalize pass; rows walked in several chunks keep their running sums in shared memory.
+#include <algorithm>
+
 #include "common.cuh"
 #include "host_util.h"
 #include "scan_params.h"
@@ -323,7 +329,7 @@ __device__ __forceinline__ void n1_emit_row_grads(const ScanParams& p, int b, in
 // Any L (rows longer than 16 warps x 256 positions are walked in chunks, last to first, from the forward's checkpoints), any
 // alignment. grads_zeroed != 0: dA / dD / d(delta_bias) are caller-zeroed accumulators; else per-(batch, channel) partials
 // go to p.part and scan_bwd_finalize sums them.
-template <bool VEC, bool SP>
+template <bool VEC, bool SP, bool DET>
 __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_kernel(const ScanParams p, const N1Geom gm, float* __restrict__ dA,
                                                                       float* __restrict__ dD, float* __restrict__ dbias,
                                                                       int grads_zeroed) {
@@ -337,7 +343,7 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_kernel(const Sc
   const bool valid = q.r < gm.rt && row < p.dpg;
   const int d = g * p.dpg + (valid ? row : 0);
   const int L = valid ? p.L : 0;
-  const bool plain = gridDim.x == 1;
+  const bool plain = DET || gridDim.x == 1;
   const float A1 = p.A[d];
   const float bias = p.bias ? p.bias[d] : 0.f;
   const float Dd = p.Dv ? p.Dv[d] : 0.f;
@@ -349,8 +355,8 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_kernel(const Sc
   const float* fC = static_cast<const float*>(p.Cm) + (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
   float* fdu = static_cast<float*>(p.du) + (p.u_mod > 0 ? ((int64_t)b * p.dim + d) * (int64_t)p.L : (int64_t)b * p.u_bs + (int64_t)d * p.u_ds);
   float* fdd = static_cast<float*>(p.ddelta) + (int64_t)b * p.dl_bs + (int64_t)d * p.dl_ds;
-  float* dBrow = p.dB + (int64_t)(b * p.G + g) * p.L;
-  float* dCrow = p.dC + (int64_t)(b * p.G + g) * p.L;
+  float* dBrow = (DET ? det_slab(p, 0, blockIdx.x) : p.dB) + (int64_t)(b * p.G + g) * p.L;
+  float* dCrow = (DET ? det_slab(p, 1, blockIdx.x) : p.dC) + (int64_t)(b * p.G + g) * p.L;
   const float dfill = SP ? -INFINITY : 0.f;
 
   auto body = [&](auto REVT) {
@@ -409,7 +415,7 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_kernel(const Sc
       }
     }
     n1_row_sum3(accA, accD, accb, lane, q, gm, s_red + q.r * gm.wpr, 1 + q.r);
-    if (q.t == 0 && valid) n1_emit_row_grads(p, b, d, accA, accD, accb, dA, dD, dbias, grads_zeroed);
+    if (q.t == 0 && valid) n1_emit_row_grads(p, b, d, accA, accD, accb, dA, dD, dbias, !DET && grads_zeroed);
   };
   if (p.layout == SS2D_LAYOUT_NATURAL && p.dirs[g] == 3) body(std::true_type{}); else body(std::false_type{});
 }
@@ -422,7 +428,7 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_kernel(const Sc
 // each chunk as the slab that sums dB / dC over the row lanes.
 constexpr int N1_MAX_RSEQ = 64;
 
-template <bool SP>
+template <bool SP, bool DET>
 __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_rows_kernel(const ScanParams p, const N1Geom gm, float* __restrict__ dA,
                                                                            float* __restrict__ dD, float* __restrict__ dbias,
                                                                            int grads_zeroed) {
@@ -431,6 +437,7 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_rows_kernel(con
   __shared__ float s_red[2][N1_MAX_WARPS][3];
   __shared__ float s_tc[N1_MAX_WARPS][N1_MAX_RSEQ];        // reverse carry of each row between chunks (multi-chunk rows)
   __shared__ __align__(8) uint64_t s_full[N1_MAX_WARPS][2];
+  __shared__ float s_racc[DET ? N1_MAX_RSEQ : 1][3];       // DET, multi-chunk rows (one row lane): per-row running sums
   N1Geom gq = gm;
   gq.seg = 32;                                             // compile-time constant for the shuffle scans below
   const N1Thread q = n1_thread(gq);
@@ -442,11 +449,11 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_rows_kernel(con
   const int row_base = blockIdx.x * rows_cta + q.r;
   // rows this lane walks: row_base + j rt for j < nj
   const int nj = row_base < p.dpg ? min(gm.rseq, (p.dpg - row_base + gm.rt - 1) / gm.rt) : 0;
-  const bool plain = gridDim.x == 1;
+  const bool plain = DET || gridDim.x == 1;
   const float* fB = static_cast<const float*>(p.Bm) + (int64_t)b * p.B_bs + (int64_t)g * p.B_gs;
   const float* fC = static_cast<const float*>(p.Cm) + (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
-  float* dBrow = p.dB + (int64_t)(b * p.G + g) * L;
-  float* dCrow = p.dC + (int64_t)(b * p.G + g) * L;
+  float* dBrow = (DET ? det_slab(p, 0, blockIdx.x) : p.dB) + (int64_t)(b * p.G + g) * L;
+  float* dCrow = (DET ? det_slab(p, 1, blockIdx.x) : p.dC) + (int64_t)(b * p.G + g) * L;
   float* ring = s_ring + (size_t)q.r * 6 * lr;
   const bool leader = q.t == 0;                            // issues this row lane's TMA copies
   const int total_it = nj * gm.nchunks;
@@ -543,13 +550,24 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_rows_kernel(con
           }
         }
         if (q.t == 0) {
-          if (grads_zeroed) {
+          if (!DET && grads_zeroed) {
             atomicAdd(dA + d, accA);
             if (dD) atomicAdd(dD + d, accD);
             if (dbias) atomicAdd(dbias + d, accb);
-          } else {                                         // single-chunk rows only (host side): partials for the finalize pass
-            float* dst = p.part + ((int64_t)b * p.dim + d) * 3;
-            dst[0] = accA; dst[1] = accD; dst[2] = accb;
+          } else {           // partials for the finalize pass (outside DET the host sends only single-chunk rows here)
+            bool last = true;
+            if constexpr (DET) {
+              if (gm.nchunks > 1) {                        // running sums over the chunks, added in chunk order
+                float* acc = s_racc[j];
+                if (ci > 0) { accA = acc[0] + accA; accD = acc[1] + accD; accb = acc[2] + accb; }
+                last = ci == gm.nchunks - 1;
+                if (!last) { acc[0] = accA; acc[1] = accD; acc[2] = accb; }
+              }
+            }
+            if (last) {
+              float* dst = p.part + ((int64_t)b * p.dim + d) * 3;
+              dst[0] = accA; dst[1] = accD; dst[2] = accb;
+            }
           }
         }
       }
@@ -684,7 +702,7 @@ static bool n1_rows_geometry(const ScanParams& p, int grads_zeroed, N1Geom* out,
     // long rows: one lane of 8 warps x 256 positions per chunk, 2 CTAs per SM. (Measured on the 512^2 batch-64 stage-1 shape:
     // backward 409 us this way, 475 us with 8 row lanes of 2 warps x 256 — the lanes then meet at a CTA-wide barrier for the
     // dB / dC slab after every chunk and B / C are fetched 4x as often.)
-    if (!grads_zeroed) return false;                         // per-chunk row sums are accumulated with atomics
+    if (!grads_zeroed && !p.det) return false;               // per-chunk row sums: atomics, or shared memory in DET mode
     gm.wpr = 8;
     rt = 1;
     lr = (size_t)gm.wpr * 32 * N1_P;
@@ -706,37 +724,69 @@ static bool n1_rows_geometry(const ScanParams& p, int grads_zeroed, N1Geom* out,
   return true;
 }
 
+static int n1_one_row_smem(const N1Geom& gm) { return gm.rt > 1 ? 2 * gm.rt * gm.lc * (int)sizeof(float) : 0; }
+
+// deterministic mode: one slab per CTA along the group, for whichever of the two kernels takes the call
+int scan_n1_bwd_det_slabs(const ScanParams& p) {
+  if (!n1_eligible(p, true)) return 0;
+  int slabs = 0;
+  N1Geom gr;
+  size_t smem_rows = 0;
+  if (n1_rows_geometry(p, 0, &gr, &smem_rows)) slabs = (p.dpg + gr.rt * gr.rseq - 1) / (gr.rt * gr.rseq);
+  const N1Geom gm = n1_geometry(p);
+  if (n1_one_row_smem(gm) <= 40 * 1024) slabs = std::max(slabs, (p.dpg + gm.rt - 1) / gm.rt);
+  return slabs;
+}
+
+template <bool DET>
+static cudaError_t n1_bwd_rows_launch(const ScanParams& p, const N1Geom& gr, size_t smem, float* dA, float* dD, float* dbias,
+                                      int grads_zeroed, cudaStream_t stream) {
+  const bool sp = p.softplus != 0;
+  static PerDeviceOnce once_sp, once_nosp;
+  cudaError_t e = sp ? func_attr_once(once_sp, reinterpret_cast<const void*>(scan_n1_bwd_rows_kernel<true, DET>),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024)
+                     : func_attr_once(once_nosp, reinterpret_cast<const void*>(scan_n1_bwd_rows_kernel<false, DET>),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024);
+  if (e != cudaSuccess) return e;
+  const int rows_cta = gr.rt * gr.rseq;
+  dim3 grid((p.dpg + rows_cta - 1) / rows_cta, p.G, p.batch);
+  const int nt = gr.rt * gr.wpr * 32;
+  if (sp) scan_n1_bwd_rows_kernel<true, DET><<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed);
+  else scan_n1_bwd_rows_kernel<false, DET><<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed);
+  return cudaGetLastError();
+}
+
+template <bool DET>
+static cudaError_t n1_bwd_launch(const ScanParams& p, const N1Geom& gm, bool vec, float* dA, float* dD, float* dbias,
+                                 int grads_zeroed, cudaStream_t stream) {
+  const bool sp = p.softplus != 0;
+  dim3 grid((p.dpg + gm.rt - 1) / gm.rt, p.G, p.batch);
+  const size_t smem = n1_one_row_smem(gm);
+  const int nt = n1_threads(gm);
+  if (vec && sp) scan_n1_bwd_kernel<true, true, DET><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
+  else if (vec) scan_n1_bwd_kernel<true, false, DET><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
+  else if (sp) scan_n1_bwd_kernel<false, true, DET><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
+  else scan_n1_bwd_kernel<false, false, DET><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
+  return cudaGetLastError();
+}
+
 bool scan_n1_bwd_try(const ScanParams& p, float* dA, float* dD, float* dbias, int grads_zeroed, cudaStream_t stream,
-                     cudaError_t* err) {
+                     cudaError_t* err, int* slabs) {
   if (!n1_eligible(p, true)) return false;
-  const bool vec = n1_vec(p, true), sp = p.softplus != 0;
+  const bool vec = n1_vec(p, true);
   N1Geom gr;
   size_t smem_rows = 0;
   if (vec && n1_rows_geometry(p, grads_zeroed, &gr, &smem_rows)) {
-    static PerDeviceOnce once_sp, once_nosp;
-    cudaError_t e = sp ? func_attr_once(once_sp, reinterpret_cast<const void*>(scan_n1_bwd_rows_kernel<true>),
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024)
-                       : func_attr_once(once_nosp, reinterpret_cast<const void*>(scan_n1_bwd_rows_kernel<false>),
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024);
-    if (e != cudaSuccess) { *err = e; return true; }
-    const int rows_cta = gr.rt * gr.rseq;
-    dim3 grid((p.dpg + rows_cta - 1) / rows_cta, p.G, p.batch);
-    const int nt = gr.rt * gr.wpr * 32;
-    if (sp) scan_n1_bwd_rows_kernel<true><<<grid, nt, smem_rows, stream>>>(p, gr, dA, dD, dbias, grads_zeroed);
-    else scan_n1_bwd_rows_kernel<false><<<grid, nt, smem_rows, stream>>>(p, gr, dA, dD, dbias, grads_zeroed);
-    *err = cudaGetLastError();
+    *slabs = p.det ? (p.dpg + gr.rt * gr.rseq - 1) / (gr.rt * gr.rseq) : 0;
+    *err = p.det ? n1_bwd_rows_launch<true>(p, gr, smem_rows, dA, dD, dbias, grads_zeroed, stream)
+                 : n1_bwd_rows_launch<false>(p, gr, smem_rows, dA, dD, dbias, grads_zeroed, stream);
     return true;
   }
   const N1Geom gm = n1_geometry(p);
-  dim3 grid((p.dpg + gm.rt - 1) / gm.rt, p.G, p.batch);
-  const size_t smem = gm.rt > 1 ? (size_t)2 * gm.rt * gm.lc * sizeof(float) : 0;
-  if (smem > 40 * 1024) return false;
-  const int nt = n1_threads(gm);
-  if (vec && sp) scan_n1_bwd_kernel<true, true><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
-  else if (vec) scan_n1_bwd_kernel<true, false><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
-  else if (sp) scan_n1_bwd_kernel<false, true><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
-  else scan_n1_bwd_kernel<false, false><<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
-  *err = cudaGetLastError();
+  if (n1_one_row_smem(gm) > 40 * 1024) return false;
+  *slabs = p.det ? (p.dpg + gm.rt - 1) / gm.rt : 0;
+  *err = p.det ? n1_bwd_launch<true>(p, gm, vec, dA, dD, dbias, grads_zeroed, stream)
+               : n1_bwd_launch<false>(p, gm, vec, dA, dD, dbias, grads_zeroed, stream);
   return true;
 }
 

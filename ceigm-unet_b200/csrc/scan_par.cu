@@ -229,7 +229,8 @@ __global__ void __launch_bounds__(kParThreads) scan_par_fwd_kernel(const ScanPar
 }
 
 // ------------------------------------------------------------------------------------------------- backward
-template <int T>
+// DET: dB / dC go to partial slab blockIdx.x with plain stores (summed in slab order by scan_bwd_fold_kernel)
+template <int T, bool DET>
 __global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_kernel(const ScanParams p) {
   using S = ParShape<T>;
   constexpr int P = 8, LC = T * P;
@@ -246,7 +247,7 @@ __global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_kernel(const Scan
   so.dir = p.layout == SS2D_LAYOUT_NATURAL ? p.dirs[g] : 0;
   so.H = p.H; so.W = p.W; so.L = L;
   const int l_end = valid ? L : 0;
-  const bool single_cta_group = gridDim.x == 1;
+  const bool single_cta_group = DET || gridDim.x == 1;
 
   const float A1 = valid ? p.A[(int64_t)d * p.A_ld] : 0.f;
   const float A2 = A1 * kLog2e;
@@ -259,8 +260,8 @@ __global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_kernel(const Scan
   const int64_t dy_ro = (int64_t)b * p.out_bs + (int64_t)u_ch * p.out_ds;
   const int64_t B_ro = (int64_t)b * p.B_bs + (int64_t)g * p.B_gs;
   const int64_t C_ro = (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
-  float* dBrow = p.dB + (int64_t)(b * p.G + g) * p.A_ld * L;
-  float* dCrow = p.dC + (int64_t)(b * p.G + g) * p.A_ld * L;
+  float* dBrow = (DET ? det_slab(p, 0, blockIdx.x) : p.dB) + (int64_t)(b * p.G + g) * p.A_ld * L;
+  float* dCrow = (DET ? det_slab(p, 1, blockIdx.x) : p.dC) + (int64_t)(b * p.G + g) * p.A_ld * L;
 
   const bool rev = so.reversed();
   const bool fast_io = valid && p.io_dtype == SS2D_F32 && p.out_dtype == SS2D_F32 && so.contiguous() && (L & 3) == 0 &&
@@ -418,26 +419,37 @@ __global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_kernel(const Scan
   }
 }
 
+// threads per row: the smallest power of two whose T*P positions cover the row, at most 128 (longer rows are chunked)
+static int pick_T(int L, int P) {
+  int T = 4;
+  while (T < 128 && T * P < L) T <<= 1;
+  return T;
+}
+
 template <int T>
 static cudaError_t launch_par_fwd(const ScanParams& p, cudaStream_t stream) {
   dim3 grid((p.dpg + ParShape<T>::RT - 1) / ParShape<T>::RT, p.G, p.batch);
   scan_par_fwd_kernel<T><<<grid, kParThreads, 0, stream>>>(p);
   return cudaGetLastError();
 }
-template <int T>
+template <int T, bool DET>
 static cudaError_t launch_par_bwd(const ScanParams& p, cudaStream_t stream) {
   dim3 grid((p.dpg + ParShape<T>::RT - 1) / ParShape<T>::RT, p.G, p.batch);
   static PerDeviceOnce once;   // 16.6 KB of static shared memory per CTA: ask for a carve-out that fits several CTAs per SM
-  func_attr_once(once, reinterpret_cast<const void*>(scan_par_bwd_kernel<T>), cudaFuncAttributePreferredSharedMemoryCarveout, 50);
-  scan_par_bwd_kernel<T><<<grid, kParThreads, 0, stream>>>(p);
+  func_attr_once(once, reinterpret_cast<const void*>(scan_par_bwd_kernel<T, DET>), cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+  scan_par_bwd_kernel<T, DET><<<grid, kParThreads, 0, stream>>>(p);
   return cudaGetLastError();
 }
-
-// threads per row: the smallest power of two whose T*P positions cover the row, at most 128 (longer rows are chunked)
-static int pick_T(int L, int P) {
-  int T = 4;
-  while (T < 128 && T * P < L) T <<= 1;
-  return T;
+template <bool DET>
+static cudaError_t par_bwd_launch(const ScanParams& p, cudaStream_t stream) {
+  switch (pick_T(p.L, 8)) {
+    case 4: return launch_par_bwd<4, DET>(p, stream);
+    case 8: return launch_par_bwd<8, DET>(p, stream);
+    case 16: return launch_par_bwd<16, DET>(p, stream);
+    case 32: return launch_par_bwd<32, DET>(p, stream);
+    case 64: return launch_par_bwd<64, DET>(p, stream);
+    default: return launch_par_bwd<128, DET>(p, stream);
+  }
 }
 
 cudaError_t scan_par_fwd_dispatch(const ScanParams& p, cudaStream_t stream) {
@@ -451,15 +463,15 @@ cudaError_t scan_par_fwd_dispatch(const ScanParams& p, cudaStream_t stream) {
   }
 }
 
-cudaError_t scan_par_bwd_dispatch(const ScanParams& p, cudaStream_t stream) {
-  switch (pick_T(p.L, 8)) {
-    case 4: return launch_par_bwd<4>(p, stream);
-    case 8: return launch_par_bwd<8>(p, stream);
-    case 16: return launch_par_bwd<16>(p, stream);
-    case 32: return launch_par_bwd<32>(p, stream);
-    case 64: return launch_par_bwd<64>(p, stream);
-    default: return launch_par_bwd<128>(p, stream);
-  }
+// deterministic mode: one slab per CTA along the group (= gridDim.x of launch_par_bwd)
+int scan_par_bwd_det_slabs(const ScanParams& p) {
+  const int rt = kParThreads / pick_T(p.L, 8);
+  return (p.dpg + rt - 1) / rt;
+}
+
+cudaError_t scan_par_bwd_dispatch(const ScanParams& p, cudaStream_t stream, int* slabs) {
+  *slabs = p.det ? scan_par_bwd_det_slabs(p) : 0;
+  return p.det ? par_bwd_launch<true>(p, stream) : par_bwd_launch<false>(p, stream);
 }
 
 }  // namespace ss2d

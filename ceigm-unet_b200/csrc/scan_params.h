@@ -38,7 +38,20 @@ struct ScanParams {
   float* dB;            // fp32 [batch][G][N][L], pre-zeroed, accumulated with red.global when a group spans several CTAs
   float* dC;
   float* part;          // workspace: [batch][dim][N + 2] per-batch partial sums of dA, dD, dbias
+  // deterministic backward: the CTAs (scan_bwd2: warps) that share a group store their dB / dC sums into partial slab s =
+  // their index along the group instead of reducing into dB / dC; slab 0 is dB / dC itself, slab s > 0 lives at
+  // slabB / slabC + (s - 1) * slab_stride (same indexing as dB / dC), and scan_bwd_fold sums the slabs in slab order
+  int det;
+  float* slabB;
+  float* slabC;
+  int64_t slab_stride;
 };
+
+// destination of partial slab s of dB (which 0) or dC (which 1)
+__host__ __device__ inline float* det_slab(const ScanParams& p, int which, int s) {
+  if (s == 0) return which ? p.dC : p.dB;
+  return (which ? p.slabC : p.slabB) + (int64_t)(s - 1) * p.slab_stride;
+}
 
 // Opaque 128-byte TMA tensor-map descriptors (CUtensorMap), filled on the host by cuTensorMapEncodeTiled and passed
 // to the kernels as a __grid_constant__ parameter.

@@ -149,7 +149,10 @@ class ScanProblem:
     # ---- backward ----
     def backward(self, dout, x=None):
         """-> [du, ddelta, dA, dB, dC, dD, ddelta_bias] with the reference's dtypes (selective_scan.cpp:319-347):
-        du/ddelta in u's dtype, dA/dD/ddelta_bias fp32, dB/dC accumulated in fp32 then cast to B's dtype."""
+        du/ddelta in u's dtype, dA/dD/ddelta_bias fp32, dB/dC accumulated in fp32 then cast to B's dtype.
+
+        Under torch.use_deterministic_algorithms(True) (warn_only included) the kernels that take no global atomics run:
+        the seven gradients are then bit-identical from call to call on the same GPU model (ss2d_scan_desc.deterministic)."""
         d, dev = self.desc, self.delta.device
         dch = self.u_mod if self.u_mod else self.dim
         _require(dout.is_cuda and dout.dtype == self.out_dtype, "dout must be a CUDA tensor of out's dtype")
@@ -174,9 +177,12 @@ class ScanProblem:
         du = torch.empty((self.batch, self.dim, self.L), dtype=u.dtype, device=dev) if self.u_mod else torch.empty_like(u)
         ddelta = torch.empty_like(delta)
         # one zero-fill launch for every accumulator (the live GM-UNet regime is launch-bound: 104 scan calls per step):
-        # dB | dC always; for d_state = 1 also dA | dD | ddelta_bias, which the lean kernel then adds into directly
+        # dB | dC always; for d_state = 1 also dA | dD | ddelta_bias, which the lean kernel then adds into directly —
+        # except in deterministic mode, where those three are overwritten by the fixed-order finalize pass
+        det = torch.are_deterministic_algorithms_enabled()
+        d.deterministic = int(det)
         nbc = self.batch * self.G * self.N * self.L
-        small = self.N == 1
+        small = self.N == 1 and not det
         extra = self.dim * (self.N + 2) if small else 0
         zbuf = torch.zeros(2 * nbc + extra, dtype=torch.float32, device=dev)
         dB, dC = zbuf[:nbc].view(self.batch, self.G, self.N, self.L), zbuf[nbc:2 * nbc].view(self.batch, self.G, self.N, self.L)

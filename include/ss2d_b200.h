@@ -92,6 +92,14 @@ typedef struct ss2d_scan_desc {
    * buffer) and may be accumulated into; the d_state = 1 path then adds its per-batch sums straight into them and the call is
    * a single kernel. 0: they are fully overwritten (per-batch partials in `workspace` + a fixed-order finalize pass). */
   int32_t grads_prezeroed;
+  /* Backward only. 1: every output of ss2d_scan_bwd is a function of its inputs alone — no floating-point sum depends on
+   * the order in which CTAs finish, so the results are bit-identical across calls, streams and CUDA-graph replays on the
+   * same GPU model with the same library build. The launch geometry depends on the SM count, so results are NOT promised
+   * to match across GPU models. dA, dD and ddelta_bias are then fully overwritten whatever grads_prezeroed says; dB / dC
+   * are fully written (zeroing them first is harmless). The CTAs that share a group write partial slabs (in `workspace`,
+   * see ss2d_scan_bwd_workspace_bytes) that a second pass sums in slab order. 0: the default; values other than 0 / 1
+   * are rejected (SS2D_ERR_BAD_SHAPE). */
+  int32_t deterministic;
 } ss2d_scan_desc;
 
 /* ---- forward -------------------------------------------------------------------------------
@@ -122,6 +130,8 @@ int ss2d_scan_bwd(const ss2d_scan_desc* desc, const void* u, const void* delta, 
                   float* dC, float* dD, float* ddelta_bias, void* workspace, size_t workspace_bytes,
                   ss2d_stream_t stream);
 
+/* Includes the partial dB / dC slabs when desc->deterministic is 1 (about (S - 1) x 2 x batch x groups x dstate x L floats,
+ * S = the most CTAs or warps one group is split over); with it at 0 the size does not depend on the field. */
 size_t ss2d_scan_bwd_workspace_bytes(const ss2d_scan_desc* desc, int have_ckpt);
 
 /* ---- stand-alone cross-scan / cross-merge (exact permutations; model/gm/csms6s.py:11-206) ----
