@@ -21,6 +21,7 @@ MAX_DSTATE = 256
 # every symbol include/ss2d_b200.h declares (tests/test_abi.py checks the library exports all of them)
 EXPORTS = [
     "ss2d_scan_fwd", "ss2d_scan_ckpt_floats", "ss2d_scan_bwd", "ss2d_scan_bwd_workspace_bytes",
+    "ss2d_scan_fwd_state", "ss2d_scan_bwd_state",
     "ss2d_cross_scan", "ss2d_cross_merge", "ss2d_out_gate_fwd", "ss2d_out_gate_bwd",
     "ss2d_out_gate_bwd_partials", "ss2d_group_gate_fwd", "ss2d_group_gate_bwd", "ss2d_out_gate_max_width", "ss2d_wgrad_ts", "ss2d_wgrad_ts_workspace_bytes",
     "ss2d_layernorm_fwd", "ss2d_layernorm_bwd", "ss2d_layernorm_bwd_partials",
@@ -84,6 +85,10 @@ def lib() -> ctypes.CDLL:
     L.ss2d_scan_ckpt_floats.restype = sz
     L.ss2d_scan_bwd.argtypes = [dp, vp, vp, fp, vp, vp, fp, fp, vp, fp, vp, vp, fp, fp, fp, fp, fp, vp, sz, vp]
     L.ss2d_scan_bwd.restype = ctypes.c_int
+    L.ss2d_scan_fwd_state.argtypes = [dp, vp, vp, fp, vp, vp, fp, fp, fp, vp, fp, fp, vp]
+    L.ss2d_scan_fwd_state.restype = ctypes.c_int
+    L.ss2d_scan_bwd_state.argtypes = [dp, vp, vp, fp, vp, vp, fp, fp, fp, vp, fp, fp, vp, vp, fp, fp, fp, fp, fp, fp, vp, sz, vp]
+    L.ss2d_scan_bwd_state.restype = ctypes.c_int
     L.ss2d_scan_bwd_workspace_bytes.argtypes = [dp, ctypes.c_int]
     L.ss2d_scan_bwd_workspace_bytes.restype = sz
     ip = ctypes.POINTER(ctypes.c_int32)

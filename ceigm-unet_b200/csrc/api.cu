@@ -12,8 +12,8 @@
 #include "ss2d_b200.h"
 
 namespace ss2d {
-cudaError_t scan_fwd_dispatch(const ScanParams& p, cudaStream_t stream);
-bool scan_fwdr_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err);
+cudaError_t scan_fwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream);
+bool scan_fwdr_try(const ScanParams& p, const ScanState& st, cudaStream_t stream, cudaError_t* err);
 constexpr int kDwnMaxSeg = 4;
 struct DwnSegs { int nseg; int cbeg[kDwnMaxSeg + 1]; int k[kDwnMaxSeg]; const float* w[kDwnMaxSeg]; const float* b[kDwnMaxSeg]; };
 cudaError_t dwnhwc_stencil_launch(const void* x, const void* aux, void* y, const DwnSegs& sg, int flip, int epi, int B, int H,
@@ -23,14 +23,14 @@ cudaError_t dwnhwc_wgrad_launch(const void* x, const void* g, int c0, int nc, in
                                 int C, int dt, float* part, cudaStream_t stream);
 // backward launchers: *slabs receives the number of dB / dC partial slabs the launch wrote in deterministic mode (0 or 1:
 // dB / dC hold the result already)
-cudaError_t scan_bwd_dispatch(const ScanParams& p, cudaStream_t stream, int* slabs);
+cudaError_t scan_bwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream, int* slabs);
 cudaError_t scan_bwd_finalize(const ScanParams& p, float* dA, float* dD, float* dbias, cudaStream_t stream);
 cudaError_t scan_bwd_fold(const ScanParams& p, int slabs, cudaStream_t stream);
-cudaError_t scan_par_fwd_dispatch(const ScanParams& p, cudaStream_t stream);
-cudaError_t scan_par_bwd_dispatch(const ScanParams& p, cudaStream_t stream, int* slabs);
-bool scan_n1_fwd_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err);
-bool scan_n1_bwd_try(const ScanParams& p, float* dA, float* dD, float* dbias, int grads_zeroed, cudaStream_t stream,
-                     cudaError_t* err, int* slabs);
+cudaError_t scan_par_fwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream);
+cudaError_t scan_par_bwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream, int* slabs);
+bool scan_n1_fwd_try(const ScanParams& p, const ScanState& st, cudaStream_t stream, cudaError_t* err);
+bool scan_n1_bwd_try(const ScanParams& p, const ScanState& st, float* dA, float* dD, float* dbias, int grads_zeroed,
+                     cudaStream_t stream, cudaError_t* err, int* slabs);
 // most partial slabs any backward kernel the dispatcher may pick for this pass writes in deterministic mode
 int scan_bwd_det_slabs(const ScanParams& p);
 int scan_n1_bwd_det_slabs(const ScanParams& p);
@@ -219,12 +219,18 @@ size_t ss2d_scan_bwd_workspace_bytes(const ss2d_scan_desc* d, int have_ckpt) {
 int ss2d_scan_fwd(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
                   const void* Cmat, const float* Dvec, const float* delta_bias, void* out, float* ckpt,
                   float* last_state, ss2d_stream_t stream) {
+  return ss2d_scan_fwd_state(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, nullptr, out, ckpt, last_state, stream);
+}
+
+int ss2d_scan_fwd_state(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, void* out,
+                        float* ckpt, float* last_state, ss2d_stream_t stream) {
   int rc = validate(d);
   if (rc != SS2D_OK) return rc;
   if (!u || !delta || !A || !Bmat || !Cmat || (!out && !ckpt && !last_state)) return SS2D_ERR_NULL_POINTER;
   if (!aligned(u, esize(d->io_dtype)) || !aligned(delta, esize(d->io_dtype)) || !aligned(Bmat, esize(d->io_dtype)) ||
       !aligned(Cmat, esize(d->io_dtype)) || !aligned(A, 4) || (out && !aligned(out, esize(d->out_dtype))) ||
-      (ckpt && !aligned(ckpt, 16)))
+      (ckpt && !aligned(ckpt, 16)) || !aligned(h0, 16))
     return SS2D_ERR_ALIGNMENT;
   ScanParams p;
   pack(d, p);
@@ -241,12 +247,13 @@ int ss2d_scan_fwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
     p.Cm = static_cast<const char*>(Cmat) + (size_t)n0 * d->C_state_stride * esize(d->io_dtype);
     p.ckpt = ckpt ? ckpt + ck_off : nullptr;
     p.last_state = last_state ? last_state + (d->last_state_interleaved ? 2 : 1) * n0 : nullptr;
+    const ScanState st = {h0 ? h0 + n0 : nullptr, nullptr, nullptr};
     ck_off += round4(ckpt_floats_pass(d, n));
     cudaError_t e;
     if (use_par(p)) {      // d_state = 1: lean fp32 kernels (scan_n1.cu) when eligible, else the generic parallel-along-L ones
-      if (!scan_n1_fwd_try(p, static_cast<cudaStream_t>(stream), &e)) e = scan_par_fwd_dispatch(p, static_cast<cudaStream_t>(stream));
-    } else if (!scan_fwdr_try(p, static_cast<cudaStream_t>(stream), &e)) {     // lane-owns-row fast path (scan_fwdr.cu)
-      e = scan_fwd_dispatch(p, static_cast<cudaStream_t>(stream));
+      if (!scan_n1_fwd_try(p, st, static_cast<cudaStream_t>(stream), &e)) e = scan_par_fwd_dispatch(p, st, static_cast<cudaStream_t>(stream));
+    } else if (!scan_fwdr_try(p, st, static_cast<cudaStream_t>(stream), &e)) {     // lane-owns-row fast path (scan_fwdr.cu)
+      e = scan_fwd_dispatch(p, st, static_cast<cudaStream_t>(stream));
     }
     if (e != cudaSuccess) return cuda_fail(e);
     ++g_launches;
@@ -258,6 +265,15 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
                   const void* Cmat, const float* Dvec, const float* delta_bias, const void* dout, const float* ckpt,
                   void* du, void* ddelta, float* dA, float* dB, float* dC, float* dD, float* ddelta_bias,
                   void* workspace, size_t workspace_bytes, ss2d_stream_t stream) {
+  return ss2d_scan_bwd_state(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, nullptr, dout, nullptr, ckpt, du, ddelta, dA, dB,
+                             dC, dD, ddelta_bias, nullptr, workspace, workspace_bytes, stream);
+}
+
+int ss2d_scan_bwd_state(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* dout,
+                        const float* dlast, const float* ckpt, void* du, void* ddelta, float* dA, float* dB, float* dC,
+                        float* dD, float* ddelta_bias, float* dh0, void* workspace, size_t workspace_bytes,
+                        ss2d_stream_t stream) {
   int rc = validate(d);
   if (rc != SS2D_OK) return rc;
   if (!u || !delta || !A || !Bmat || !Cmat || !dout || !du || !ddelta || !dA || !dB || !dC) return SS2D_ERR_NULL_POINTER;
@@ -270,9 +286,9 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
   if (!aligned(u, esize(d->io_dtype)) || !aligned(delta, esize(d->io_dtype)) || !aligned(Bmat, esize(d->io_dtype)) ||
       !aligned(Cmat, esize(d->io_dtype)) || !aligned(A, 4) || !aligned(dout, esize(d->out_dtype)) ||
       !aligned(du, esize(d->io_dtype)) || !aligned(ddelta, esize(d->io_dtype)) || !aligned(dA, 4) ||
-      !aligned(dB, bc_al) || !aligned(dC, bc_al))
+      !aligned(dB, bc_al) || !aligned(dC, bc_al) || !aligned(h0, 16) || !aligned(dlast, 16) || !aligned(dh0, 16))
     return SS2D_ERR_ALIGNMENT;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  cudaStream_t cst = static_cast<cudaStream_t>(stream);
   float* ws = static_cast<float*>(workspace);
   const int nmax = d->dstate < kStatesPerPass ? d->dstate : kStatesPerPass;
   float* part = ws;
@@ -280,7 +296,7 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
   float* slab_base = own_ckpt + (ckpt ? 0 : ss2d_scan_ckpt_floats(d));
   const int smax = det_slabs(d);
   if (!ckpt) {   // recompute the chunk states with a forward sweep that writes nothing else
-    rc = ss2d_scan_fwd(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, nullptr, own_ckpt, nullptr, stream);
+    rc = ss2d_scan_fwd_state(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, h0, nullptr, own_ckpt, nullptr, stream);
     if (rc != SS2D_OK) return rc;
     ckpt = own_ckpt;
   }
@@ -306,25 +322,26 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
     p.dC = dC + (size_t)n0 * d->seqlen;
     p.slabB = slab_base + (size_t)n0 * d->seqlen;
     p.slabC = slab_base + (size_t)(smax > 1 ? smax - 1 : 0) * p.slab_stride + (size_t)n0 * d->seqlen;
+    const ScanState st = {h0 ? h0 + n0 : nullptr, dlast ? dlast + n0 : nullptr, dh0 ? dh0 + n0 : nullptr};
     ck_off += round4(ckpt_floats_pass(d, n));
     cudaError_t e;
     bool finalize = true;
     int slabs = 0;
     if (use_par(p)) {
-      if (scan_n1_bwd_try(p, dA, dD, ddelta_bias, zeroed, st, &e, &slabs)) finalize = !zeroed;
-      else e = scan_par_bwd_dispatch(p, st, &slabs);
+      if (scan_n1_bwd_try(p, st, dA, dD, ddelta_bias, zeroed, cst, &e, &slabs)) finalize = !zeroed;
+      else e = scan_par_bwd_dispatch(p, st, cst, &slabs);
     } else {
-      e = scan_bwd_dispatch(p, st, &slabs);
+      e = scan_bwd_dispatch(p, st, cst, &slabs);
     }
     if (e != cudaSuccess) return cuda_fail(e);
     ++g_launches;
     if (slabs > 1) {
-      e = scan_bwd_fold(p, slabs, st);
+      e = scan_bwd_fold(p, slabs, cst);
       if (e != cudaSuccess) return cuda_fail(e);
       ++g_launches;
     }
     if (finalize) {
-      e = scan_bwd_finalize(p, dA + n0, dD, ddelta_bias, st);
+      e = scan_bwd_finalize(p, dA + n0, dD, ddelta_bias, cst);
       if (e != cudaSuccess) return cuda_fail(e);
       ++g_launches;
     }

@@ -44,8 +44,10 @@ struct FwdShape {
 //       writing the same swizzled layout.
 //   warps 0-3 (consumers) own RPW channel rows each: wait `full`, activate delta for their own rows, run the
 //   recurrence over the tile, then release the stage through its `empty` mbarrier. B/C are read-only and shared.
-template <int NS, int R, int RPT, int STAGES>
-__global__ void __launch_bounds__(kFwdThreads) scan_fwd_kernel(const ScanParams p, const __grid_constant__ TmaMaps maps) {
+// STATE: the rows start from st.h0 instead of 0
+template <int NS, int R, int RPT, int STAGES, bool STATE>
+__global__ void __launch_bounds__(kFwdThreads) scan_fwd_kernel(const ScanParams p, const __grid_constant__ TmaMaps maps,
+                                                                const ScanState st) {
   using S = FwdShape<NS, R, RPT, STAGES>;
   constexpr int CH = S::CH, NP = S::NP, NPB = S::NPB, RL = S::RL, RPW = S::RPW;
   extern __shared__ __align__(16) float smem_raw[];
@@ -135,7 +137,7 @@ __global__ void __launch_bounds__(kFwdThreads) scan_fwd_kernel(const ScanParams 
     for (int j = 0; j < NS; ++j) {
       const int n = j * R + q;
       A2[k][j] = (rk[k] < rows_valid && n < p.N) ? p.A[(int64_t)(d0 + rk[k]) * p.A_ld + n] * kLog2e : 0.f;
-      h[k][j] = 0.f;
+      h[k][j] = (STATE && rk[k] < rows_valid && n < p.N) ? st.h0[state_slot(p, b, d0 + rk[k], n)] : 0.f;
     }
   }
 
@@ -258,10 +260,10 @@ __global__ void __launch_bounds__(kFwdThreads) scan_fwd_kernel(const ScanParams 
   }
 }
 
-template <int NS, int R, int RPT, int STAGES>
-static cudaError_t launch_fwd(ScanParams p, cudaStream_t stream) {
+template <int NS, int R, int RPT, int STAGES, bool STATE>
+static cudaError_t launch_fwd(ScanParams p, const ScanState& st, cudaStream_t stream) {
   using S = FwdShape<NS, R, RPT, STAGES>;
-  auto kern = scan_fwd_kernel<NS, R, RPT, STAGES>;
+  auto kern = scan_fwd_kernel<NS, R, RPT, STAGES, STATE>;
   static PerDeviceOnce once;     // per instantiation and per device (the attribute is per-function, per-device and sticky)
   cudaError_t ea = func_attr_once(once, reinterpret_cast<const void*>(kern), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::smem_bytes);
   if (ea != cudaSuccess) return ea;
@@ -270,18 +272,23 @@ static cudaError_t launch_fwd(ScanParams p, cudaStream_t stream) {
   if (p.tma_ok && !make_scan_maps(p, S::CH, S::NPB, false, &maps)) p.tma_ok = 0;
   if (!p.tma_ok) memset(&maps, 0, sizeof(maps));
   dim3 grid((p.dpg + S::CH - 1) / S::CH, p.G, p.batch);
-  kern<<<grid, kFwdThreads, S::smem_bytes, stream>>>(p, maps);
+  kern<<<grid, kFwdThreads, S::smem_bytes, stream>>>(p, maps, st);
   return cudaGetLastError();
 }
 
-cudaError_t scan_fwd_dispatch(const ScanParams& p, cudaStream_t stream) {
+template <bool STATE>
+static cudaError_t fwd_variant(const ScanParams& p, const ScanState& st, cudaStream_t stream) {
   const Variant v = pick_variant(p.N);
-  if (v.NS == 1) return launch_fwd<1, 1, 1, 3>(p, stream);
-  if (v.NS == 2) return launch_fwd<2, 1, 1, 3>(p, stream);
-  if (v.R == 1) return launch_fwd<4, 1, 1, 3>(p, stream);
-  if (v.R == 2) return launch_fwd<4, 2, 1, 3>(p, stream);
-  if (v.R == 4) return launch_fwd<4, 4, 1, 3>(p, stream);     // measured best of RPT in {1, 2} x STAGES in {2, 3, 4} (DESIGN.md §3.1)
-  return launch_fwd<4, 8, 1, 3>(p, stream);
+  if (v.NS == 1) return launch_fwd<1, 1, 1, 3, STATE>(p, st, stream);
+  if (v.NS == 2) return launch_fwd<2, 1, 1, 3, STATE>(p, st, stream);
+  if (v.R == 1) return launch_fwd<4, 1, 1, 3, STATE>(p, st, stream);
+  if (v.R == 2) return launch_fwd<4, 2, 1, 3, STATE>(p, st, stream);
+  if (v.R == 4) return launch_fwd<4, 4, 1, 3, STATE>(p, st, stream);     // measured best of RPT in {1, 2} x STAGES in {2, 3, 4} (DESIGN.md §3.1)
+  return launch_fwd<4, 8, 1, 3, STATE>(p, st, stream);
+}
+
+cudaError_t scan_fwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream) {
+  return st.h0 ? fwd_variant<true>(p, st, stream) : fwd_variant<false>(p, st, stream);
 }
 
 }  // namespace ss2d

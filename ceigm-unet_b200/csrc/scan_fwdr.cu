@@ -40,9 +40,12 @@ struct FwdrShape {
   static constexpr size_t smem_bytes = (size_t)FR_NW * warp_bytes + FR_NW * FR_STAGES * 8 + 1024;
 };
 
-template <int NS, int R, bool SOFTPLUS, bool SEG>
+// STATE (whole-row mode only): the rows start from st.h0 instead of 0. Segmented mode scans every segment from zero and
+// leaves h0 to the carry / fix-up kernels.
+template <int NS, int R, bool SOFTPLUS, bool SEG, bool STATE>
 __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams p, const __grid_constant__ FwdrMaps maps,
-                                                               const int nrb, const int nwb, const int nseg_arg, const int tps) {
+                                                               const int nrb, const int nwb, const int nseg_arg, const int tps,
+                                                               const ScanState st) {
   const int nseg = SEG ? nseg_arg : 1;                     // compile-time 1 in the whole-row instantiation
   using S = FwdrShape<R>;
   constexpr int ROWS = S::ROWS;
@@ -98,7 +101,7 @@ __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams 
   for (int j = 0; j < NS; ++j) {
     const int n = j * R + q;
     A2[j] = (valid && n < p.N) ? p.A[(int64_t)d * p.A_ld + n] * kLog2e : 0.f;
-    h[j] = 0.f;
+    h[j] = (STATE && valid && n < p.N) ? st.h0[state_slot(p, b, d, n)] : 0.f;
   }
   const float bias = (valid && p.bias) ? p.bias[d] : 0.f;
   const float Dd = (valid && p.Dv) ? p.Dv[d] : 0.f;
@@ -253,10 +256,11 @@ static bool fwdr_maps(const ScanParams& p, FwdrMaps* m) {
          make_tmap(&m->B, p.Bm, 4, d4, s4B, 16, R > 1) && make_tmap(&m->C, p.Cm, 4, d4, s4C, 16, R > 1);
 }
 
-template <int NS, int R, bool SOFTPLUS, bool SEG>
-static cudaError_t launch_fwdr(const ScanParams& p, const FwdrMaps& maps, cudaStream_t stream, int nseg = 1, int tps = 0) {
+template <int NS, int R, bool SOFTPLUS, bool SEG, bool STATE>
+static cudaError_t launch_fwdr(const ScanParams& p, const FwdrMaps& maps, const ScanState& st, cudaStream_t stream, int nseg = 1,
+                               int tps = 0) {
   using S = FwdrShape<R>;
-  auto kern = scan_fwdr_kernel<NS, R, SOFTPLUS, SEG>;
+  auto kern = scan_fwdr_kernel<NS, R, SOFTPLUS, SEG, STATE>;
   static PerDeviceOnce once;
   cudaError_t e = func_attr_once(once, reinterpret_cast<const void*>(kern), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::smem_bytes);
   if (e != cudaSuccess) return e;
@@ -264,7 +268,7 @@ static cudaError_t launch_fwdr(const ScanParams& p, const FwdrMaps& maps, cudaSt
   const int nrb = (p.dpg + S::ROWS - 1) / S::ROWS;
   const long long nwb = (long long)nrb * p.G * p.batch * nseg;
   if (tps <= 0) tps = (p.L + FR_LT - 1) / FR_LT;
-  kern<<<(unsigned)((nwb + FR_NW - 1) / FR_NW), FR_NW * 32, S::smem_bytes, stream>>>(p, maps, nrb, (int)nwb, nseg, tps);
+  kern<<<(unsigned)((nwb + FR_NW - 1) / FR_NW), FR_NW * 32, S::smem_bytes, stream>>>(p, maps, nrb, (int)nwb, nseg, tps, st);
   return cudaGetLastError();
 }
 
@@ -296,9 +300,10 @@ __device__ __forceinline__ float4 activate4(float4 x, float bias) {
   return x;
 }
 
-// CTA per row: its four warps split the segments for the sums, warp 0 runs the carry chain
-template <bool SOFTPLUS>
-__global__ void __launch_bounds__(128) scan_fwd_carry_kernel(const ScanParams p, const int tps, const int nseg) {
+// CTA per row: its four warps split the segments for the sums, warp 0 runs the carry chain.
+// STATE: the chain starts from h0, so segment 0's end state changes too.
+template <bool SOFTPLUS, bool STATE>
+__global__ void __launch_bounds__(128) scan_fwd_carry_kernel(const ScanParams p, const int tps, const int nseg, const ScanState st) {
   __shared__ float s_sum[FX_MAX_SEG];
   __shared__ float s_e[FX_MAX_SEG][16];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -329,11 +334,11 @@ __global__ void __launch_bounds__(128) scan_fwd_carry_kernel(const ScanParams p,
   // phase 2: h_s = e_s + exp(A S_s) h_(s-1), the true end state of segment s
   if (warp == 0 && lane < N) {
     const float A2l = p.A[(int64_t)d * p.A_ld + lane] * kLog2e;
-    float h = 0.f;
+    float h = STATE ? st.h0[state_slot(p, b, d, lane)] : 0.f;
     for (int s = 0; s < nseg; ++s) {
       h = fmaf(ex2f(A2l * s_sum[s]), h, s_e[s][lane]);
       const int tl = min(ntiles, (s + 1) * tps) - 1;
-      if (s > 0) ck[(int64_t)tl * N + lane] = h;
+      if (STATE || s > 0) ck[(int64_t)tl * N + lane] = h;
     }
     if (p.last_state != nullptr) {
       const int64_t slot = ((int64_t)b * p.dim + d) * p.A_ld + lane;
@@ -343,13 +348,15 @@ __global__ void __launch_bounds__(128) scan_fwd_carry_kernel(const ScanParams p,
   }
 }
 
-// warp per (row, segment >= 1); a lane owns 4 consecutive positions of a 128-position step
-template <bool SOFTPLUS>
-__global__ void __launch_bounds__(128) scan_fwd_fixup_kernel(const ScanParams p, const int tps, const int nseg) {
+// warp per (row, segment >= 1; STATE: segment >= 0, whose carried-in state is h0); a lane owns 4 consecutive positions of a
+// 128-position step
+template <bool SOFTPLUS, bool STATE>
+__global__ void __launch_bounds__(128) scan_fwd_fixup_kernel(const ScanParams p, const int tps, const int nseg, const ScanState st) {
+  constexpr int S0 = STATE ? 0 : 1;      // first segment fixed up
   const int lane = threadIdx.x & 31;
   const int64_t wid = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
-  if (wid >= (int64_t)p.batch * p.dim * (nseg - 1)) return;
-  const int row = (int)(wid / (nseg - 1)), seg = 1 + (int)(wid % (nseg - 1));
+  if (wid >= (int64_t)p.batch * p.dim * (nseg - S0)) return;
+  const int row = (int)(wid / (nseg - S0)), seg = S0 + (int)(wid % (nseg - S0));
   const int b = row / p.dim, d = row - b * p.dim, g = d / p.dpg;
   const int L = p.L, N = p.N;
   const bool rev = p.layout == SS2D_LAYOUT_NATURAL && p.dirs[g] == 3;
@@ -362,7 +369,8 @@ __global__ void __launch_bounds__(128) scan_fwd_fixup_kernel(const ScanParams p,
   float* ck = p.ckpt + ((int64_t)b * p.dim + d) * p.nck * N;
   const float bias = p.bias ? p.bias[d] : 0.f;
   const float A2l = lane < N ? p.A[(int64_t)d * p.A_ld + lane] * kLog2e : 0.f;
-  const float hl = lane < N ? ck[(int64_t)(tb - 1) * N + lane] : 0.f;     // true state entering the segment (carry kernel)
+  // true state entering the segment (carry kernel; h0 for segment 0)
+  const float hl = lane >= N ? 0.f : (STATE && seg == 0) ? st.h0[state_slot(p, b, d, lane)] : ck[(int64_t)(tb - 1) * N + lane];
   float A2[16], hin[16];
 #pragma unroll
   for (int n = 0; n < 16; ++n) {
@@ -423,10 +431,30 @@ __global__ void __launch_bounds__(128) scan_fwd_fixup_kernel(const ScanParams p,
   }
 }
 
+template <bool STATE>
+static cudaError_t fwdr_launch_all(const ScanParams& p, const FwdrMaps& maps, const ScanState& st, cudaStream_t stream, bool r1,
+                                   int nseg, int tps) {
+  if (r1) return p.softplus ? launch_fwdr<16, 1, true, false, STATE>(p, maps, st, stream) : launch_fwdr<16, 1, false, false, STATE>(p, maps, st, stream);
+  if (nseg == 1) return p.softplus ? launch_fwdr<8, 2, true, false, STATE>(p, maps, st, stream) : launch_fwdr<8, 2, false, false, STATE>(p, maps, st, stream);
+  cudaError_t e = p.softplus ? launch_fwdr<8, 2, true, true, false>(p, maps, st, stream, nseg, tps)
+                             : launch_fwdr<8, 2, false, true, false>(p, maps, st, stream, nseg, tps);
+  if (e != cudaSuccess) return e;
+  const long long rows = (long long)p.batch * p.dim;
+  const unsigned gc = (unsigned)rows, gf = (unsigned)((rows * (nseg - (STATE ? 0 : 1)) + 3) / 4);
+  if (p.softplus) {
+    scan_fwd_carry_kernel<true, STATE><<<gc, 128, 0, stream>>>(p, tps, nseg, st);
+    scan_fwd_fixup_kernel<true, STATE><<<gf, 128, 0, stream>>>(p, tps, nseg, st);
+  } else {
+    scan_fwd_carry_kernel<false, STATE><<<gc, 128, 0, stream>>>(p, tps, nseg, st);
+    scan_fwd_fixup_kernel<false, STATE><<<gf, 128, 0, stream>>>(p, tps, nseg, st);
+  }
+  return cudaGetLastError();
+}
+
 int scan_path_policy();     // api.cu
 
 // Returns true when the fast path took the call (*err holds the launch status).
-bool scan_fwdr_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err) {
+bool scan_fwdr_try(const ScanParams& p, const ScanState& st, cudaStream_t stream, cudaError_t* err) {
   if (!p.tma_ok || p.N <= 4 || p.N > 16 || p.accum || p.io_dtype != SS2D_F32 || p.out_dtype != SS2D_F32) return false;
   if (p.u_mod > 0 && p.u_mod % p.dpg != 0) return false;
   for (int g = 0; g < p.G; ++g) {
@@ -462,26 +490,8 @@ bool scan_fwdr_try(const ScanParams& p, cudaStream_t stream, cudaError_t* err) {
   }
   const bool r1 = nseg == 1 && (policy == 0 ? wb1 >= need : policy == 1);
   FwdrMaps maps;
-  if (r1) {
-    if (!fwdr_maps<1>(p, &maps)) return false;
-    *err = p.softplus ? launch_fwdr<16, 1, true, false>(p, maps, stream) : launch_fwdr<16, 1, false, false>(p, maps, stream);
-    return true;
-  }
-  if (!fwdr_maps<2>(p, &maps)) return false;
-  if (nseg > 1) *err = p.softplus ? launch_fwdr<8, 2, true, true>(p, maps, stream, nseg, tps) : launch_fwdr<8, 2, false, true>(p, maps, stream, nseg, tps);
-  else *err = p.softplus ? launch_fwdr<8, 2, true, false>(p, maps, stream) : launch_fwdr<8, 2, false, false>(p, maps, stream);
-  if (nseg > 1 && *err == cudaSuccess) {
-    const long long rows = (long long)p.batch * p.dim;
-    const unsigned gc = (unsigned)rows, gf = (unsigned)((rows * (nseg - 1) + 3) / 4);
-    if (p.softplus) {
-      scan_fwd_carry_kernel<true><<<gc, 128, 0, stream>>>(p, tps, nseg);
-      scan_fwd_fixup_kernel<true><<<gf, 128, 0, stream>>>(p, tps, nseg);
-    } else {
-      scan_fwd_carry_kernel<false><<<gc, 128, 0, stream>>>(p, tps, nseg);
-      scan_fwd_fixup_kernel<false><<<gf, 128, 0, stream>>>(p, tps, nseg);
-    }
-    *err = cudaGetLastError();
-  }
+  if (!(r1 ? fwdr_maps<1>(p, &maps) : fwdr_maps<2>(p, &maps))) return false;
+  *err = st.h0 ? fwdr_launch_all<true>(p, maps, st, stream, r1, nseg, tps) : fwdr_launch_all<false>(p, maps, st, stream, r1, nseg, tps);
   return true;
 }
 

@@ -47,6 +47,23 @@ struct ScanParams {
   int64_t slab_stride;
 };
 
+// State passing, a separate kernel argument of the STATE instantiations (ScanParams keeps its layout, so the default kernels
+// keep their instructions). Rows of A_ld floats like A; this pass's states start at element 0. Forward: the state before a
+// row's first position is h0 (non-null whenever STATE). Backward: h0 starts the recompute of chunk 0, dlast is the adjoint
+// entering the row's last position, dh0 receives the adjoint of h0; each may be null.
+struct ScanState {
+  const float* h0;
+  const float* dlast;
+  float* dh0;
+};
+// backward: the STATE instantiation runs when any of the three pointers is set
+inline bool has_state(const ScanState& st) { return st.h0 || st.dlast || st.dh0; }
+
+// state element n of row (b, d): h0 / dlast / dh0 layout
+__host__ __device__ inline int64_t state_slot(const ScanParams& p, int b, int d, int n) {
+  return ((int64_t)b * p.dim + d) * p.A_ld + n;
+}
+
 // destination of partial slab s of dB (which 0) or dC (which 1)
 __host__ __device__ inline float* det_slab(const ScanParams& p, int which, int s) {
   if (s == 0) return which ? p.dC : p.dB;

@@ -65,6 +65,43 @@ class SelectiveScanOflex(torch.autograd.Function):
     backward = SelectiveScanCore.backward
 
 
+class _SelectiveScanState(torch.autograd.Function):
+    """selective_scan with an initial state and the final state as a differentiable output (see `selective_scan`)."""
+
+    @staticmethod
+    def forward(ctx, u, delta, A, B, C, D, delta_bias, delta_softplus, h0):
+        prob = ops.ScanProblem(u, delta, A, B, C, D, delta_bias, delta_softplus, out_float=False)
+        out, x = prob.forward(want_state=True, h0=h0)
+        last = x[:, :, 0, 1::2].contiguous()
+        ctx.delta_softplus = delta_softplus
+        ctx.has_h0 = h0 is not None
+        ctx.save_for_backward(u, delta, A, B, C, D, delta_bias, h0, x)
+        return out, last
+
+    @staticmethod
+    def backward(ctx, dout, dlast):
+        u, delta, A, B, C, D, delta_bias, h0, x = ctx.saved_tensors
+        prob = ops.ScanProblem(u, delta, A, B, C, D, delta_bias, ctx.delta_softplus, out_float=False)
+        du, ddelta, dA, dB, dC, dD, dbias, dh0 = prob.backward(dout.contiguous(), x, h0=h0, dlast=dlast,
+                                                              want_dh0=ctx.needs_input_grad[8])
+        return du, ddelta, dA, dB, dC, dD, dbias, None, dh0
+
+
+def selective_scan(u, delta, A, B, C, D=None, delta_bias=None, delta_softplus=False, initial_state=None,
+                   return_last_state=False):
+    """Differentiable selective scan with state passing, in the reference extension's SCAN layout and dtype rules:
+    u, delta (B, Dt, L) and B, C (B, G, N, L) or (B, N, L) of one dtype (fp32 / fp16 / bf16), A (Dt, N) fp32, D and
+    delta_bias (Dt) fp32 or None; out has u's dtype.
+
+        h_l = exp(delta_l A) * h_(l-1) + delta_l u_l B_l,  h_(-1) = initial_state (zeros when None),  out_l = C_l . h_l + D u_l
+
+    initial_state: (B, Dt, N) fp32 or None; gradients flow to it. return_last_state: also return h_(L-1) as a (B, Dt, N)
+    fp32 tensor whose gradient flows back through the scan, so a sequence split into pieces can be chained call by call.
+    Under torch.use_deterministic_algorithms(True) every gradient is bit-identical from call to call."""
+    out, last = _SelectiveScanState.apply(u, delta, A, B, C, D, delta_bias, bool(delta_softplus), initial_state)
+    return (out, last) if return_last_state else out
+
+
 # ---- cross scan / merge ---------------------------------------------------------------------------
 def _make_cross_pair(dirs, suffix):
     dirs = tuple(dirs)

@@ -111,12 +111,26 @@ class ScanProblem:
                                       self.softplus, out_float=True, hw=self.hw, dirs=self.dirs, u_mod=self.u_mod)
         return self._inner
 
+    def _state_arg(self, t: Optional[torch.Tensor], name: str) -> Optional[torch.Tensor]:
+        """h0 / dlast: None, or a (batch, dim, dstate) fp32 CUDA tensor (made contiguous)."""
+        if t is None:
+            return None
+        _require(t.is_cuda and t.dtype == torch.float32, f"{name} must be a float32 CUDA tensor")
+        _require(tuple(t.shape) == (self.batch, self.dim, self.N), f"{name} must be (batch, dim, dstate)")
+        t = t.contiguous()
+        if t.data_ptr() % 16:
+            t = t.clone()
+        return t
+
     # ---- forward ----
-    def forward(self, want_state: bool = True):
+    def forward(self, want_state: bool = True, h0: Optional[torch.Tensor] = None):
         """-> (out (B, Dt, L), x). `x` has the reference's shape convention (B, Dt, 1, 2N): x[:, :, -1, 1::2] is the
-        final state; the chunk checkpoints for the backward live in front of it in the same storage."""
+        final state; the chunk checkpoints for the backward live in front of it in the same storage.
+        h0: optional (B, Dt, N) fp32 state before the first position (default zeros); a backward of this forward's `x` must
+        be given the same h0."""
+        h0 = self._state_arg(h0, "h0")
         if self._upcast:
-            out32, x = self._fp32_twin().forward(want_state)
+            out32, x = self._fp32_twin().forward(want_state, h0)
             return out32.to(self.out_dtype), x
         d, dev = self.desc, self.delta.device
         out = torch.empty((self.batch, self.dim, self.L), dtype=self.out_dtype, device=dev)
@@ -130,9 +144,14 @@ class ScanProblem:
             last = x
             d.last_state_interleaved = 1
         with torch.cuda.device(dev):
-            rc = _lib.lib().ss2d_scan_fwd(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
-                                          _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(out), _ptr(ckpt),
-                                          _ptr(last), _stream(dev))
+            if h0 is None:
+                rc = _lib.lib().ss2d_scan_fwd(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
+                                              _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(out), _ptr(ckpt),
+                                              _ptr(last), _stream(dev))
+            else:
+                rc = _lib.lib().ss2d_scan_fwd_state(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
+                                                    _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(out), _ptr(ckpt),
+                                                    _ptr(last), _stream(dev))
         _lib.check(rc, "ss2d_scan_fwd")
         return out, x
 
@@ -147,22 +166,29 @@ class ScanProblem:
         return torch.empty(0, dtype=torch.float32, device=x.device).set_(x.untyped_storage(), 0, (head,), (1,))
 
     # ---- backward ----
-    def backward(self, dout, x=None):
+    def backward(self, dout, x=None, h0: Optional[torch.Tensor] = None, dlast: Optional[torch.Tensor] = None,
+                 want_dh0: bool = False):
         """-> [du, ddelta, dA, dB, dC, dD, ddelta_bias] with the reference's dtypes (selective_scan.cpp:319-347):
         du/ddelta in u's dtype, dA/dD/ddelta_bias fp32, dB/dC accumulated in fp32 then cast to B's dtype.
 
         Under torch.use_deterministic_algorithms(True) (warn_only included) the kernels that take no global atomics run:
-        the seven gradients are then bit-identical from call to call on the same GPU model (ss2d_scan_desc.deterministic)."""
+        the seven gradients are then bit-identical from call to call on the same GPU model (ss2d_scan_desc.deterministic).
+
+        State passing: h0 is the forward's initial state (None: zeros), dlast the gradient of the final state (None: zeros).
+        With any of h0 / dlast / want_dh0 given, an eighth entry dh0 (B, Dt, N) fp32 (or None unless want_dh0) is appended."""
         d, dev = self.desc, self.delta.device
         dch = self.u_mod if self.u_mod else self.dim
         _require(dout.is_cuda and dout.dtype == self.out_dtype, "dout must be a CUDA tensor of out's dtype")
         _require(tuple(dout.shape) == (self.batch, dch, self.L), "dout must be (batch, dim, seqlen)")
+        h0, dlast = self._state_arg(h0, "h0"), self._state_arg(dlast, "dlast")
+        stateful = h0 is not None or dlast is not None or want_dh0
         if self._upcast:
-            du, ddelta, dA, dB, dC, dD, dbias = self._fp32_twin().backward(dout.float(), x)
+            grads = self._fp32_twin().backward(dout.float(), x, h0, dlast, want_dh0)
+            du, ddelta, dA, dB, dC, dD, dbias = grads[:7]
             dB, dC = dB.to(self.B.dtype), dC.to(self.C.dtype)
             if self.squeeze_BC:
                 dB, dC = dB[:, 0], dC[:, 0]
-            return [du.to(self.u.dtype), ddelta.to(self.delta.dtype), dA, dB, dC, dD, dbias]
+            return [du.to(self.u.dtype), ddelta.to(self.delta.dtype), dA, dB, dC, dD, dbias] + grads[7:]
         if dout.stride(-1) != 1:                                  # csms6s.py:360-361 does the same before calling bwd
             dout = dout.contiguous()
         d.out_batch_stride, d.out_dim_stride = dout.stride(0), dout.stride(1)
@@ -200,17 +226,25 @@ class ScanProblem:
         L = _lib.lib()
         ws_bytes = int(L.ss2d_scan_bwd_workspace_bytes(ctypes.byref(d), 1 if ckpt is not None else 0))
         ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=dev)
+        dh0 = torch.empty((self.batch, self.dim, self.N), dtype=torch.float32, device=dev) if want_dh0 else None
         with torch.cuda.device(dev):
-            rc = L.ss2d_scan_bwd(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B),
-                                 _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(dout), _ptr(ckpt), _ptr(du),
-                                 _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD), _ptr(dbias), _ptr(ws),
-                                 ctypes.c_size_t(ws_bytes), _stream(dev))
+            if not stateful:
+                rc = L.ss2d_scan_bwd(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B),
+                                     _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(dout), _ptr(ckpt), _ptr(du),
+                                     _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD), _ptr(dbias), _ptr(ws),
+                                     ctypes.c_size_t(ws_bytes), _stream(dev))
+            else:
+                rc = L.ss2d_scan_bwd_state(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B),
+                                           _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(dout), _ptr(dlast),
+                                           _ptr(ckpt), _ptr(du), _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD),
+                                           _ptr(dbias), _ptr(dh0), _ptr(ws), ctypes.c_size_t(ws_bytes), _stream(dev))
         _lib.check(rc, "ss2d_scan_bwd")
         if self.B.dtype != torch.float32:
             dB, dC = dB.to(self.B.dtype), dC.to(self.C.dtype)
         if self.squeeze_BC:
             dB, dC = dB[:, 0], dC[:, 0]
-        return [du, ddelta, dA, dB, dC, dD, dbias]
+        grads = [du, ddelta, dA, dB, dC, dD, dbias]
+        return grads + [dh0] if stateful else grads
 
 
 # ---- stand-alone permutations ------------------------------------------------------------------

@@ -134,6 +134,28 @@ int ss2d_scan_bwd(const ss2d_scan_desc* desc, const void* u, const void* delta, 
  * S = the most CTAs or warps one group is split over); with it at 0 the size does not depend on the field. */
 size_t ss2d_scan_bwd_workspace_bytes(const ss2d_scan_desc* desc, int have_ckpt);
 
+/* ---- state passing: a scan that starts from a given state, and its adjoint ----------------------
+ * The same calls as ss2d_scan_fwd / ss2d_scan_bwd (which are these with NULL state pointers), with
+ *   h_(-1) = h0 instead of 0:  h_l = exp(dt_l A) h_(l-1) + dt_l u_l B_l, l counted in traversal order (in NATURAL
+ *   layout h0 is the state before the first element the direction visits: the last pixel for directions 3 / 4);
+ *   backward: the adjoint entering position L - 1 from the right is dlast instead of 0, and dh0 = dloss / dh0 =
+ *   exp(dt_0 A) g_0 with g_0 the adjoint of h_0. The terms of h0 in dA and d(delta) at position 0 are included.
+ * h0, dlast, dh0: fp32 (batch, dim, dstate) contiguous (last_state's non-interleaved layout), 16-byte aligned, else
+ *   SS2D_ERR_ALIGNMENT. h0 / dlast NULL: zeros. dh0 NULL: not computed; else fully overwritten, each element by one thread
+ *   (deterministic whatever desc->deterministic says).
+ * Chaining: the forward of [0, m) hands its last_state to the forward of [m, L) as h0; the backward of [m, L) hands its
+ *   dh0 to the backward of [0, m) as dlast. dA, dD and d(delta_bias) of the two calls add up to those of one call over [0, L).
+ * ckpt from a forward given h0 must go to a backward given the same h0; with ckpt == NULL the recompute starts from h0.
+ * ss2d_scan_bwd_workspace_bytes applies unchanged. */
+int ss2d_scan_fwd_state(const ss2d_scan_desc* desc, const void* u, const void* delta, const float* A,
+                        const void* Bmat, const void* Cmat, const float* Dvec, const float* delta_bias,
+                        const float* h0, void* out, float* ckpt, float* last_state, ss2d_stream_t stream);
+int ss2d_scan_bwd_state(const ss2d_scan_desc* desc, const void* u, const void* delta, const float* A,
+                        const void* Bmat, const void* Cmat, const float* Dvec, const float* delta_bias,
+                        const float* h0, const void* dout, const float* dlast, const float* ckpt,
+                        void* du, void* ddelta, float* dA, float* dB, float* dC, float* dD, float* ddelta_bias,
+                        float* dh0, void* workspace, size_t workspace_bytes, ss2d_stream_t stream);
+
 /* ---- stand-alone cross-scan / cross-merge (exact permutations; model/gm/csms6s.py:11-206) ----
  * cross_scan : x (batch, channels, H, W) -> xs (batch, K, channels, L), xs[:,k] in direction dirs[k].
  * cross_merge: ys (batch, K, channels, L) in scan order -> y (batch, channels, L) natural order,
