@@ -1,9 +1,9 @@
 """ceigm-unet_b200 — B200-native (sm_100a) implementation of GM-UNet's SS2D selective-scan hot path.
 
 Layers (SURVEY.md §8b):
-  b1  dropin/selective_scan_cuda_core.py, dropin/selective_scan_cuda_oflex.py — the reference extension modules'
-      `fwd` / `bwd` functions; `install_dropin()` registers them in sys.modules so that the reference's own
-      `model/gm/csms6s.py` picks them up unchanged.
+  b1  dropin/selective_scan_cuda_core.py, dropin/selective_scan_cuda_oflex.py, dropin/selective_scan_cuda.py (mamba_ssm's
+      module, with the z gate) — the reference extension modules' `fwd` / `bwd` functions; `install_dropin()` registers them
+      in sys.modules so that the reference's own `model/gm/csms6s.py` picks them up unchanged.
   b2  functional.py — SelectiveScanCore/Oflex, CrossScan[_k], CrossMerge[_k] autograd Functions.
   b3  modules.py — SS2D, GroupMambaLayer (and the FFNs next to them: PVT2FFN, custom_ffn) with the reference's state_dict.
 Underneath: ops.py -> _lib.py (ctypes) -> libss2d_b200.so (csrc/*.cu, C ABI in include/ss2d_b200.h).
@@ -38,10 +38,12 @@ def graphed(module, sample_args, num_warmup_iters: int = 3):
 
 
 def install_dropin() -> None:
-    """Make `import selective_scan_cuda_core` / `selective_scan_cuda_oflex` resolve to this package's modules
-    (the reference imports them at module import time inside try/except: model/gm/csms6s.py:209-220)."""
+    """Make `import selective_scan_cuda_core` / `selective_scan_cuda_oflex` / `selective_scan_cuda` (mamba_ssm's module)
+    resolve to this package's modules (the reference imports them at module import time inside try/except:
+    model/gm/csms6s.py:209-220)."""
     import sys
 
-    from .dropin import selective_scan_cuda_core, selective_scan_cuda_oflex
+    from .dropin import selective_scan_cuda, selective_scan_cuda_core, selective_scan_cuda_oflex
     sys.modules["selective_scan_cuda_core"] = selective_scan_cuda_core
     sys.modules["selective_scan_cuda_oflex"] = selective_scan_cuda_oflex
+    sys.modules["selective_scan_cuda"] = selective_scan_cuda

@@ -22,6 +22,7 @@ MAX_DSTATE = 256
 EXPORTS = [
     "ss2d_scan_fwd", "ss2d_scan_ckpt_floats", "ss2d_scan_bwd", "ss2d_scan_bwd_workspace_bytes",
     "ss2d_scan_fwd_state", "ss2d_scan_bwd_state",
+    "ss2d_scan_fwd_gated", "ss2d_scan_bwd_gated", "ss2d_scan_bwd_gated_workspace_bytes",
     "ss2d_cross_scan", "ss2d_cross_merge", "ss2d_out_gate_fwd", "ss2d_out_gate_bwd",
     "ss2d_out_gate_bwd_partials", "ss2d_group_gate_fwd", "ss2d_group_gate_bwd", "ss2d_out_gate_max_width", "ss2d_wgrad_ts", "ss2d_wgrad_ts_workspace_bytes",
     "ss2d_layernorm_fwd", "ss2d_layernorm_bwd", "ss2d_layernorm_bwd_partials",
@@ -89,6 +90,13 @@ def lib() -> ctypes.CDLL:
     L.ss2d_scan_fwd_state.restype = ctypes.c_int
     L.ss2d_scan_bwd_state.argtypes = [dp, vp, vp, fp, vp, vp, fp, fp, fp, vp, fp, fp, vp, vp, fp, fp, fp, fp, fp, fp, vp, sz, vp]
     L.ss2d_scan_bwd_state.restype = ctypes.c_int
+    L.ss2d_scan_fwd_gated.argtypes = [dp, vp, vp, fp, vp, vp, fp, fp, fp, vp, vp, vp, fp, fp, vp]
+    L.ss2d_scan_fwd_gated.restype = ctypes.c_int
+    L.ss2d_scan_bwd_gated.argtypes = [dp, vp, vp, fp, vp, vp, fp, fp, fp, vp, vp, vp, fp, fp, vp, vp, fp, fp, fp, fp, fp, vp, fp,
+                                      vp, sz, vp]
+    L.ss2d_scan_bwd_gated.restype = ctypes.c_int
+    L.ss2d_scan_bwd_gated_workspace_bytes.argtypes = [dp, ctypes.c_int]
+    L.ss2d_scan_bwd_gated_workspace_bytes.restype = sz
     L.ss2d_scan_bwd_workspace_bytes.argtypes = [dp, ctypes.c_int]
     L.ss2d_scan_bwd_workspace_bytes.restype = sz
     ip = ctypes.POINTER(ctypes.c_int32)
@@ -169,7 +177,7 @@ def check(rc: int, what: str) -> None:
 
 
 def test_force_path(policy: int) -> None:
-    """TEST HOOK (include/ss2d_b200.h: ss2d_test_force_path): 0 automatic, 1 / 2 lane-owns-row forward (32 / 16-row warps), 3 the 8-row-warp forward (and the tiled FFN stencil), 4 the segmented forward."""
+    """TEST HOOK (include/ss2d_b200.h: ss2d_test_force_path): 0 automatic, 1 / 2 lane-owns-row forward (32 / 16-row warps), 3 the 8-row-warp forward (and the tiled FFN stencil), 4 the segmented forward; policy + 8: the same, with the output gate never fused into scan_fwdr."""
     rc = lib().ss2d_test_force_path(int(policy))
     if rc != 0:
         raise RuntimeError("ss2d_test_force_path(%d) -> %d" % (policy, rc))

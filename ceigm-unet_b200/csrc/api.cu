@@ -13,7 +13,12 @@
 
 namespace ss2d {
 cudaError_t scan_fwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream);
-bool scan_fwdr_try(const ScanParams& p, const ScanState& st, cudaStream_t stream, cudaError_t* err);
+bool scan_fwdr_try(const ScanParams& p, const ScanState& st, const ScanGate& gt, cudaStream_t stream, cudaError_t* err,
+                   bool* gated);
+// output gate passes (scan_gate.cu): out_z = y silu(z); dy = dout_z silu(z) (fp32, dense (batch, dim, L)), dz
+cudaError_t scan_gate_fwd_launch(const ss2d_scan_desc* d, const void* y, const void* z, void* out_z, cudaStream_t s);
+cudaError_t scan_gate_bwd_launch(const ss2d_scan_desc* d, const void* dout_z, const void* z, const void* y, float* dy, void* dz,
+                                 cudaStream_t s);
 constexpr int kDwnMaxSeg = 4;
 struct DwnSegs { int nseg; int cbeg[kDwnMaxSeg + 1]; int k[kDwnMaxSeg]; const float* w[kDwnMaxSeg]; const float* b[kDwnMaxSeg]; };
 cudaError_t dwnhwc_stencil_launch(const void* x, const void* aux, void* y, const DwnSegs& sg, int flip, int epi, int B, int H,
@@ -95,7 +100,8 @@ thread_local char g_cuda_err[256] = "";
 // process-wide: the autograd engine launches the backward kernels from its own per-device threads
 static std::atomic<int64_t> g_launches{0};
 static std::atomic<int> g_path_policy{0};
-int scan_path_policy() { return g_path_policy.load(std::memory_order_relaxed); }
+int scan_path_policy() { return g_path_policy.load(std::memory_order_relaxed) & 7; }
+bool scan_gate_fusion() { return !(g_path_policy.load(std::memory_order_relaxed) & 8); }
 
 static int cuda_fail(cudaError_t e) {
   snprintf(g_cuda_err, sizeof(g_cuda_err), "%s: %s", cudaGetErrorName(e), cudaGetErrorString(e));
@@ -222,9 +228,19 @@ int ss2d_scan_fwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
   return ss2d_scan_fwd_state(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, nullptr, out, ckpt, last_state, stream);
 }
 
-int ss2d_scan_fwd_state(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
-                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, void* out,
-                        float* ckpt, float* last_state, ss2d_stream_t stream) {
+}  // extern "C"
+
+static int bwd_check(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                     const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* dout,
+                     const float* dlast, const float* ckpt, void* du, void* ddelta, float* dA, float* dB, float* dC,
+                     float* dD, float* ddelta_bias, float* dh0, void* workspace, size_t workspace_bytes);
+
+// The forward of ss2d_scan_fwd_state; gt.z != nullptr offers the output gate to scan_fwdr when the call is one state pass,
+// and *gated reports whether the scan kernel wrote out_z.
+static int scan_fwd_impl(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                         const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, void* out, float* ckpt,
+                         float* last_state, const ScanGate& gt, ss2d_stream_t stream, bool* gated) {
+  *gated = false;
   int rc = validate(d);
   if (rc != SS2D_OK) return rc;
   if (!u || !delta || !A || !Bmat || !Cmat || (!out && !ckpt && !last_state)) return SS2D_ERR_NULL_POINTER;
@@ -252,13 +268,84 @@ int ss2d_scan_fwd_state(const ss2d_scan_desc* d, const void* u, const void* delt
     cudaError_t e;
     if (use_par(p)) {      // d_state = 1: lean fp32 kernels (scan_n1.cu) when eligible, else the generic parallel-along-L ones
       if (!scan_n1_fwd_try(p, st, static_cast<cudaStream_t>(stream), &e)) e = scan_par_fwd_dispatch(p, st, static_cast<cudaStream_t>(stream));
-    } else if (!scan_fwdr_try(p, st, static_cast<cudaStream_t>(stream), &e)) {     // lane-owns-row fast path (scan_fwdr.cu)
+    } else if (!scan_fwdr_try(p, st, n_passes(d->dstate) == 1 ? gt : ScanGate{nullptr, nullptr},
+                              static_cast<cudaStream_t>(stream), &e, gated)) {     // lane-owns-row fast path (scan_fwdr.cu)
       e = scan_fwd_dispatch(p, st, static_cast<cudaStream_t>(stream));
     }
     if (e != cudaSuccess) return cuda_fail(e);
     ++g_launches;
   }
   return SS2D_OK;
+}
+
+extern "C" {
+
+int ss2d_scan_fwd_state(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, void* out,
+                        float* ckpt, float* last_state, ss2d_stream_t stream) {
+  bool gated;
+  return scan_fwd_impl(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, h0, out, ckpt, last_state, ScanGate{nullptr, nullptr},
+                       stream, &gated);
+}
+
+// NULL / alignment / layout checks shared by the gated calls
+static int gate_check(const ss2d_scan_desc* d, const void* z, const void* y, const void* g) {
+  int rc = validate(d);
+  if (rc != SS2D_OK) return rc;
+  if (!z || !y || !g) return SS2D_ERR_NULL_POINTER;
+  if (d->u_dim_modulo > 0) return SS2D_ERR_UNSUPPORTED;
+  if (!aligned(z, esize(d->io_dtype)) || !aligned(y, esize(d->out_dtype)) || !aligned(g, esize(d->out_dtype)))
+    return SS2D_ERR_ALIGNMENT;
+  return SS2D_OK;
+}
+
+int ss2d_scan_fwd_gated(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* z, void* out,
+                        void* out_z, float* ckpt, float* last_state, ss2d_stream_t stream) {
+  int rc = gate_check(d, z, out, out_z);
+  if (rc != SS2D_OK) return rc;
+  bool gated = false;
+  rc = scan_fwd_impl(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, h0, out, ckpt, last_state, ScanGate{z, out_z}, stream, &gated);
+  if (rc != SS2D_OK || gated) return rc;
+  // every other forward path: y is final only after the call's last kernel (segmented fix-up, last state pass)
+  const cudaError_t e = scan_gate_fwd_launch(d, out, z, out_z, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  ++g_launches;
+  return SS2D_OK;
+}
+
+size_t ss2d_scan_bwd_gated_workspace_bytes(const ss2d_scan_desc* d, int have_ckpt) {
+  if (validate(d) != SS2D_OK) return 0;
+  return ss2d_scan_bwd_workspace_bytes(d, have_ckpt) + (size_t)d->batch * d->dim * d->seqlen * sizeof(float);
+}
+
+int ss2d_scan_bwd_gated(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* z,
+                        const void* out, const void* dout_z, const float* dlast, const float* ckpt, void* du, void* ddelta,
+                        float* dA, float* dB, float* dC, float* dD, float* ddelta_bias, void* dz, float* dh0, void* workspace,
+                        size_t workspace_bytes, ss2d_stream_t stream) {
+  int rc = gate_check(d, z, out, dout_z);
+  if (rc != SS2D_OK) return rc;
+  if (!dz) return SS2D_ERR_NULL_POINTER;
+  if (!aligned(dz, esize(d->io_dtype))) return SS2D_ERR_ALIGNMENT;
+  const size_t inner_bytes = ss2d_scan_bwd_workspace_bytes(d, ckpt != nullptr);
+  if (!workspace || workspace_bytes < ss2d_scan_bwd_gated_workspace_bytes(d, ckpt != nullptr) || !aligned(workspace, 16))
+    return SS2D_ERR_WORKSPACE;
+  // dy lives behind the ungated workspace (whose size is a multiple of 16 bytes); the ungated backward reads it as an fp32
+  // dout with dense strides, which the workspace query does not depend on
+  float* dy = reinterpret_cast<float*>(static_cast<char*>(workspace) + inner_bytes);
+  ss2d_scan_desc di = *d;
+  di.out_dtype = SS2D_F32;
+  di.out_batch_stride = (int64_t)d->dim * d->seqlen;
+  di.out_dim_stride = d->seqlen;
+  rc = bwd_check(&di, u, delta, A, Bmat, Cmat, Dvec, delta_bias, h0, dy, dlast, ckpt, du, ddelta, dA, dB, dC, dD, ddelta_bias, dh0,
+                 workspace, inner_bytes);
+  if (rc != SS2D_OK) return rc;
+  cudaError_t e = scan_gate_bwd_launch(d, dout_z, z, out, dy, dz, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  ++g_launches;
+  return ss2d_scan_bwd_state(&di, u, delta, A, Bmat, Cmat, Dvec, delta_bias, h0, dy, dlast, ckpt, du, ddelta, dA, dB, dC, dD,
+                             ddelta_bias, dh0, workspace, inner_bytes, stream);
 }
 
 int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
@@ -269,11 +356,13 @@ int ss2d_scan_bwd(const ss2d_scan_desc* d, const void* u, const void* delta, con
                              dC, dD, ddelta_bias, nullptr, workspace, workspace_bytes, stream);
 }
 
-int ss2d_scan_bwd_state(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
-                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* dout,
-                        const float* dlast, const float* ckpt, void* du, void* ddelta, float* dA, float* dB, float* dC,
-                        float* dD, float* ddelta_bias, float* dh0, void* workspace, size_t workspace_bytes,
-                        ss2d_stream_t stream) {
+}  // extern "C"
+
+// argument checks of ss2d_scan_bwd_state, also run by ss2d_scan_bwd_gated before it launches anything
+static int bwd_check(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                     const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* dout,
+                     const float* dlast, const float* ckpt, void* du, void* ddelta, float* dA, float* dB, float* dC,
+                     float* dD, float* ddelta_bias, float* dh0, void* workspace, size_t workspace_bytes) {
   int rc = validate(d);
   if (rc != SS2D_OK) return rc;
   if (!u || !delta || !A || !Bmat || !Cmat || !dout || !du || !ddelta || !dA || !dB || !dC) return SS2D_ERR_NULL_POINTER;
@@ -288,6 +377,19 @@ int ss2d_scan_bwd_state(const ss2d_scan_desc* d, const void* u, const void* delt
       !aligned(du, esize(d->io_dtype)) || !aligned(ddelta, esize(d->io_dtype)) || !aligned(dA, 4) ||
       !aligned(dB, bc_al) || !aligned(dC, bc_al) || !aligned(h0, 16) || !aligned(dlast, 16) || !aligned(dh0, 16))
     return SS2D_ERR_ALIGNMENT;
+  return SS2D_OK;
+}
+
+extern "C" {
+
+int ss2d_scan_bwd_state(const ss2d_scan_desc* d, const void* u, const void* delta, const float* A, const void* Bmat,
+                        const void* Cmat, const float* Dvec, const float* delta_bias, const float* h0, const void* dout,
+                        const float* dlast, const float* ckpt, void* du, void* ddelta, float* dA, float* dB, float* dC,
+                        float* dD, float* ddelta_bias, float* dh0, void* workspace, size_t workspace_bytes,
+                        ss2d_stream_t stream) {
+  int rc = bwd_check(d, u, delta, A, Bmat, Cmat, Dvec, delta_bias, h0, dout, dlast, ckpt, du, ddelta, dA, dB, dC, dD, ddelta_bias,
+                     dh0, workspace, workspace_bytes);
+  if (rc != SS2D_OK) return rc;
   cudaStream_t cst = static_cast<cudaStream_t>(stream);
   float* ws = static_cast<float*>(workspace);
   const int nmax = d->dstate < kStatesPerPass ? d->dstate : kStatesPerPass;
@@ -667,7 +769,7 @@ int64_t ss2d_launch_count(int reset) {
   return reset ? g_launches.exchange(0) : g_launches.load();
 }
 int32_t ss2d_test_force_path(int32_t policy) {
-  if (policy < 0 || policy > 4) return SS2D_ERR_BAD_SHAPE;
+  if (policy < 0 || (policy & 7) > 4 || policy > 12) return SS2D_ERR_BAD_SHAPE;
   g_path_policy.store(policy, std::memory_order_relaxed);
   return SS2D_OK;
 }

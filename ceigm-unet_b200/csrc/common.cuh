@@ -38,6 +38,12 @@ __device__ __forceinline__ float softplus20_grad(float x) {
   const float e = ex2f(-x * kLog2e);
   return x > 20.f ? 1.f : __fdividef(1.f, 1.f + e);
 }
+// silu(x) = x sigmoid(x) and its derivative s (1 + x (1 - s)), s = sigmoid(x)
+__device__ __forceinline__ float silu_f(float x) { return __fdividef(x, 1.f + ex2f(-x * kLog2e)); }
+__device__ __forceinline__ float silu_grad_f(float x) {
+  const float s = __fdividef(1.f, 1.f + ex2f(-x * kLog2e));
+  return s * (1.f + x * (1.f - s));
+}
 
 // ---- dtype-erased 4-element loads/stores (runtime dtype: the math is always fp32 from shared memory) ----
 __device__ __forceinline__ size_t dtype_size(int dt) { return dt == SS2D_F32 ? 4 : 2; }

@@ -55,12 +55,6 @@ __device__ __forceinline__ float merge_k(const float* __restrict__ ys, int K, in
   return acc;
 }
 
-__device__ __forceinline__ float silu_f(float x) { return __fdividef(x, 1.f + ex2f(-x * kLog2e)); }
-__device__ __forceinline__ float silu_grad_f(float x) {
-  const float s = __fdividef(1.f, 1.f + ex2f(-x * kLog2e));
-  return s * (1.f + x * (1.f - s));
-}
-
 // Loads the merged tile y[d][px] of batch b into s_y[d * 33 + px]. s_pix[px] = natural flattened index of the tile's pixel px
 // (or -1). A thread keeps ONE pixel (px = tid % 32: its natural / transposed offsets are computed once per tile, not once per
 // element) and walks the channels d = tid / 32, + 8, ...: a warp reads 32 pixels of one channel plane — contiguous runs of 32 /

@@ -42,10 +42,15 @@ struct FwdrShape {
 
 // STATE (whole-row mode only): the rows start from st.h0 instead of 0. Segmented mode scans every segment from zero and
 // leaves h0 to the carry / fix-up kernels.
-template <int NS, int R, bool SOFTPLUS, bool SEG, bool STATE>
+// GATE (whole-row mode only, ss2d_scan_fwd_gated): the store step also writes gt.out_z = y * silu(z). z is not staged in the
+// ring: a fifth tile would take the 32-row CTA from 97 to 129 KB of shared memory, one CTA per SM instead of two. The lane
+// that stores a 4-position group reads its z quad from global memory one group pair ahead instead. The GATE instantiations
+// take h0 from st.h0 when it is set (a runtime test once per row), so that their names keep STATE = false.
+template <int NS, int R, bool SOFTPLUS, bool SEG, bool GATE, bool STATE>
 __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams p, const __grid_constant__ FwdrMaps maps,
                                                                const int nrb, const int nwb, const int nseg_arg, const int tps,
-                                                               const ScanState st) {
+                                                               const ScanState st, const ScanGate gt) {
+  static_assert(!(GATE && (SEG || STATE)), "the gated instantiations are whole-row and read h0 at run time");
   const int nseg = SEG ? nseg_arg : 1;                     // compile-time 1 in the whole-row instantiation
   using S = FwdrShape<R>;
   constexpr int ROWS = S::ROWS;
@@ -101,7 +106,7 @@ __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams 
   for (int j = 0; j < NS; ++j) {
     const int n = j * R + q;
     A2[j] = (valid && n < p.N) ? p.A[(int64_t)d * p.A_ld + n] * kLog2e : 0.f;
-    h[j] = (STATE && valid && n < p.N) ? st.h0[state_slot(p, b, d, n)] : 0.f;
+    h[j] = ((STATE || (GATE && st.h0 != nullptr)) && valid && n < p.N) ? st.h0[state_slot(p, b, d, n)] : 0.f;
   }
   const float bias = (valid && p.bias) ? p.bias[d] : 0.f;
   const float Dd = (valid && p.Dv) ? p.Dv[d] : 0.f;
@@ -144,6 +149,16 @@ __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams 
         f4_at(dum_n, e) = x * f4_at(um_n, e);
       }
     };
+    // GATE: z quads of the group pair being computed (zc) and of the next one (zn), in memory order like y4
+    const float* zrow = GATE ? static_cast<const float*>(gt.z) + out_ro : nullptr;
+    float4 zc[2], zn[2];
+    auto load_z = [&](int pos) -> float4 {      // scan position of the quad's first element
+      return pos < L ? __ldg(reinterpret_cast<const float4*>(zrow + (REVV ? L - 4 - pos : pos))) : make_float4(0.f, 0.f, 0.f, 0.f);
+    };
+    if constexpr (GATE) {
+#pragma unroll
+      for (int k = 0; k < 2; ++k) zn[k] = load_z((k * R + q) * 4);
+    }
     mbar_wait(&full[0], 0);
     activate(st_dl(0), st_u(0), 0, min(FR_LT, L - tb * FR_LT));
     for (int t = tb; t < ntiles; ++t) {
@@ -159,6 +174,13 @@ __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams 
       for (int i4 = 0; i4 < FR_LT / 4; i4 += 2 * R) {
         const bool last_pair = i4 == FR_LT / 4 - 2 * R;
         if (last_pair && more) mbar_wait(&full[sn], ((t + 1 - tb) / FR_STAGES) & 1);    // requested one tile ago: there by now
+        if constexpr (GATE) {
+#pragma unroll
+          for (int k = 0; k < 2; ++k) {
+            zc[k] = zn[k];
+            zn[k] = load_z(l0 + (i4 + k * R + q) * 4 + 8 * R);
+          }
+        }
 #pragma unroll
         for (int k = 0; k < 2; ++k) {
           const int ii = i4 + k * R;
@@ -208,6 +230,11 @@ __global__ void __launch_bounds__(FR_NW * 32) scan_fwdr_kernel(const ScanParams 
           if (REVV) y4 = make_float4(y4.w, y4.z, y4.y, y4.x);
           const int mpos = REVV ? L - 4 - (l0 + cm) : l0 + cm;    // memory position of the group's first element
           if (do_out && cm < len) *reinterpret_cast<float4*>(outp + mpos) = y4;
+          if constexpr (GATE) {
+            const float4 zq = zc[k];
+            const float4 g4 = make_float4(y4.x * silu_f(zq.x), y4.y * silu_f(zq.y), y4.z * silu_f(zq.z), y4.w * silu_f(zq.w));
+            if (do_out && cm < len) *reinterpret_cast<float4*>(static_cast<float*>(gt.out_z) + out_ro + mpos) = g4;
+          }
         }
       }
       // state checkpoint at the end of the tile, for the backward's recompute: ckpt[b][d][tile][n]
@@ -256,11 +283,11 @@ static bool fwdr_maps(const ScanParams& p, FwdrMaps* m) {
          make_tmap(&m->B, p.Bm, 4, d4, s4B, 16, R > 1) && make_tmap(&m->C, p.Cm, 4, d4, s4C, 16, R > 1);
 }
 
-template <int NS, int R, bool SOFTPLUS, bool SEG, bool STATE>
+template <int NS, int R, bool SOFTPLUS, bool SEG, bool STATE, bool GATE = false>
 static cudaError_t launch_fwdr(const ScanParams& p, const FwdrMaps& maps, const ScanState& st, cudaStream_t stream, int nseg = 1,
-                               int tps = 0) {
+                               int tps = 0, const ScanGate& gt = ScanGate{nullptr, nullptr}) {
   using S = FwdrShape<R>;
-  auto kern = scan_fwdr_kernel<NS, R, SOFTPLUS, SEG, STATE>;
+  auto kern = scan_fwdr_kernel<NS, R, SOFTPLUS, SEG, GATE, STATE>;
   static PerDeviceOnce once;
   cudaError_t e = func_attr_once(once, reinterpret_cast<const void*>(kern), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::smem_bytes);
   if (e != cudaSuccess) return e;
@@ -268,7 +295,7 @@ static cudaError_t launch_fwdr(const ScanParams& p, const FwdrMaps& maps, const 
   const int nrb = (p.dpg + S::ROWS - 1) / S::ROWS;
   const long long nwb = (long long)nrb * p.G * p.batch * nseg;
   if (tps <= 0) tps = (p.L + FR_LT - 1) / FR_LT;
-  kern<<<(unsigned)((nwb + FR_NW - 1) / FR_NW), FR_NW * 32, S::smem_bytes, stream>>>(p, maps, nrb, (int)nwb, nseg, tps, st);
+  kern<<<(unsigned)((nwb + FR_NW - 1) / FR_NW), FR_NW * 32, S::smem_bytes, stream>>>(p, maps, nrb, (int)nwb, nseg, tps, st, gt);
   return cudaGetLastError();
 }
 
@@ -451,10 +478,23 @@ static cudaError_t fwdr_launch_all(const ScanParams& p, const FwdrMaps& maps, co
   return cudaGetLastError();
 }
 
-int scan_path_policy();     // api.cu
+// whole-row gated launch: the z / out_z pointers checked by the caller, h0 read at run time
+static cudaError_t fwdr_launch_gated(const ScanParams& p, const FwdrMaps& maps, const ScanState& st, const ScanGate& gt,
+                                     cudaStream_t stream, bool r1) {
+  if (r1) return p.softplus ? launch_fwdr<16, 1, true, false, false, true>(p, maps, st, stream, 1, 0, gt)
+                            : launch_fwdr<16, 1, false, false, false, true>(p, maps, st, stream, 1, 0, gt);
+  return p.softplus ? launch_fwdr<8, 2, true, false, false, true>(p, maps, st, stream, 1, 0, gt)
+                    : launch_fwdr<8, 2, false, false, false, true>(p, maps, st, stream, 1, 0, gt);
+}
 
-// Returns true when the fast path took the call (*err holds the launch status).
-bool scan_fwdr_try(const ScanParams& p, const ScanState& st, cudaStream_t stream, cudaError_t* err) {
+int scan_path_policy();     // api.cu
+bool scan_gate_fusion();    // api.cu: false when the test hook keeps the gate of a gated call in its own pass
+
+// Returns true when the fast path took the call (*err holds the launch status). gt: the output gate of a gated call
+// (gt.z == nullptr otherwise); *gated tells whether the launch wrote out_z too (whole-row mode, z / out_z 16-byte aligned).
+bool scan_fwdr_try(const ScanParams& p, const ScanState& st, const ScanGate& gt, cudaStream_t stream, cudaError_t* err,
+                   bool* gated) {
+  *gated = false;
   if (!p.tma_ok || p.N <= 4 || p.N > 16 || p.accum || p.io_dtype != SS2D_F32 || p.out_dtype != SS2D_F32) return false;
   if (p.u_mod > 0 && p.u_mod % p.dpg != 0) return false;
   for (int g = 0; g < p.G; ++g) {
@@ -491,6 +531,11 @@ bool scan_fwdr_try(const ScanParams& p, const ScanState& st, cudaStream_t stream
   const bool r1 = nseg == 1 && (policy == 0 ? wb1 >= need : policy == 1);
   FwdrMaps maps;
   if (!(r1 ? fwdr_maps<1>(p, &maps) : fwdr_maps<2>(p, &maps))) return false;
+  if (gt.z && scan_gate_fusion() && nseg == 1 && !(reinterpret_cast<uintptr_t>(gt.z) & 15) && !(reinterpret_cast<uintptr_t>(gt.out_z) & 15)) {
+    *gated = true;              // out's strides (shared by z / out_z) are multiples of 4: checked above
+    *err = fwdr_launch_gated(p, maps, st, gt, stream, r1);
+    return true;
+  }
   *err = st.h0 ? fwdr_launch_all<true>(p, maps, st, stream, r1, nseg, tps) : fwdr_launch_all<false>(p, maps, st, stream, r1, nseg, tps);
   return true;
 }

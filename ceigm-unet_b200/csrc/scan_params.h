@@ -56,6 +56,12 @@ struct ScanState {
   const float* dlast;
   float* dh0;
 };
+// Output gate of ss2d_scan_fwd_gated, a separate argument of the scan_fwdr kernels for the same reason: out_z = out * silu(z),
+// both fp32 with out's strides. The GATE instantiations read it; the others are passed zeros.
+struct ScanGate {
+  const void* z;
+  void* out_z;
+};
 // backward: the STATE instantiation runs when any of the three pointers is set
 inline bool has_state(const ScanState& st) { return st.h0 || st.dlast || st.dh0; }
 

@@ -66,29 +66,32 @@ class SelectiveScanOflex(torch.autograd.Function):
 
 
 class _SelectiveScanState(torch.autograd.Function):
-    """selective_scan with an initial state and the final state as a differentiable output (see `selective_scan`)."""
+    """selective_scan with an initial state and the final state as a differentiable output (see `selective_scan`).
+    With a gate z the first output is out * silu(z); the ungated out is saved for the backward, as mamba_ssm does."""
 
     @staticmethod
-    def forward(ctx, u, delta, A, B, C, D, delta_bias, delta_softplus, h0):
+    def forward(ctx, u, delta, A, B, C, D, delta_bias, delta_softplus, h0, z=None):
         prob = ops.ScanProblem(u, delta, A, B, C, D, delta_bias, delta_softplus, out_float=False)
-        out, x = prob.forward(want_state=True, h0=h0)
+        res = prob.forward(want_state=True, h0=h0, z=z)
+        x = res[1]
         last = x[:, :, 0, 1::2].contiguous()
         ctx.delta_softplus = delta_softplus
         ctx.has_h0 = h0 is not None
-        ctx.save_for_backward(u, delta, A, B, C, D, delta_bias, h0, x)
-        return out, last
+        ctx.save_for_backward(u, delta, A, B, C, D, delta_bias, h0, x, z, res[0] if z is not None else None)
+        return (res[0] if z is None else res[2]), last
 
     @staticmethod
     def backward(ctx, dout, dlast):
-        u, delta, A, B, C, D, delta_bias, h0, x = ctx.saved_tensors
+        u, delta, A, B, C, D, delta_bias, h0, x, z, y = ctx.saved_tensors
         prob = ops.ScanProblem(u, delta, A, B, C, D, delta_bias, ctx.delta_softplus, out_float=False)
-        du, ddelta, dA, dB, dC, dD, dbias, dh0 = prob.backward(dout.contiguous(), x, h0=h0, dlast=dlast,
-                                                              want_dh0=ctx.needs_input_grad[8])
-        return du, ddelta, dA, dB, dC, dD, dbias, None, dh0
+        grads = prob.backward(dout.contiguous(), x, h0=h0, dlast=dlast, want_dh0=ctx.needs_input_grad[8], z=z, out=y)
+        du, ddelta, dA, dB, dC, dD, dbias = grads[:7]
+        dz = grads[7] if z is not None else None
+        return du, ddelta, dA, dB, dC, dD, dbias, None, grads[-1], dz
 
 
 def selective_scan(u, delta, A, B, C, D=None, delta_bias=None, delta_softplus=False, initial_state=None,
-                   return_last_state=False):
+                   return_last_state=False, *, z=None):
     """Differentiable selective scan with state passing, in the reference extension's SCAN layout and dtype rules:
     u, delta (B, Dt, L) and B, C (B, G, N, L) or (B, N, L) of one dtype (fp32 / fp16 / bf16), A (Dt, N) fp32, D and
     delta_bias (Dt) fp32 or None; out has u's dtype.
@@ -97,8 +100,10 @@ def selective_scan(u, delta, A, B, C, D=None, delta_bias=None, delta_softplus=Fa
 
     initial_state: (B, Dt, N) fp32 or None; gradients flow to it. return_last_state: also return h_(L-1) as a (B, Dt, N)
     fp32 tensor whose gradient flows back through the scan, so a sequence split into pieces can be chained call by call.
+    z: optional (B, Dt, L) gate of u's dtype (mamba_ssm's selective_scan_fn z): the result is then out * silu(z), with the
+    gate applied inside the library (gradients flow to z too).
     Under torch.use_deterministic_algorithms(True) every gradient is bit-identical from call to call."""
-    out, last = _SelectiveScanState.apply(u, delta, A, B, C, D, delta_bias, bool(delta_softplus), initial_state)
+    out, last = _SelectiveScanState.apply(u, delta, A, B, C, D, delta_bias, bool(delta_softplus), initial_state, z)
     return (out, last) if return_last_state else out
 
 

@@ -122,16 +122,27 @@ class ScanProblem:
             t = t.clone()
         return t
 
+    def _gate_arg(self, t: torch.Tensor, name: str, dtype) -> torch.Tensor:
+        """z / out / dout of a gated call: a (batch, dim, seqlen) CUDA tensor of `dtype`, made contiguous (the C ABI gives the
+        gate operands out's strides)."""
+        _require(not self.u_mod, "the output gate needs one dout plane per channel (u_mod == 0)")
+        _require(t.is_cuda and t.dtype == dtype, f"{name} must be a CUDA tensor of dtype {dtype}")
+        _require(tuple(t.shape) == (self.batch, self.dim, self.L), f"{name} must be (batch, dim, seqlen)")
+        return t.contiguous()
+
     # ---- forward ----
-    def forward(self, want_state: bool = True, h0: Optional[torch.Tensor] = None):
+    def forward(self, want_state: bool = True, h0: Optional[torch.Tensor] = None, z: Optional[torch.Tensor] = None):
         """-> (out (B, Dt, L), x). `x` has the reference's shape convention (B, Dt, 1, 2N): x[:, :, -1, 1::2] is the
         final state; the chunk checkpoints for the backward live in front of it in the same storage.
         h0: optional (B, Dt, N) fp32 state before the first position (default zeros); a backward of this forward's `x` must
-        be given the same h0."""
+        be given the same h0.
+        z: optional (B, Dt, L) gate of u's dtype: a third value out_z = out * silu(z) (out's dtype) is returned."""
         h0 = self._state_arg(h0, "h0")
+        if z is not None:
+            z = self._gate_arg(z, "z", self.u.dtype)
         if self._upcast:
-            out32, x = self._fp32_twin().forward(want_state, h0)
-            return out32.to(self.out_dtype), x
+            res = self._fp32_twin().forward(want_state, h0, None if z is None else z.float())
+            return (res[0].to(self.out_dtype), res[1]) + tuple(r.to(self.out_dtype) for r in res[2:])
         d, dev = self.desc, self.delta.device
         out = torch.empty((self.batch, self.dim, self.L), dtype=self.out_dtype, device=dev)
         d.out_batch_stride, d.out_dim_stride = out.stride(0), out.stride(1)
@@ -143,8 +154,14 @@ class ScanProblem:
             x = buf[head:].view(self.batch, self.dim, 1, 2 * self.N)
             last = x
             d.last_state_interleaved = 1
+        out_z = None
         with torch.cuda.device(dev):
-            if h0 is None:
+            if z is not None:
+                out_z = torch.empty_like(out)
+                rc = _lib.lib().ss2d_scan_fwd_gated(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
+                                                    _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(z), _ptr(out),
+                                                    _ptr(out_z), _ptr(ckpt), _ptr(last), _stream(dev))
+            elif h0 is None:
                 rc = _lib.lib().ss2d_scan_fwd(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
                                               _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(out), _ptr(ckpt),
                                               _ptr(last), _stream(dev))
@@ -153,7 +170,7 @@ class ScanProblem:
                                                     _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(out), _ptr(ckpt),
                                                     _ptr(last), _stream(dev))
         _lib.check(rc, "ss2d_scan_fwd")
-        return out, x
+        return (out, x) if z is None else (out, x, out_z)
 
     def _ckpt_from_x(self, x: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
         """Recover the checkpoint buffer that `forward` placed in front of `x` (None if x is foreign)."""
@@ -167,7 +184,7 @@ class ScanProblem:
 
     # ---- backward ----
     def backward(self, dout, x=None, h0: Optional[torch.Tensor] = None, dlast: Optional[torch.Tensor] = None,
-                 want_dh0: bool = False):
+                 want_dh0: bool = False, z: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None):
         """-> [du, ddelta, dA, dB, dC, dD, ddelta_bias] with the reference's dtypes (selective_scan.cpp:319-347):
         du/ddelta in u's dtype, dA/dD/ddelta_bias fp32, dB/dC accumulated in fp32 then cast to B's dtype.
 
@@ -175,20 +192,32 @@ class ScanProblem:
         the seven gradients are then bit-identical from call to call on the same GPU model (ss2d_scan_desc.deterministic).
 
         State passing: h0 is the forward's initial state (None: zeros), dlast the gradient of the final state (None: zeros).
-        With any of h0 / dlast / want_dh0 given, an eighth entry dh0 (B, Dt, N) fp32 (or None unless want_dh0) is appended."""
+        With any of h0 / dlast / want_dh0 given, an eighth entry dh0 (B, Dt, N) fp32 (or None unless want_dh0) is appended.
+
+        Output gate: with z (the forward's gate) and out (the forward's ungated output y, required with z), dout is the
+        gradient of out_z = out * silu(z), and dz (z's dtype) is appended after the seven gradients, before dh0."""
         d, dev = self.desc, self.delta.device
         dch = self.u_mod if self.u_mod else self.dim
         _require(dout.is_cuda and dout.dtype == self.out_dtype, "dout must be a CUDA tensor of out's dtype")
         _require(tuple(dout.shape) == (self.batch, dch, self.L), "dout must be (batch, dim, seqlen)")
         h0, dlast = self._state_arg(h0, "h0"), self._state_arg(dlast, "dlast")
         stateful = h0 is not None or dlast is not None or want_dh0
+        gated = z is not None
+        if gated:
+            _require(out is not None, "out (the forward's ungated output) is required with z")
+            z, out = self._gate_arg(z, "z", self.u.dtype), self._gate_arg(out, "out", self.out_dtype)
+            dout = self._gate_arg(dout, "dout", self.out_dtype)
         if self._upcast:
-            grads = self._fp32_twin().backward(dout.float(), x, h0, dlast, want_dh0)
+            grads = self._fp32_twin().backward(dout.float(), x, h0, dlast, want_dh0, z=None if z is None else z.float(),
+                                               out=None if out is None else out.float())
             du, ddelta, dA, dB, dC, dD, dbias = grads[:7]
             dB, dC = dB.to(self.B.dtype), dC.to(self.C.dtype)
             if self.squeeze_BC:
                 dB, dC = dB[:, 0], dC[:, 0]
-            return [du.to(self.u.dtype), ddelta.to(self.delta.dtype), dA, dB, dC, dD, dbias] + grads[7:]
+            rest = grads[7:]
+            if gated:
+                rest = [rest[0].to(self.u.dtype)] + rest[1:]
+            return [du.to(self.u.dtype), ddelta.to(self.delta.dtype), dA, dB, dC, dD, dbias] + rest
         if dout.stride(-1) != 1:                                  # csms6s.py:360-361 does the same before calling bwd
             dout = dout.contiguous()
         d.out_batch_stride, d.out_dim_stride = dout.stride(0), dout.stride(1)
@@ -224,11 +253,18 @@ class ScanProblem:
             d.grads_prezeroed = 0
         ckpt = self._ckpt_from_x(x)
         L = _lib.lib()
-        ws_bytes = int(L.ss2d_scan_bwd_workspace_bytes(ctypes.byref(d), 1 if ckpt is not None else 0))
+        ws_query = L.ss2d_scan_bwd_gated_workspace_bytes if gated else L.ss2d_scan_bwd_workspace_bytes
+        ws_bytes = int(ws_query(ctypes.byref(d), 1 if ckpt is not None else 0))
         ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=dev)
         dh0 = torch.empty((self.batch, self.dim, self.N), dtype=torch.float32, device=dev) if want_dh0 else None
+        dz = torch.empty_like(z) if gated else None
         with torch.cuda.device(dev):
-            if not stateful:
+            if gated:
+                rc = L.ss2d_scan_bwd_gated(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B), _ptr(self.C),
+                                           _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(z), _ptr(out), _ptr(dout), _ptr(dlast),
+                                           _ptr(ckpt), _ptr(du), _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD),
+                                           _ptr(dbias), _ptr(dz), _ptr(dh0), _ptr(ws), ctypes.c_size_t(ws_bytes), _stream(dev))
+            elif not stateful:
                 rc = L.ss2d_scan_bwd(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B),
                                      _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(dout), _ptr(ckpt), _ptr(du),
                                      _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD), _ptr(dbias), _ptr(ws),
@@ -243,7 +279,7 @@ class ScanProblem:
             dB, dC = dB.to(self.B.dtype), dC.to(self.C.dtype)
         if self.squeeze_BC:
             dB, dC = dB[:, 0], dC[:, 0]
-        grads = [du, ddelta, dA, dB, dC, dD, dbias]
+        grads = [du, ddelta, dA, dB, dC, dD, dbias] + ([dz] if gated else [])
         return grads + [dh0] if stateful else grads
 
 

@@ -156,6 +156,29 @@ int ss2d_scan_bwd_state(const ss2d_scan_desc* desc, const void* u, const void* d
                         void* du, void* ddelta, float* dA, float* dB, float* dC, float* dD, float* ddelta_bias,
                         float* dh0, void* workspace, size_t workspace_bytes, ss2d_stream_t stream);
 
+/* ---- output gate: the z argument of mamba_ssm's selective_scan_cuda --------------------------------------------
+ * The state calls above with the gate of the Mamba selective-scan contract applied to y = out:
+ *   out_z = y * silu(z),  silu(z) = z / (1 + exp(-z));
+ *   backward, given dout_z:  dy = dout_z * silu(z) (the ungated backward runs on dy),
+ *                            dz = dout_z * y * s * (1 + z (1 - s)),  s = sigmoid(z).
+ * z, dz: io dtype; out, out_z, dout_z: out dtype. All five use out's strides (desc->out_*_stride, innermost stride 1).
+ * out is still written: the backward reads y from it. NULL z / out / out_z / dout_z / dz: SS2D_ERR_NULL_POINTER; a pointer not
+ * aligned to its element size: SS2D_ERR_ALIGNMENT; u_dim_modulo > 0 (a shared dout plane cannot carry per-direction gates):
+ * SS2D_ERR_UNSUPPORTED. The gate terms are elementwise, so the gradients are deterministic exactly when the ungated ones are.
+ * workspace: ss2d_scan_bwd_gated_workspace_bytes(desc, ckpt != NULL) bytes, 16-byte aligned: the ungated size plus an fp32
+ * (batch, dim, L) buffer for dy. */
+int ss2d_scan_fwd_gated(const ss2d_scan_desc* desc, const void* u, const void* delta, const float* A,
+                        const void* Bmat, const void* Cmat, const float* Dvec, const float* delta_bias,
+                        const float* h0, const void* z, void* out, void* out_z, float* ckpt, float* last_state,
+                        ss2d_stream_t stream);
+size_t ss2d_scan_bwd_gated_workspace_bytes(const ss2d_scan_desc* desc, int have_ckpt);
+int ss2d_scan_bwd_gated(const ss2d_scan_desc* desc, const void* u, const void* delta, const float* A,
+                        const void* Bmat, const void* Cmat, const float* Dvec, const float* delta_bias,
+                        const float* h0, const void* z, const void* out, const void* dout_z, const float* dlast,
+                        const float* ckpt, void* du, void* ddelta, float* dA, float* dB, float* dC, float* dD,
+                        float* ddelta_bias, void* dz, float* dh0, void* workspace, size_t workspace_bytes,
+                        ss2d_stream_t stream);
+
 /* ---- stand-alone cross-scan / cross-merge (exact permutations; model/gm/csms6s.py:11-206) ----
  * cross_scan : x (batch, channels, H, W) -> xs (batch, K, channels, L), xs[:,k] in direction dirs[k].
  * cross_merge: ys (batch, K, channels, L) in scan order -> y (batch, channels, L) natural order,
@@ -362,6 +385,7 @@ int64_t ss2d_launch_count(int reset);
  * forward with 32-row warps; 2: the same with 16-row warps; 3: the 8-row-warp forward (scan_fwd.cu) — and, for
  * ss2d_dwnhwc_stencil, the tiled kernel where the single-segment 3 x 3 case would take the column walker (csrc/ffn_dw.cu);
  * 4: the segmented forward of small calls (sequence split over several warps + carry + fix-up kernels, csrc/scan_fwdr.cu).
+ * policy + 8: the same path, and ss2d_scan_fwd_gated never applies the gate inside scan_fwdr (its separate pass always runs).
  * Process-wide; returns SS2D_OK or SS2D_ERR_BAD_SHAPE. */
 int32_t ss2d_test_force_path(int32_t policy);
 
