@@ -490,7 +490,7 @@ int ss2d_out_gate_fwd(const float* ys, int32_t K, const float* ln_weight, const 
   if (batch <= 0 || D <= 0 || L <= 0 || K <= 0 || K > SS2D_MAX_GROUP_DIRS) return SS2D_ERR_BAD_SHAPE;
   if (transposed_mask && (H <= 0 || W <= 0 || (int64_t)H * W != L)) return SS2D_ERR_BAD_SHAPE;
   if (!dtype_ok(z_dtype) || !dtype_ok(out_dtype)) return SS2D_ERR_BAD_DTYPE;
-  if (D > epi_max_D(false)) return SS2D_ERR_UNSUPPORTED;
+  if (D > epi_max_D(false) || (ln_bias && !ln_weight)) return SS2D_ERR_UNSUPPORTED;
   cudaError_t e = out_gate_fwd_launch(ys, K, ln_weight, ln_bias, z, z_row_stride, z_act, out, mean_rstd, batch, D, L, eps,
                                       z_dtype, out_dtype, H, W, transposed_mask, static_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e);
@@ -509,7 +509,7 @@ int ss2d_out_gate_bwd(const float* ys, int32_t K, const float* ln_weight, const 
   if (dy_two_planes && (K < 2 || !transposed_mask)) return SS2D_ERR_UNSUPPORTED;      // patch tiles are what makes the second store cheap
   if (n_partials != epi_bwd_partials(batch, L)) return SS2D_ERR_WORKSPACE;
   if (!dtype_ok(z_dtype) || !dtype_ok(out_dtype)) return SS2D_ERR_BAD_DTYPE;
-  if (D > epi_max_D(true)) return SS2D_ERR_UNSUPPORTED;
+  if (D > epi_max_D(true) || (ln_bias && !ln_weight)) return SS2D_ERR_UNSUPPORTED;
   cudaError_t e = out_gate_bwd_launch(ys, K, ln_weight, ln_bias, z, z_row_stride, z_act, dout, mean_rstd, dy, dz,
                                       dz_row_stride, dln_weight_partial, dln_bias_partial, n_partials, batch, D, L,
                                       z_dtype, out_dtype, H, W, transposed_mask, dy_two_planes, static_cast<cudaStream_t>(stream));
@@ -518,14 +518,19 @@ int ss2d_out_gate_bwd(const float* ys, int32_t K, const float* ln_weight, const 
   return SS2D_OK;
 }
 
-static int group_gate_check(int32_t G, const int32_t* plane_of, int32_t batch, int32_t D, int32_t L, int32_t H, int32_t W,
-                            int32_t z_dtype, int32_t out_dtype, bool backward) {
+static int group_gate_check(int32_t G, const int32_t* plane_of, const float* ln_weight, const float* ln_bias, int32_t batch,
+                            int32_t D, int32_t L, int32_t H, int32_t W, int32_t z_dtype, int32_t out_dtype, bool backward) {
   if (!plane_of) return SS2D_ERR_NULL_POINTER;
   if (G <= 0 || G > SS2D_MAX_EPI_GROUPS || batch <= 0 || D <= 0 || L <= 0 || H <= 0 || W <= 0 || (int64_t)H * W != L)
     return SS2D_ERR_BAD_SHAPE;
-  for (int g = 0; g < G; ++g) if (plane_of[g] < 0 || plane_of[g] >= G) return SS2D_ERR_BAD_LAYOUT;
+  // a permutation: the backward writes group g's dy into plane plane_of[g], so two groups on one plane would race
+  unsigned seen = 0;
+  for (int g = 0; g < G; ++g) {
+    if (plane_of[g] < 0 || plane_of[g] >= G || ((seen >> plane_of[g]) & 1u)) return SS2D_ERR_BAD_LAYOUT;
+    seen |= 1u << plane_of[g];
+  }
   if (!dtype_ok(z_dtype) || !dtype_ok(out_dtype)) return SS2D_ERR_BAD_DTYPE;
-  if (D > epi_max_D(backward)) return SS2D_ERR_UNSUPPORTED;
+  if (D > epi_max_D(backward) || (ln_bias && !ln_weight)) return SS2D_ERR_UNSUPPORTED;
   return SS2D_OK;
 }
 
@@ -535,7 +540,7 @@ int ss2d_group_gate_fwd(const float* ys, int32_t G, const int32_t* plane_of, uin
                         int32_t batch, int32_t D, int32_t L, float eps, int32_t z_dtype, int32_t out_dtype, int32_t H,
                         int32_t W, ss2d_stream_t stream) {
   if (!ys || !z || !out) return SS2D_ERR_NULL_POINTER;
-  int rc = group_gate_check(G, plane_of, batch, D, L, H, W, z_dtype, out_dtype, false);
+  int rc = group_gate_check(G, plane_of, ln_weight, ln_bias, batch, D, L, H, W, z_dtype, out_dtype, false);
   if (rc != SS2D_OK) return rc;
   cudaError_t e = group_gate_fwd_launch(ys, G, plane_of, transposed_planes, ln_weight, ln_bias, z, z_row_stride, z_col0,
                                         z_group_stride, out, out_row_stride, mean_rstd, batch, D, L, eps, z_dtype, out_dtype,
@@ -553,7 +558,7 @@ int ss2d_group_gate_bwd(const float* ys, int32_t G, const int32_t* plane_of, uin
                         int32_t D, int32_t L, int32_t z_dtype, int32_t out_dtype, int32_t H, int32_t W,
                         ss2d_stream_t stream) {
   if (!ys || !z || !dout || !mean_rstd || !dy || !dz || !dln_weight_partial || !dln_bias_partial) return SS2D_ERR_NULL_POINTER;
-  int rc = group_gate_check(G, plane_of, batch, D, L, H, W, z_dtype, out_dtype, true);
+  int rc = group_gate_check(G, plane_of, ln_weight, ln_bias, batch, D, L, H, W, z_dtype, out_dtype, true);
   if (rc != SS2D_OK) return rc;
   if (n_partials != epi_bwd_partials(batch, L)) return SS2D_ERR_WORKSPACE;
   cudaError_t e = group_gate_bwd_launch(ys, G, plane_of, transposed_planes, ln_weight, ln_bias, z, z_row_stride, z_col0,

@@ -447,7 +447,7 @@ int gate_proj_tc_launch(const float* ys, int K, unsigned tmask, const float* lnw
   *cerr = cudaSuccess;
   if (!ys || (C > 0 && (!W || !out)) || (C == 0 && !g_out)) return SS2D_ERR_NULL_POINTER;
   if (batch <= 0 || L <= 0 || H <= 0 || Wd <= 0 || (int64_t)H * Wd != L) return SS2D_ERR_BAD_SHAPE;
-  if (!gate_proj_tc_supported(D, C, K, dtype)) return SS2D_ERR_UNSUPPORTED;
+  if (!gate_proj_tc_supported(D, C, K, dtype) || (lnb && !lnw)) return SS2D_ERR_UNSUPPORTED;
   const int esize = dtype == SS2D_F32 ? 4 : 2;
   auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
   if ((C > 0 && (!al16(out) || ((out_rs * esize) & 15))) || (z && (!al16(z) || ((z_rs * esize) & 15))) || (g_out && (!al16(g_out) || ((g_rs * esize) & 15))) ||

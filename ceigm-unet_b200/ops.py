@@ -364,7 +364,8 @@ def _row_stride(z, Bn, L) -> int:
 
 def out_gate_bwd(ys, ln_w, ln_b, z, z_act: bool, dout, stats, dz_out: Optional[torch.Tensor], hw=(0, 0), tmask: int = 0,
                  two_planes: bool = False):
-    """-> dy (B, D, L) fp32, dln_w, dln_b. dz is written into `dz_out` (a (B, L, D) uniformly strided view).
+    """-> dy (B, D, L) fp32, dln_w, dln_b. dz is written into `dz_out` (a (B, L, D) uniformly strided view), or not computed
+    when `dz_out` is None.
     two_planes (K > 1, tmask != 0): dy is (B, 2, D, L) — the merged gradient in natural and in transposed pixel order."""
     Bn, K, D, L = ys.shape
     dout = dout.contiguous()
@@ -374,7 +375,9 @@ def out_gate_bwd(ys, ln_w, ln_b, z, z_act: bool, dout, stats, dz_out: Optional[t
     zrs, zdt, dzrs = 0, _lib.SS2D_F32, 0
     if z is not None:
         zrs, zdt = _row_stride(z, Bn, L), _DT[z.dtype]
-        dzrs = _row_stride(dz_out, Bn, L)
+        if dz_out is not None:
+            _require(dz_out.dtype == z.dtype, "dz_out must have z's dtype (the kernel writes dz in it)")
+            dzrs = _row_stride(dz_out, Bn, L)
     with torch.cuda.device(ys.device):
         rc = _lib.lib().ss2d_out_gate_bwd(_ptr(ys), K, _ptr(ln_w), _ptr(ln_b), _ptr(z), zrs, int(z_act), _ptr(dout),
                                           _ptr(stats), _ptr(dy), _ptr(dz_out) if z is not None else None, dzrs,

@@ -201,7 +201,8 @@ int32_t ss2d_out_gate_max_width(int32_t backward);
  * z:  gate rows, element (b, l, d) at z[(b*L + l) * z_row_stride + d] (a strided view of in_proj's output),
  *     or NULL for no gate; z_act != 0 applies SiLU to z inside the kernel.
  * out: (batch, L, D) channels-last. mean_rstd: (batch, L, 2) fp32 saved for the backward (may be NULL).
- * ln_weight / ln_bias: (D) fp32 or NULL (no affine). D <= 1664 forward, <= 832 backward.
+ * ln_weight / ln_bias: (D) fp32 or NULL (no affine); a bias without a weight (which nn.LayerNorm cannot produce) is
+ *     SS2D_ERR_UNSUPPORTED. D <= 1664 forward, <= 832 backward.
  * transposed_mask: bit k set = plane k of ys is in the pixel order of the TRANSPOSED (W, H) image — how the
  *     column-major directions 2 and 4 are run (as directions 1 and 3 of a transposed input); the kernel undoes
  *     the transposition while merging. H, W are the natural image sizes (only read when the mask is non-zero). */
@@ -228,9 +229,11 @@ int32_t ss2d_out_gate_bwd_partials(int32_t batch, int32_t L);
 
 /* ---- grouped epilogue: the G single-direction SS2Ds of one GroupMambaLayer in one launch ---------------------
  * (model/gm/groupmamba.py:143-149: four SS2D modules on channel quarters, outputs concatenated along C.)
- * ys: fp32 (batch, G, D, L) scan outputs, one plane per group; group g's plane is plane_of[g]; bit p of transposed_planes:
- *     plane p is stored in the pixel order of the TRANSPOSED image (column-major directions run as row-major scans of it).
- * ln_weight / ln_bias: fp32 (G, D) — each group's own out_norm (ss2d.py:498). z: rows of z_row_stride elements; group g's
+ * ys: fp32 (batch, G, D, L) scan outputs, one plane per group; group g's plane is plane_of[g], a permutation of 0 ... G - 1
+ *     (an index out of range or repeated: SS2D_ERR_BAD_LAYOUT); bit p of transposed_planes: plane p is stored in the pixel
+ *     order of the TRANSPOSED image (column-major directions run as row-major scans of it).
+ * ln_weight / ln_bias: fp32 (G, D) — each group's own out_norm (ss2d.py:498); as for ss2d_out_gate_fwd, either may be NULL,
+ * but a bias without a weight is SS2D_ERR_UNSUPPORTED. z: rows of z_row_stride elements; group g's
  * D gate values start at column z_col0 + g * z_group_stride of a row (raw, SiLU applied here: ss2d.py:506-508, 517).
  * out: (batch, L, ...) rows of out_row_stride elements; group g writes columns g*D ... g*D + D - 1 — the concatenation.
  * mean_rstd: fp32 (G, batch, L, 2), kept for the backward.
@@ -362,7 +365,8 @@ int32_t ss2d_linear_tc_supported(int32_t n_cols, int32_t K, int32_t dtype);
  * z: rows of z_row_stride elements (batch * L rows, D columns), dtype `dtype`, or NULL; z_act != 0: SiLU(z).
  * W: (C, D) rows ldw elements apart, `dtype`; bias: (C) fp32 or NULL. out: (batch * L, C) rows out_row_stride apart, `dtype`.
  * g_out: optional (batch * L, D) rows: the gated tensor (what out_proj's weight gradient needs); mean_rstd: optional
- * (batch * L, 2) fp32 for ss2d_out_gate_bwd. D % 64 == 0, C % 16 == 0, C <= 256, operand tile + weight within shared memory
+ * (batch * L, 2) fp32 for ss2d_out_gate_bwd. ln_weight / ln_bias as for ss2d_out_gate_fwd (a bias without a weight:
+ * SS2D_ERR_UNSUPPORTED). D % 64 == 0, C % 16 == 0, C <= 256, operand tile + weight within shared memory
  * (ss2d_gate_proj_supported); H % 4 == 0 and Wd % 4 == 0 (the planes are read as TMA boxes); all row pointers / strides
  * 16-byte aligned.
  * C == 0 (W = NULL, out = NULL): epilogue only — the kernel stops after the gate and g_out (required) receives what
