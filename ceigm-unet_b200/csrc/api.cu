@@ -164,20 +164,25 @@ static bool tma_eligible(const ss2d_scan_desc* d, const void* u, const void* del
   return aligned(u, 16) && aligned(delta, 16) && aligned(B, 16) && aligned(C, 16) && (!extra || aligned(extra, 16));
 }
 
-// states are processed in passes of <= 32; pass i covers [32 i, 32 i + n_i)
+// states are processed in passes of <= 32; pass i covers states [n0, n0 + n) = [32 i, 32 i + n)
 static int n_passes(int N) { return (N + kStatesPerPass - 1) / kStatesPerPass; }
+struct Pass { int n0, n; };
+static Pass pass_states(int dstate, int i) {
+  const int n0 = i * kStatesPerPass;
+  return {n0, std::min(dstate - n0, kStatesPerPass)};
+}
 static size_t ckpt_floats_pass(const ss2d_scan_desc* d, int n) {
   const size_t nck = (d->seqlen + SS2D_CHUNK - 1) / SS2D_CHUNK;
   return (size_t)d->batch * d->dim * nck * (size_t)n;
 }
 static size_t round4(size_t x) { return (x + 3) & ~(size_t)3; }
 
-// pass i of the backward: state count, kernel variant, whether later passes accumulate
-static void set_pass(ScanParams& p, const ss2d_scan_desc* d, int i) {
-  const int n0 = i * kStatesPerPass;
-  const int n = d->dstate - n0 < kStatesPerPass ? d->dstate - n0 : kStatesPerPass;
-  const Variant v = pick_variant(n);
-  p.N = n; p.NP = v.NS * v.R; p.accum = i > 0;
+// pass i: state count, kernel variant, whether later passes accumulate; returns the pass' states
+static Pass set_pass(ScanParams& p, const ss2d_scan_desc* d, int i) {
+  const Pass ps = pass_states(d->dstate, i);
+  const Variant v = pick_variant(ps.n);
+  p.N = ps.n; p.NP = v.NS * v.R; p.accum = i > 0;
+  return ps;
 }
 
 // Deterministic mode: one partial slab (batch, G, dstate, L) of dB and one of dC per extra CTA a group is split over, for the
@@ -205,10 +210,7 @@ extern "C" {
 size_t ss2d_scan_ckpt_floats(const ss2d_scan_desc* d) {
   if (validate(d) != SS2D_OK) return 0;
   size_t total = 0;
-  for (int i = 0; i < n_passes(d->dstate); ++i) {
-    const int n = d->dstate - i * kStatesPerPass < kStatesPerPass ? d->dstate - i * kStatesPerPass : kStatesPerPass;
-    total += round4(ckpt_floats_pass(d, n));
-  }
+  for (int i = 0; i < n_passes(d->dstate); ++i) total += round4(ckpt_floats_pass(d, pass_states(d->dstate, i).n));
   return total;
 }
 
@@ -254,10 +256,7 @@ static int scan_fwd_impl(const ss2d_scan_desc* d, const void* u, const void* del
   p.tma_ok = tma_eligible(d, u, delta, Bmat, Cmat, nullptr);
   size_t ck_off = 0;
   for (int i = 0; i < n_passes(d->dstate); ++i) {
-    const int n0 = i * kStatesPerPass;
-    const int n = d->dstate - n0 < kStatesPerPass ? d->dstate - n0 : kStatesPerPass;
-    const Variant v = pick_variant(n);
-    p.N = n; p.NP = v.NS * v.R; p.accum = i > 0;
+    const auto [n0, n] = set_pass(p, d, i);
     p.A = A + n0;
     p.Bm = static_cast<const char*>(Bmat) + (size_t)n0 * d->B_state_stride * esize(d->io_dtype);
     p.Cm = static_cast<const char*>(Cmat) + (size_t)n0 * d->C_state_stride * esize(d->io_dtype);
@@ -413,9 +412,7 @@ int ss2d_scan_bwd_state(const ss2d_scan_desc* d, const void* u, const void* delt
   const int zeroed = d->grads_prezeroed && !d->deterministic;
   size_t ck_off = 0;
   for (int i = 0; i < n_passes(d->dstate); ++i) {
-    const int n0 = i * kStatesPerPass;
-    const int n = d->dstate - n0 < kStatesPerPass ? d->dstate - n0 : kStatesPerPass;
-    set_pass(p, d, i);
+    const auto [n0, n] = set_pass(p, d, i);
     p.A = A + n0;
     p.Bm = static_cast<const char*>(Bmat) + (size_t)n0 * d->B_state_stride * esize(d->io_dtype);
     p.Cm = static_cast<const char*>(Cmat) + (size_t)n0 * d->C_state_stride * esize(d->io_dtype);

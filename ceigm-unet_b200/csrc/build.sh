@@ -13,7 +13,7 @@ FLAGS=(-std=c++17 -O3 -gencode arch=compute_100a,code=sm_100a -lineinfo --use_fa
        -Xcompiler -fPIC -I"$ROOT/include" -I"$HERE" -Xptxas -v "$@")
 mkdir -p "$OBJ"
 : > "$LOG"
-newest_hdr=$(ls -t "$HERE"/*.cuh "$HERE"/*.h "$HERE"/*.inc "$ROOT"/include/*.h "$HERE/build.sh" | head -1)
+newest_hdr=$(ls -t "$HERE"/*.cuh "$HERE"/*.h "$ROOT"/include/*.h "$HERE/build.sh" | head -1)
 pids=()
 srcs=("$HERE"/*.cu)
 for src in "${srcs[@]}"; do

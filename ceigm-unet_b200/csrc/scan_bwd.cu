@@ -102,16 +102,444 @@ __device__ __forceinline__ void store_states(float* __restrict__ dst, const floa
 
 // STATE: the recompute of tile 0 starts from st.h0, the adjoint from st.dlast, and st.dh0 receives the adjoint of h0 (each
 // pointer may be null)
-template <int NS, int R, int RPT, bool DET>
-__global__ void __launch_bounds__(kBwdThreads, RPT == 1 ? 4 : 3) scan_bwd_kernel(const ScanParams p, const __grid_constant__ TmaMaps maps) {
-  constexpr bool STATE = false;
-  const ScanState st{};
-#include "scan_bwd_body.inc"
-}
-template <int NS, int R, int RPT, bool DET>
-__global__ void __launch_bounds__(kBwdThreads, RPT == 1 ? 4 : 3) scan_bwd_state_kernel(const ScanParams p, const __grid_constant__ TmaMaps maps, const ScanState st) {
-  constexpr bool STATE = true;
-#include "scan_bwd_body.inc"
+template <int NS, int R, int RPT, bool STATE, bool DET>
+__global__ void __launch_bounds__(kBwdThreads, RPT == 1 ? 4 : 3) scan_bwd_kernel(const ScanParams p, const __grid_constant__ TmaMaps maps, const ScanState st) {
+  using S = BwdShape<NS, R, RPT>;
+  constexpr int CH = S::CH, NP = S::NP, NPB = S::NPB, RL = S::RL, RPW = S::RPW, CNT = S::CNT, NW = kBwdConsumerWarps;
+  extern __shared__ __align__(16) float smem_raw[];
+  float* smem = smem_raw + ((1024 - (smem_u32(smem_raw) & 1023)) & 1023) / 4;
+  float* s_slab = smem + kBwdStages * S::stage_floats;             // [2 buffers][NW][2][NP][16]
+  float* s_hs = s_slab + 2 * NW * S::slab_floats;                  // [NW][8 groups][RPT][32 lanes][NS]
+  float* s_bias = s_hs + NW * S::hs_floats;                        // [CH]
+  float* s_D = s_bias + CH;                                        // [CH]
+  uint64_t* full = reinterpret_cast<uint64_t*>(s_D + CH);          // [stages]
+  uint64_t* empty = full + kBwdStages;                             // [stages]
+  uint64_t* slab_full = empty + kBwdStages;                        // [2]
+  uint64_t* slab_empty = slab_full + 2;                            // [2]
+  auto st_dl = [&](int s) { return smem + s * S::stage_floats; };                          // delta -> d(delta)
+  auto st_u = [&](int s) { return smem + s * S::stage_floats + CH * BLT; };                // u
+  auto st_dy = [&](int s) { return smem + s * S::stage_floats + 2 * CH * BLT; };           // dout -> du
+  auto st_B = [&](int s) { return smem + s * S::stage_floats + 3 * CH * BLT; };            // [NPB][32]
+  auto st_C = [&](int s) { return smem + s * S::stage_floats + (3 * CH + NPB) * BLT; };    // [NPB][32]
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.z, g = blockIdx.y;
+  const int row0 = blockIdx.x * CH;
+  const int rows_valid = min(CH, p.dpg - row0);
+  const int d0 = g * p.dpg + row0;
+  const int L = p.L;
+  ScanOrder so;
+  so.dir = p.layout == SS2D_LAYOUT_NATURAL ? p.dirs[g] : 0;
+  so.H = p.H; so.W = p.W; so.L = L;
+  const bool tma = p.tma_ok && so.contiguous();          // SCAN layout, directions 1 and 3
+  const bool rev = tma && so.reversed();                 // TMA-staged tiles of a reversed traversal are mirrored
+  const int ntiles = (L + BLT - 1) / BLT;
+
+  for (int r = tid; r < CH; r += kBwdThreads) {
+    const bool ok = r < rows_valid;
+    s_bias[r] = (ok && p.bias) ? p.bias[d0 + r] : 0.f;
+    s_D[r] = (ok && p.Dv && !p.accum) ? p.Dv[d0 + r] : 0.f;
+  }
+  if (tid == 0) {
+    for (int s = 0; s < kBwdStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], NW); }
+    for (int s = 0; s < 2; ++s) { mbar_init(&slab_full[s], NW); mbar_init(&slab_empty[s], 1); }
+    fence_mbar_init();
+  }
+  __syncthreads();
+
+  const int64_t u_boff = (int64_t)b * p.u_bs, dl_boff = (int64_t)b * p.dl_bs, out_boff = (int64_t)b * p.out_bs;
+  auto u_off = [&](int r) { const int d = d0 + r; return u_boff + (int64_t)(p.u_mod > 0 ? d % p.u_mod : d) * p.u_ds; };
+  // du has u's strides, except when the groups share u (u_mod > 0): then it is a dense (batch, dim, L) tensor
+  auto du_off = [&](int r) {
+    return p.u_mod > 0 ? ((int64_t)b * p.dim + d0 + r) * (int64_t)L : u_boff + (int64_t)(d0 + r) * p.u_ds;
+  };
+  auto dl_off = [&](int r) { return dl_boff + (int64_t)(d0 + r) * p.dl_ds; };
+  auto dy_off = [&](int r) { const int d = d0 + r; return out_boff + (int64_t)(p.u_mod > 0 ? d % p.u_mod : d) * p.out_ds; };
+  const int64_t B_base = (int64_t)b * p.B_bs + (int64_t)g * p.B_gs;
+  const int64_t C_base = (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
+  auto B_off = [&](int n) { return B_base + (int64_t)n * p.B_ns; };
+  auto C_off = [&](int n) { return C_base + (int64_t)n * p.C_ns; };
+
+  if (warp == NW) {
+    // =============================== producer warp ===============================
+    if (tma && lane == 0) {
+      tma_prefetch_desc(&maps.u); tma_prefetch_desc(&maps.dl); tma_prefetch_desc(&maps.dy);
+      tma_prefetch_desc(&maps.B); tma_prefetch_desc(&maps.C);
+    }
+    const int urow0 = p.u_mod > 0 ? d0 % p.u_mod : d0;
+    const bool single_cta_group = DET || gridDim.x == 1;
+    // fold the NW per-warp slabs of half tile `hc` (processing order) and send the sums to dB / dC
+    auto flush_half = [&](int hc) {
+      const int buf = hc & 1;
+      mbar_wait_relaxed(&slab_full[buf], (hc >> 1) & 1);
+      const int it = hc >> 1, t = ntiles - 1 - it;              // tile index along the scan
+      const int half = (hc & 1) ? 0 : 1;                        // the upper half of a tile is processed first
+      const int l_base = t * BLT + half * kHalf;
+      const float* base = s_slab + (size_t)buf * NW * S::slab_floats;
+      for (int i = lane; i < 2 * NP * (kHalf / 4); i += 32) {
+        const int which = i / (NP * (kHalf / 4)), rem = i - which * NP * (kHalf / 4);
+        const int n = rem / (kHalf / 4), c = (rem - n * (kHalf / 4)) * 4;
+        float4 acc = *reinterpret_cast<const float4*>(base + (which * NP + n) * S::kSlabPitch + c);
+#pragma unroll
+        for (int w = 1; w < NW; ++w) {
+          const float4 v = *reinterpret_cast<const float4*>(base + w * S::slab_floats + (which * NP + n) * S::kSlabPitch + c);
+          acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+        }
+        const int l = l_base + c;
+        if (n < p.N && l < L) {
+          float* dst = (DET ? det_slab(p, which, blockIdx.x) : (which == 0 ? p.dB : p.dC)) + ((int64_t)(b * p.G + g) * p.A_ld + n) * L;
+          if (so.dir <= 1 && l + 3 < L && (L & 3) == 0) {
+            float4* q4 = reinterpret_cast<float4*>(dst + l);
+            if (single_cta_group) *q4 = acc;
+            else asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(q4), "f"(acc.x), "f"(acc.y), "f"(acc.z), "f"(acc.w) : "memory");
+          } else {
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              if (l + e < L) {
+                float* q1 = dst + so.natural(l + e);
+                if (single_cta_group) *q1 = f4_at(acc, e);
+                else atomicAdd(q1, f4_at(acc, e));
+              }
+            }
+          }
+        }
+      }
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&slab_empty[buf]);
+    };
+    for (int it = 0; it < ntiles; ++it) {
+      const int t = ntiles - 1 - it;
+      const int s = it % kBwdStages, use = it / kBwdStages;
+      const int l0 = t * BLT, len = min(BLT, L - l0);
+      mbar_wait_relaxed(&empty[s], (use & 1) ^ 1);
+      if (tma) {
+        if (lane == 0) {
+          const int m0 = rev ? L - l0 - BLT : l0;      // memory offset of the tile (may be < 0: zero-filled by TMA)
+          mbar_arrive_expect_tx(&full[s], (uint32_t)S::stage_floats * 4);
+          tma_load_3d(st_u(s), &maps.u, m0, urow0, b, &full[s]);
+          tma_load_3d(st_dl(s), &maps.dl, m0, d0, b, &full[s]);
+          tma_load_3d(st_dy(s), &maps.dy, m0, urow0, b, &full[s]);
+          tma_load_4d(st_B(s), &maps.B, m0, 0, g, b, &full[s]);
+          tma_load_4d(st_C(s), &maps.C, m0, 0, g, b, &full[s]);
+        }
+      } else {
+        stage_rows<BLT, BLT>(st_u(s), p.u, p.io_dtype, u_off, CH, rows_valid, l0, len, so, lane, 32);
+        stage_rows<BLT, BLT>(st_dl(s), p.delta, p.io_dtype, dl_off, CH, rows_valid, l0, len, so, lane, 32);
+        stage_rows<BLT, BLT>(st_dy(s), p.dout, p.out_dtype, dy_off, CH, rows_valid, l0, len, so, lane, 32);
+        stage_rows<BLT, BLT>(st_B(s), p.Bm, p.io_dtype, B_off, NPB, p.N, l0, len, so, lane, 32);
+        stage_rows<BLT, BLT>(st_C(s), p.Cm, p.io_dtype, C_off, NPB, p.N, l0, len, so, lane, 32);
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&full[s]);
+      }
+      // the stage just refilled was released by the consumers finishing tile it - kBwdStages: its slabs are complete
+      if (it >= kBwdStages) { flush_half(2 * (it - kBwdStages)); flush_half(2 * (it - kBwdStages) + 1); }
+    }
+    for (int it = max(0, ntiles - kBwdStages); it < ntiles; ++it) { flush_half(2 * it); flush_half(2 * it + 1); }
+    return;
+  }
+
+  // =============================== consumer warps ===============================
+  const int q = lane % R, rl = lane / R;
+  float* my_hs = s_hs + warp * S::hs_floats;
+  int rk[RPT];
+  float A1[RPT][NS], A2[RPT][NS], carry[RPT][NS], dDacc[RPT], dbacc[RPT];
+  float2 dA2[RPT][NS];     // dA accumulated separately on even / odd positions (packed FFMA2), summed at the end
+#pragma unroll
+  for (int k = 0; k < RPT; ++k) {
+    rk[k] = warp * RPW + k * RL + rl;
+    dDacc[k] = 0.f; dbacc[k] = 0.f;
+#pragma unroll
+    for (int j = 0; j < NS; ++j) {
+      const int n = j * R + q;
+      A1[k][j] = (rk[k] < rows_valid && n < p.N) ? p.A[(int64_t)(d0 + rk[k]) * p.A_ld + n] : 0.f;
+      A2[k][j] = A1[k][j] * kLog2e;
+      carry[k][j] = 0.f;     // a_(l+1) * g_(l+1), zero (STATE: dlast) past the end of the sequence
+      if (STATE && st.dlast && rk[k] < rows_valid && n < p.N) carry[k][j] = st.dlast[state_slot(p, b, d0 + rk[k], n)];
+      dA2[k][j] = make_float2(0.f, 0.f);
+    }
+  }
+
+  // state before tile 0: zero, or h0 (STATE)
+  auto entry_state = [&](int k, int n) -> float {
+    return (STATE && st.h0 && rk[k] < rows_valid && n < p.N) ? __ldg(st.h0 + state_slot(p, b, d0 + rk[k], n)) : 0.f;
+  };
+  float h0_next[RPT][NS];     // checkpoint (state before the tile) of the tile processed next
+#pragma unroll
+  for (int k = 0; k < RPT; ++k)
+#pragma unroll
+    for (int j = 0; j < NS; ++j) {
+      const int n = j * R + q;
+      h0_next[k][j] = (ntiles > 1 && rk[k] < rows_valid && n < p.N)
+                          ? __ldg(p.ckpt_in + (((int64_t)b * p.dim + d0 + rk[k]) * p.nck + (ntiles - 2)) * p.N + n)
+                          : (STATE && ntiles == 1) ? entry_state(k, n) : 0.f;
+    }
+
+  // the tile loop is instantiated twice so that the mirror of reversed traversals costs nothing at run time
+  auto consume = [&](auto REV) {
+    constexpr bool REVV = decltype(REV)::value;
+  for (int it = 0; it < ntiles; ++it) {
+    const int t = ntiles - 1 - it;
+    const int s = it % kBwdStages, use = it / kBwdStages;
+    const int l0 = t * BLT, len = min(BLT, L - l0);
+    float* s_dl = st_dl(s);
+    const float* s_u = st_u(s);
+    float* s_dy = st_dy(s);
+    const float* s_B = st_B(s);
+    const float* s_C = st_C(s);
+    mbar_wait(&full[s], use & 1);
+    // activate delta for this warp's own rows, in place
+    for (int i = lane; i < RPW * (BLT / 4); i += 32) {
+      const int r = warp * RPW + i / (BLT / 4), c = (i % (BLT / 4)) * 4;    // c: scan column of the 4-group
+      float4 dv = tile_ld4(s_dl, r, c, REVV);
+      const float bias = s_bias[r];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        float x = f4_at(dv, e) + bias;
+        if (p.softplus) x = softplus20(x);
+        f4_at(dv, e) = (c + e < len && r < rows_valid) ? x : 0.f;   // idle rows may hold a neighbour group's data (TMA)
+      }
+      tile_st4(s_dl, r, c, REVV, dv);
+    }
+    __syncwarp();
+
+    // ---- (1) forward recompute of h over the tile from the checkpoint at the end of the previous chunk;
+    //          only the state after each group of 4 positions is kept (shared memory, private to the thread).
+    //          The checkpoint of the tile processed NEXT is fetched now, a whole tile ahead of its use. ----
+    float h0[RPT][NS];
+#pragma unroll
+    for (int k = 0; k < RPT; ++k)
+#pragma unroll
+      for (int j = 0; j < NS; ++j) {
+        h0[k][j] = h0_next[k][j];
+        const int n = j * R + q;
+        h0_next[k][j] = (t > 1 && rk[k] < rows_valid && n < p.N)
+                            ? __ldg(p.ckpt_in + (((int64_t)b * p.dim + d0 + rk[k]) * p.nck + (t - 2)) * p.N + n)
+                            : (STATE && t == 1) ? entry_state(k, n) : 0.f;
+      }
+    {
+      float h[RPT][NS];
+#pragma unroll
+      for (int k = 0; k < RPT; ++k)
+#pragma unroll
+        for (int j = 0; j < NS; ++j) h[k][j] = h0[k][j];
+#pragma unroll 2
+      for (int gi = 0; gi < BLT / 4 - 1; ++gi) {       // the state after the last group is never needed
+        const int c = gi * 4;
+        float4 Bv[NS];
+#pragma unroll
+        for (int j = 0; j < NS; ++j) Bv[j] = tile_ld4(s_B, j * R + q, c, REVV);
+#pragma unroll
+        for (int k = 0; k < RPT; ++k) {
+          const float4 dv = tile_ld4(s_dl, rk[k], c, REVV);
+          const float4 uv = tile_ld4(s_u, rk[k], c, REVV);
+#pragma unroll
+          for (int ep = 0; ep < 2; ++ep) {
+            const float2 d2 = ep == 0 ? make_float2(dv.x, dv.y) : make_float2(dv.z, dv.w);
+            const float2 u2 = __fmul2_rn(d2, ep == 0 ? make_float2(uv.x, uv.y) : make_float2(uv.z, uv.w));
+#pragma unroll
+            for (int j = 0; j < NS; ++j) {
+              const float2 arg = __fmul2_rn(d2, make_float2(A2[k][j], A2[k][j]));
+              const float2 bu = __fmul2_rn(u2, ep == 0 ? make_float2(Bv[j].x, Bv[j].y) : make_float2(Bv[j].z, Bv[j].w));
+              h[k][j] = fmaf(ex2f(arg.x), h[k][j], bu.x);
+              h[k][j] = fmaf(ex2f(arg.y), h[k][j], bu.y);
+            }
+          }
+          store_states<NS>(my_hs + ((gi * RPT + k) * 32 + lane) * NS, h[k]);
+        }
+      }
+    }
+
+    // ---- (2) groups of 4 positions, last to first: re-expand h and a, then the adjoint recurrence ----
+#pragma unroll 1
+    for (int gi = BLT / 4 - 1; gi >= 0; --gi) {
+      const int c = gi * 4;
+      float4 Bv[NS], Cv[NS];
+#pragma unroll
+      for (int j = 0; j < NS; ++j) {
+        Bv[j] = tile_ld4(s_B, j * R + q, c, REVV);
+        Cv[j] = tile_ld4(s_C, j * R + q, c, REVV);
+      }
+      // dB / dC partials [NS][2 position pairs], summed over this thread's RPT rows; packed f32x2 arithmetic throughout:
+      // only the two recurrences (h forward, g backward) are inherently scalar chains
+      float2 pB[NS][2], pC[NS][2];
+#pragma unroll
+      for (int j = 0; j < NS; ++j) { pB[j][0] = pB[j][1] = pC[j][0] = pC[j][1] = make_float2(0.f, 0.f); }
+#pragma unroll
+      for (int k = 0; k < RPT; ++k) {
+        const float4 dv = tile_ld4(s_dl, rk[k], c, REVV);
+        const float4 uv = tile_ld4(s_u, rk[k], c, REVV);
+        const float4 dy = tile_ld4(s_dy, rk[k], c, REVV);
+        const float2 dl01 = make_float2(dv.x, dv.y), dl23 = make_float2(dv.z, dv.w);
+        const float2 dy01 = make_float2(dy.x, dy.y), dy23 = make_float2(dy.z, dy.w);
+        const float2 dU01 = __fmul2_rn(dl01, make_float2(uv.x, uv.y)), dU23 = __fmul2_rn(dl23, make_float2(uv.z, uv.w));
+        float hin[NS];
+        if (gi > 0) load_states<NS>(my_hs + (((gi - 1) * RPT + k) * 32 + lane) * NS, hin);
+        else {
+#pragma unroll
+          for (int j = 0; j < NS; ++j) hin[j] = h0[k][j];
+        }
+        float2 sB01 = make_float2(0.f, 0.f), sB23 = sB01, sA01 = sB01, sA23 = sB01;
+#pragma unroll
+        for (int j = 0; j < NS; ++j) {
+          const float2 B01 = make_float2(Bv[j].x, Bv[j].y), B23 = make_float2(Bv[j].z, Bv[j].w);
+          const float2 A2p = make_float2(A2[k][j], A2[k][j]), A1p = make_float2(A1[k][j], A1[k][j]);
+          // re-expand a = exp(delta A) and h over the 4 positions
+          const float2 e01 = __fmul2_rn(dl01, A2p), e23 = __fmul2_rn(dl23, A2p);
+          const float a0 = ex2f(e01.x), a1 = ex2f(e01.y), a2 = ex2f(e23.x), a3 = ex2f(e23.y);
+          const float2 bu01 = __fmul2_rn(dU01, B01), bu23 = __fmul2_rn(dU23, B23);
+          const float hh0 = fmaf(a0, hin[j], bu01.x);
+          const float hh1 = fmaf(a1, hh0, bu01.y);
+          const float hh2 = fmaf(a2, hh1, bu23.x);
+          const float hh3 = fmaf(a3, hh2, bu23.y);
+          // adjoint chain, last position first: g_e = C_e dy_e + a_(e+1) g_(e+1);  t_e = a_e g_e
+          const float g3 = fmaf(Cv[j].w, dy.w, carry[k][j]);
+          const float t3 = g3 * a3;
+          const float g2 = fmaf(Cv[j].z, dy.z, t3);
+          const float t2 = g2 * a2;
+          const float g1 = fmaf(Cv[j].y, dy.y, t2);
+          const float t1 = g1 * a1;
+          const float g0 = fmaf(Cv[j].x, dy.x, t1);
+          const float t0 = g0 * a0;
+          carry[k][j] = t0;
+          const float2 g01 = make_float2(g0, g1), g23 = make_float2(g2, g3);
+          pB[j][0] = __ffma2_rn(g01, dU01, pB[j][0]);
+          pB[j][1] = __ffma2_rn(g23, dU23, pB[j][1]);
+          pC[j][0] = __ffma2_rn(dy01, make_float2(hh0, hh1), pC[j][0]);
+          pC[j][1] = __ffma2_rn(dy23, make_float2(hh2, hh3), pC[j][1]);
+          sB01 = __ffma2_rn(g01, B01, sB01);
+          sB23 = __ffma2_rn(g23, B23, sB23);
+          const float2 w01 = __fmul2_rn(make_float2(t0, t1), make_float2(hin[j], hh0));   // t_e h_(e-1)
+          const float2 w23 = __fmul2_rn(make_float2(t2, t3), make_float2(hh1, hh2));
+          sA01 = __ffma2_rn(w01, A1p, sA01);
+          sA23 = __ffma2_rn(w23, A1p, sA23);
+          dA2[k][j] = __ffma2_rn(w01, dl01, dA2[k][j]);
+          dA2[k][j] = __ffma2_rn(w23, dl23, dA2[k][j]);
+        }
+        const float sB[4] = {sB01.x, sB01.y, sB23.x, sB23.y}, sA[4] = {sA01.x, sA01.y, sA23.x, sA23.y};
+        float sums[8];     // [e][sB | sA]
+#pragma unroll
+        for (int e = 0; e < 4; ++e) { sums[e * 2] = sB[e]; sums[e * 2 + 1] = sA[e]; }
+        // combine the R state lanes of the row; afterwards lane q owns 4/R positions (or half of one for R = 8)
+        lane_reduce_scatter<R, 1, 8>(sums, q);
+        constexpr int PER = (8 / R) > 0 ? (8 / R) : 1;
+        float other = 0.f;
+        if (R == 8) other = __shfl_xor_sync(0xffffffffu, sums[0], 1);
+        if (R < 8 || (q & 1) == 0) {
+          constexpr int NE = R == 8 ? 1 : PER / 2;     // positions owned
+          const int e0 = R == 8 ? (q >> 1) : q * NE;
+#pragma unroll
+          for (int ee = 0; ee < NE; ++ee) {
+            const int e = e0 + ee;
+            const float sBe = sums[ee * 2 + 0];
+            const float sAe = R == 8 ? other : sums[ee * 2 + 1];
+            const int idx = swz1(rk[k], c + e, REVV);
+            const float de = s_dl[idx], uu = s_u[idx], dyv = s_dy[idx];
+            const float du_out = fmaf(s_D[rk[k]], dyv, de * sBe);
+            float ddl = fmaf(uu, sBe, sAe);
+            if (p.softplus) {   // sigmoid(raw) = 1 - exp(-softplus(raw)); series for small delta avoids cancellation
+              const float sig = de < 0.015625f ? de * (1.f - de * (0.5f - de * 0.16666667f)) : 1.f - ex2f(-de * kLog2e);
+              ddl *= sig;
+            }
+            if (c + e >= len) ddl = 0.f;
+            dDacc[k] = fmaf(dyv, uu, dDacc[k]);
+            dbacc[k] += ddl;
+            // every lane of the row has consumed dy / delta of this group (the shuffles above ordered them): reuse the tiles
+            s_dy[idx] = du_out;
+            s_dl[idx] = ddl;
+          }
+        }
+      }
+      // dB/dC: sum over the RL row lanes of the warp, then park the warp's totals in its slab for this half tile
+      float part[CNT];     // [dB | dC][NS][4]
+#pragma unroll
+      for (int j = 0; j < NS; ++j) {
+        part[(0 * NS + j) * 4 + 0] = pB[j][0].x; part[(0 * NS + j) * 4 + 1] = pB[j][0].y;
+        part[(0 * NS + j) * 4 + 2] = pB[j][1].x; part[(0 * NS + j) * 4 + 3] = pB[j][1].y;
+        part[(1 * NS + j) * 4 + 0] = pC[j][0].x; part[(1 * NS + j) * 4 + 1] = pC[j][0].y;
+        part[(1 * NS + j) * 4 + 2] = pC[j][1].x; part[(1 * NS + j) * 4 + 3] = pC[j][1].y;
+      }
+      lane_reduce_scatter<RL, R, CNT>(part, rl);
+      {
+        const int hc = 2 * it + (gi >= BLT / 8 ? 0 : 1);       // half tiles in processing order
+        const int buf = hc & 1;
+        if (gi == BLT / 4 - 1 || gi == BLT / 8 - 1) mbar_wait(&slab_empty[buf], ((hc >> 1) & 1) ^ 1);   // first group of a half
+        constexpr int PER = CNT >= RL ? CNT / RL : 1;
+        constexpr int REP = CNT >= RL ? 1 : RL / CNT;          // replicas when there are fewer values than lanes
+        if ((rl % REP) == 0) {
+          const int slice = rl / REP;
+          float* slab = s_slab + ((size_t)buf * NW + warp) * S::slab_floats;
+          const int ch = c & (kHalf - 1);
+          if constexpr (PER >= 4) {      // each lane holds whole 4-position vectors of one (tensor, state): vector stores
+#pragma unroll
+            for (int i = 0; i < PER; i += 4) {
+              const int vi = slice * PER + i;                   // index into [dB | dC][NS][4]
+              const int which = vi / (NS * 4), j = (vi / 4) % NS;
+              *reinterpret_cast<float4*>(slab + (which * NP + j * R + q) * S::kSlabPitch + ch) =
+                  make_float4(part[i], part[i + 1], part[i + 2], part[i + 3]);
+            }
+          } else {
+#pragma unroll
+            for (int i = 0; i < PER; ++i) {
+              const int vi = slice * PER + i;
+              const int which = vi / (NS * 4), j = (vi / 4) % NS, e = vi & 3;
+              slab[(which * NP + j * R + q) * S::kSlabPitch + ch + e] = part[i];
+            }
+          }
+        }
+        if (gi == BLT / 8 || gi == 0) {                        // last group of a half: hand the slab to the producer
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&slab_full[buf]);
+        }
+      }
+    }
+    __syncwarp();
+    // ---- tile epilogue: this warp's rows of du / d(delta) go to global memory, then the stage is released ----
+    for (int i = lane; i < RPW * (BLT / 4); i += 32) {
+      const int r = warp * RPW + i / (BLT / 4), c = (i % (BLT / 4)) * 4;
+      if (r < rows_valid && c < len) {
+        const float4 a = tile_ld4(s_dy, r, c, REVV);
+        const float4 d = tile_ld4(s_dl, r, c, REVV);
+        store_scan4(p.du, p.io_dtype, du_off(r), l0 + c, l0 + len, a, so, p.accum != 0);
+        store_scan4(p.ddelta, p.io_dtype, dl_off(r), l0 + c, l0 + len, d, so, p.accum != 0);
+      }
+    }
+    fence_proxy_async();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&empty[s]);
+  }
+
+  };
+  if (rev) consume(std::true_type{}); else consume(std::false_type{});
+
+  if (STATE && st.dh0) {      // the carry is now a_0 g_0 = dloss / dh0
+#pragma unroll
+    for (int k = 0; k < RPT; ++k)
+#pragma unroll
+      for (int j = 0; j < NS; ++j) {
+        const int n = j * R + q;
+        if (rk[k] < rows_valid && n < p.N) st.dh0[state_slot(p, b, d0 + rk[k], n)] = carry[k][j];
+      }
+  }
+
+  // ---- per-(batch, channel) partials of dA, dD, d(delta_bias) ----
+#pragma unroll
+  for (int k = 0; k < RPT; ++k) {
+    float dd = dDacc[k], db = dbacc[k];
+#pragma unroll
+    for (int sft = R / 2; sft >= 1; sft >>= 1) {
+      dd += __shfl_xor_sync(0xffffffffu, dd, sft);
+      db += __shfl_xor_sync(0xffffffffu, db, sft);
+    }
+    if (rk[k] < rows_valid) {
+      float* dst = p.part + ((int64_t)b * p.dim + d0 + rk[k]) * (p.N + 2);
+#pragma unroll
+      for (int j = 0; j < NS; ++j) {
+        const int n = j * R + q;
+        if (n < p.N) dst[n] = dA2[k][j].x + dA2[k][j].y;
+      }
+      if (q == 0) { dst[p.N] = dd; dst[p.N + 1] = db; }
+    }
+  }
 }
 
 // dA[d][n] = sum_b part[b][d][n]; dD[d], dbias[d] likewise. One thread per (d, slot), batch-sequential: deterministic.
@@ -158,18 +586,17 @@ __global__ void __launch_bounds__(256) scan_bwd_fold_kernel(const ScanParams p, 
 template <int NS, int R, int RPT, bool DET, bool STATE>
 static cudaError_t launch_bwd(ScanParams p, const ScanState& st, cudaStream_t stream) {
   using S = BwdShape<NS, R, RPT>;
-  const void* kern = STATE ? reinterpret_cast<const void*>(scan_bwd_state_kernel<NS, R, RPT, DET>)
-                           : reinterpret_cast<const void*>(scan_bwd_kernel<NS, R, RPT, DET>);
+  const auto kern = scan_bwd_kernel<NS, R, RPT, STATE, DET>;
   static PerDeviceOnce once;
-  cudaError_t ea = func_attr_once(once, kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::smem_bytes);
+  cudaError_t ea = func_attr_once(once, reinterpret_cast<const void*>(kern), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)S::smem_bytes);
   if (ea != cudaSuccess) return ea;
   TmaMaps maps;
   if (p.tma_ok && !(p.u_mod == 0 || p.u_mod % p.dpg == 0)) p.tma_ok = 0;
   if (p.tma_ok && !make_scan_maps(p, S::CH, S::NPB, true, &maps)) p.tma_ok = 0;
   if (!p.tma_ok) memset(&maps, 0, sizeof(maps));
   dim3 grid((p.dpg + S::CH - 1) / S::CH, p.G, p.batch);
-  if constexpr (STATE) scan_bwd_state_kernel<NS, R, RPT, DET><<<grid, kBwdThreads, S::smem_bytes, stream>>>(p, maps, st);
-  else scan_bwd_kernel<NS, R, RPT, DET><<<grid, kBwdThreads, S::smem_bytes, stream>>>(p, maps);
+  kern<<<grid, kBwdThreads, S::smem_bytes, stream>>>(p, maps, st);
   return cudaGetLastError();
 }
 

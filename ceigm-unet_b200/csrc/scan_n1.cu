@@ -333,18 +333,96 @@ __device__ __forceinline__ void n1_emit_row_grads(const ScanParams& p, int b, in
 // alignment. grads_zeroed != 0: dA / dD / d(delta_bias) are caller-zeroed accumulators; else per-(batch, channel) partials
 // go to p.part and scan_bwd_finalize sums them.
 // STATE: chunk 0 starts from st.h0, the reverse carry from st.dlast, and st.dh0 receives the adjoint of h0 (each may be null)
-template <bool VEC, bool SP, bool DET>
+template <bool VEC, bool SP, bool STATE, bool DET>
 __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_kernel(const ScanParams p, const N1Geom gm, float* __restrict__ dA,
-    float* __restrict__ dD, float* __restrict__ dbias, int grads_zeroed) {
-  constexpr bool STATE = false;
-  const ScanState st{};
-#include "scan_n1_bwd_body.inc"
-}
-template <bool VEC, bool SP, bool DET>
-__global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_state_kernel(const ScanParams p, const N1Geom gm, float* __restrict__ dA,
     float* __restrict__ dD, float* __restrict__ dbias, int grads_zeroed, const ScanState st) {
-  constexpr bool STATE = true;
-#include "scan_n1_bwd_body.inc"
+  extern __shared__ __align__(16) float s_slab[];          // [2][rt][lc]: per-row dB / dC of the current chunk (rt > 1)
+  __shared__ float s_agg[2][N1_MAX_WARPS][2];
+  __shared__ float s_red[N1_MAX_WARPS][3];
+  const N1Thread q = n1_thread(gm);
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.z, g = blockIdx.y;
+  const int row = blockIdx.x * gm.rt + q.r;
+  const bool valid = q.r < gm.rt && row < p.dpg;
+  const int d = g * p.dpg + (valid ? row : 0);
+  const int L = valid ? p.L : 0;
+  const bool plain = DET || gridDim.x == 1;
+  const float A1 = p.A[d];
+  const float bias = p.bias ? p.bias[d] : 0.f;
+  const float Dd = p.Dv ? p.Dv[d] : 0.f;
+  const int u_ch = p.u_mod > 0 ? d % p.u_mod : d;
+  const float* fu = static_cast<const float*>(p.u) + (int64_t)b * p.u_bs + (int64_t)u_ch * p.u_ds;
+  const float* fd = static_cast<const float*>(p.delta) + (int64_t)b * p.dl_bs + (int64_t)d * p.dl_ds;
+  const float* fy = static_cast<const float*>(p.dout) + (int64_t)b * p.out_bs + (int64_t)u_ch * p.out_ds;
+  const float* fB = static_cast<const float*>(p.Bm) + (int64_t)b * p.B_bs + (int64_t)g * p.B_gs;
+  const float* fC = static_cast<const float*>(p.Cm) + (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
+  float* fdu = static_cast<float*>(p.du) + (p.u_mod > 0 ? ((int64_t)b * p.dim + d) * (int64_t)p.L : (int64_t)b * p.u_bs + (int64_t)d * p.u_ds);
+  float* fdd = static_cast<float*>(p.ddelta) + (int64_t)b * p.dl_bs + (int64_t)d * p.dl_ds;
+  float* dBrow = (DET ? det_slab(p, 0, blockIdx.x) : p.dB) + (int64_t)(b * p.G + g) * p.L;
+  float* dCrow = (DET ? det_slab(p, 1, blockIdx.x) : p.dC) + (int64_t)(b * p.G + g) * p.L;
+  const float dfill = SP ? -INFINITY : 0.f;
+
+  auto body = [&](auto REVT) {
+    constexpr bool REV = decltype(REVT)::value;
+    float t_carry = (STATE && st.dlast && valid) ? st.dlast[state_slot(p, b, d, 0)] : 0.f;   // a_l g_l of the first position of the chunk after this one
+    float accA = 0.f, accD = 0.f, accb = 0.f;
+    for (int c = gm.nchunks - 1; c >= 0; --c) {
+      const int l0 = c * gm.lc + q.t * N1_P;
+      float dl[N1_P], uu[N1_P], bb[N1_P], cc[N1_P], dy[N1_P];
+      n1_load<VEC, REV>(fd, l0, L, dfill, dl);
+      n1_load<VEC, REV>(fu, l0, L, 0.f, uu);
+      n1_load<VEC, REV>(fy, l0, L, 0.f, dy);
+      n1_load<VEC, REV>(fB, l0, L, 0.f, bb);
+      n1_load<VEC, REV>(fC, l0, L, 0.f, cc);
+      // state entering the chunk: checkpoint written by the forward at the end of the previous SS2D_CHUNK block
+      const float h_chunk = (c > 0 && valid) ? __ldg(p.ckpt_in + ((int64_t)b * p.dim + d) * p.nck + (c * gm.lc) / SS2D_CHUNK - 1)
+                            : (STATE && st.h0 && valid) ? __ldg(st.h0 + state_slot(p, b, d, 0)) : 0.f;
+      float dub[N1_P], ddl[N1_P], dBv[N1_P], dCv[N1_P];
+#pragma unroll
+      for (int i = 0; i < N1_P; ++i) { dBv[i] = 0.f; dCv[i] = 0.f; }
+      n1_bwd_segment<SP, STATE>(dl, uu, dy, bb, cc, l0, L, A1, bias, Dd, h_chunk, t_carry, lane, q, gm, s_agg[0] + q.r * gm.wpr,
+                         s_agg[1] + q.r * gm.wpr, dub, ddl, dBv, dCv, accA, accD, accb);
+      n1_store<VEC, REV>(fdu, l0, L, dub);
+      n1_store<VEC, REV>(fdd, l0, L, ddl);
+      // ---- dB / dC: summed over the rows of this CTA, then one store (CTA = whole group) or reduction per 4 positions ----
+      if (gm.rt == 1) {
+        n1_emit<VEC, REV>(dBrow, l0, L, dBv, plain);
+        n1_emit<VEC, REV>(dCrow, l0, L, dCv, plain);
+      } else {
+        float* slabB = s_slab + (size_t)q.r * gm.lc + q.t * N1_P;
+        float* slabC = slabB + (size_t)gm.rt * gm.lc;
+        if (q.r < gm.rt) {
+          *reinterpret_cast<float4*>(slabB) = make_float4(dBv[0], dBv[1], dBv[2], dBv[3]);
+          *reinterpret_cast<float4*>(slabB + 4) = make_float4(dBv[4], dBv[5], dBv[6], dBv[7]);
+          *reinterpret_cast<float4*>(slabC) = make_float4(dCv[0], dCv[1], dCv[2], dCv[3]);
+          *reinterpret_cast<float4*>(slabC + 4) = make_float4(dCv[4], dCv[5], dCv[6], dCv[7]);
+        }
+        __syncthreads();
+        const int L0 = p.L, c8 = gm.lc / N1_P;
+        for (int i = threadIdx.x; i < 2 * c8; i += blockDim.x) {
+          const int which = i / c8, pos = (i - which * c8) * N1_P;
+          const int l = c * gm.lc + pos;
+          if (l >= L0) continue;
+          float acc[N1_P];
+#pragma unroll
+          for (int e = 0; e < N1_P; ++e) acc[e] = 0.f;
+          const float* col = s_slab + (size_t)which * gm.rt * gm.lc + pos;
+          for (int rr = 0; rr < gm.rt; ++rr) {
+            const float4 v0 = *reinterpret_cast<const float4*>(col + (size_t)rr * gm.lc);
+            const float4 v1 = *reinterpret_cast<const float4*>(col + (size_t)rr * gm.lc + 4);
+            acc[0] += v0.x; acc[1] += v0.y; acc[2] += v0.z; acc[3] += v0.w;
+            acc[4] += v1.x; acc[5] += v1.y; acc[6] += v1.z; acc[7] += v1.w;
+          }
+          n1_emit<VEC, REV>(which == 0 ? dBrow : dCrow, l, L0, acc, plain);
+        }
+        __syncthreads();
+      }
+    }
+    if (STATE && st.dh0 && q.t == 0 && valid) st.dh0[state_slot(p, b, d, 0)] = t_carry;      // a_0 g_0
+    n1_row_sum3(accA, accD, accb, lane, q, gm, s_red + q.r * gm.wpr, 1 + q.r);
+    if (q.t == 0 && valid) n1_emit_row_grads(p, b, d, accA, accD, accb, dA, dD, dbias, !DET && grads_zeroed);
+  };
+  if (p.layout == SS2D_LAYOUT_NATURAL && p.dirs[g] == 3) body(std::true_type{}); else body(std::false_type{});
 }
 
 // ------------------------------------------------------------------------------------------------- backward, rows walked per lane
@@ -356,18 +434,187 @@ __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_state_kernel(co
 constexpr int N1_MAX_RSEQ = 64;
 
 // STATE: as scan_n1_bwd_kernel
-template <bool SP, bool DET>
+template <bool SP, bool STATE, bool DET>
 __global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_rows_kernel(const ScanParams p, const N1Geom gm, float* __restrict__ dA,
-    float* __restrict__ dD, float* __restrict__ dbias, int grads_zeroed) {
-  constexpr bool STATE = false;
-  const ScanState state{};
-#include "scan_n1_bwd_rows_body.inc"
-}
-template <bool SP, bool DET>
-__global__ void __launch_bounds__(N1_MAX_WARPS * 32) scan_n1_bwd_rows_state_kernel(const ScanParams p, const N1Geom gm, float* __restrict__ dA,
-    float* __restrict__ dD, float* __restrict__ dbias, int grads_zeroed, const ScanState state) {
-  constexpr bool STATE = true;
-#include "scan_n1_bwd_rows_body.inc"
+    float* __restrict__ dD, float* __restrict__ dbias, int grads_zeroed, const ScanState st) {
+  extern __shared__ __align__(128) float s_ring[];         // [rt][2 stages][3][lr]
+  __shared__ float s_agg[2][N1_MAX_WARPS][2];
+  __shared__ float s_red[2][N1_MAX_WARPS][3];
+  __shared__ float s_tc[N1_MAX_WARPS][N1_MAX_RSEQ];        // reverse carry of each row between chunks (multi-chunk rows)
+  __shared__ __align__(8) uint64_t s_full[N1_MAX_WARPS][2];
+  __shared__ float s_racc[DET ? N1_MAX_RSEQ : 1][3];       // DET, multi-chunk rows (one row lane): per-row running sums
+  N1Geom gq = gm;
+  gq.seg = 32;                                             // compile-time constant for the shuffle scans below
+  const N1Thread q = n1_thread(gq);
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.z, g = blockIdx.y;
+  const int L = p.L;
+  const int lr = gm.nchunks == 1 ? ((L + 31) & ~31) : gm.lc;          // ring row length (floats), a multiple of 128 bytes
+  const int rows_cta = gm.rt * gm.rseq;
+  const int row_base = blockIdx.x * rows_cta + q.r;
+  // rows this lane walks: row_base + j rt for j < nj
+  const int nj = row_base < p.dpg ? min(gm.rseq, (p.dpg - row_base + gm.rt - 1) / gm.rt) : 0;
+  const bool plain = DET || gridDim.x == 1;
+  const float* fB = static_cast<const float*>(p.Bm) + (int64_t)b * p.B_bs + (int64_t)g * p.B_gs;
+  const float* fC = static_cast<const float*>(p.Cm) + (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
+  float* dBrow = (DET ? det_slab(p, 0, blockIdx.x) : p.dB) + (int64_t)(b * p.G + g) * L;
+  float* dCrow = (DET ? det_slab(p, 1, blockIdx.x) : p.dC) + (int64_t)(b * p.G + g) * L;
+  float* ring = s_ring + (size_t)q.r * 6 * lr;
+  const bool leader = q.t == 0;                            // issues this row lane's TMA copies
+  const int total_it = nj * gm.nchunks;
+
+  auto body = [&](auto REVT) {
+    constexpr bool REV = decltype(REVT)::value;
+    auto issue = [&](int it) {                             // leader only; it = (chunk counted from the end) * nj + j
+      if (it >= total_it) return;
+      const int ci = it / nj, j = it - ci * nj, c = gm.nchunks - 1 - ci, s = it & 1;
+      const int d = g * p.dpg + row_base + j * gm.rt;
+      const int u_ch = p.u_mod > 0 ? d % p.u_mod : d;
+      const int len = min(gm.lc, L - c * gm.lc);
+      const int64_t m0 = REV ? L - c * gm.lc - len : c * gm.lc;       // first memory position of the piece
+      const uint32_t bytes = (uint32_t)len * 4u;
+      float* stg = ring + (size_t)s * 3 * lr;
+      mbar_arrive_expect_tx(&s_full[q.r][s], 3u * bytes);
+      tma_load_1d(stg, static_cast<const float*>(p.delta) + (int64_t)b * p.dl_bs + (int64_t)d * p.dl_ds + m0, bytes, &s_full[q.r][s]);
+      tma_load_1d(stg + lr, static_cast<const float*>(p.u) + (int64_t)b * p.u_bs + (int64_t)u_ch * p.u_ds + m0, bytes, &s_full[q.r][s]);
+      tma_load_1d(stg + 2 * lr, static_cast<const float*>(p.dout) + (int64_t)b * p.out_bs + (int64_t)u_ch * p.out_ds + m0, bytes, &s_full[q.r][s]);
+    };
+    if (leader) { mbar_init(&s_full[q.r][0], 1); mbar_init(&s_full[q.r][1], 1); fence_mbar_init(); }
+    __syncthreads();
+    if (leader) { issue(0); issue(1); }
+
+    for (int ci = 0; ci < gm.nchunks; ++ci) {
+      const int c = gm.nchunks - 1 - ci;
+      const int len = min(gm.lc, L - c * gm.lc);           // positions of this chunk
+      const int lq = q.t * N1_P;                           // this thread's first position inside the chunk
+      const int l0 = c * gm.lc + lq;
+      float bb[N1_P], cB[N1_P];
+      n1_load<true, REV>(fB, l0, nj > 0 ? L : 0, 0.f, bb);
+      n1_load<true, REV>(fC, l0, nj > 0 ? L : 0, 0.f, cB);
+      float dBv[N1_P], dCv[N1_P];
+#pragma unroll
+      for (int i = 0; i < N1_P; ++i) { dBv[i] = 0.f; dCv[i] = 0.f; }
+      for (int j = 0; j < nj; ++j) {
+        const int it = ci * nj + j, s = it & 1;
+        const int d = g * p.dpg + row_base + j * gm.rt;
+        const float A1 = p.A[d];
+        const float bias = p.bias ? p.bias[d] : 0.f;
+        const float Dd = p.Dv ? p.Dv[d] : 0.f;
+        const float h_chunk = c > 0 ? __ldg(p.ckpt_in + ((int64_t)b * p.dim + d) * p.nck + (c * gm.lc) / SS2D_CHUNK - 1)
+                              : (STATE && st.h0) ? __ldg(st.h0 + state_slot(p, b, d, 0)) : 0.f;
+        // written one chunk ago, several row-lane barriers back
+        float t_carry = ci > 0 ? s_tc[q.r][j] : (STATE && st.dlast) ? st.dlast[state_slot(p, b, d, 0)] : 0.f;
+        mbar_wait(&s_full[q.r][s], (uint32_t)(it >> 1) & 1u);
+        const float* stg = ring + (size_t)s * 3 * lr;
+        float dl[N1_P], uu[N1_P], dy[N1_P];
+#pragma unroll
+        for (int cch = 0; cch < N1_P; cch += 4) {
+          const bool in = lq + cch < len;
+          const int off = REV ? len - 4 - (lq + cch) : lq + cch;
+          float4 v0 = make_float4(SP ? -INFINITY : 0.f, SP ? -INFINITY : 0.f, SP ? -INFINITY : 0.f, SP ? -INFINITY : 0.f);
+          float4 v1 = make_float4(0.f, 0.f, 0.f, 0.f), v2 = v1;
+          if (in) {
+            v0 = *reinterpret_cast<const float4*>(stg + off);
+            v1 = *reinterpret_cast<const float4*>(stg + lr + off);
+            v2 = *reinterpret_cast<const float4*>(stg + 2 * lr + off);
+          }
+          dl[cch] = REV ? v0.w : v0.x; dl[cch + 1] = REV ? v0.z : v0.y; dl[cch + 2] = REV ? v0.y : v0.z; dl[cch + 3] = REV ? v0.x : v0.w;
+          uu[cch] = REV ? v1.w : v1.x; uu[cch + 1] = REV ? v1.z : v1.y; uu[cch + 2] = REV ? v1.y : v1.z; uu[cch + 3] = REV ? v1.x : v1.w;
+          dy[cch] = REV ? v2.w : v2.x; dy[cch + 1] = REV ? v2.z : v2.y; dy[cch + 2] = REV ? v2.y : v2.z; dy[cch + 3] = REV ? v2.x : v2.w;
+        }
+        float dub[N1_P], ddl[N1_P];
+        float accA = 0.f, accD = 0.f, accb = 0.f;
+        n1_bwd_segment<SP, STATE>(dl, uu, dy, bb, cB, l0, L, A1, bias, Dd, h_chunk, t_carry, lane, q, gq, s_agg[0] + q.r * gm.wpr,
+                                  s_agg[1] + q.r * gm.wpr, dub, ddl, dBv, dCv, accA, accD, accb);
+        if (STATE && st.dh0 && c == 0 && leader) st.dh0[state_slot(p, b, d, 0)] = t_carry;      // a_0 g_0
+        // every thread of the row lane passed the barriers inside the segment after its reads of stage s: refill it
+        if (gm.wpr == 1) __syncwarp();
+        if (leader) { fence_proxy_async(); issue(it + 2); if (gm.nchunks > 1) s_tc[q.r][j] = t_carry; }
+        float* fdu = static_cast<float*>(p.du) + (p.u_mod > 0 ? ((int64_t)b * p.dim + d) * (int64_t)L : (int64_t)b * p.u_bs + (int64_t)d * p.u_ds);
+        float* fdd = static_cast<float*>(p.ddelta) + (int64_t)b * p.dl_bs + (int64_t)d * p.dl_ds;
+        n1_store<true, REV>(fdu, l0, L, dub);
+        n1_store<true, REV>(fdd, l0, L, ddl);
+        // per-row sums of dA / dD / d(delta_bias): shuffle tree, one shared-memory hop, warp 0 of the row finishes
+#pragma unroll
+        for (int off = 16; off >= 1; off >>= 1) {
+          accA += __shfl_xor_sync(0xffffffffu, accA, off);
+          accD += __shfl_xor_sync(0xffffffffu, accD, off);
+          accb += __shfl_xor_sync(0xffffffffu, accb, off);
+        }
+        if (gm.wpr > 1) {
+          float (*red)[3] = s_red[it & 1] + q.r * gm.wpr;
+          if (lane == 0) { red[q.wir][0] = accA; red[q.wir][1] = accD; red[q.wir][2] = accb; }
+          n1_bar(1 + q.r, gm.wpr * 32);
+          if (q.wir == 0) {
+            accA = lane < gm.wpr ? red[lane][0] : 0.f;
+            accD = lane < gm.wpr ? red[lane][1] : 0.f;
+            accb = lane < gm.wpr ? red[lane][2] : 0.f;
+#pragma unroll
+            for (int off = 8; off >= 1; off >>= 1) {
+              accA += __shfl_xor_sync(0xffffffffu, accA, off);
+              accD += __shfl_xor_sync(0xffffffffu, accD, off);
+              accb += __shfl_xor_sync(0xffffffffu, accb, off);
+            }
+          }
+        }
+        if (q.t == 0) {
+          if (!DET && grads_zeroed) {
+            atomicAdd(dA + d, accA);
+            if (dD) atomicAdd(dD + d, accD);
+            if (dbias) atomicAdd(dbias + d, accb);
+          } else {           // partials for the finalize pass (outside DET the host sends only single-chunk rows here)
+            bool last = true;
+            if constexpr (DET) {
+              if (gm.nchunks > 1) {                        // running sums over the chunks, added in chunk order
+                float* acc = s_racc[j];
+                if (ci > 0) { accA = acc[0] + accA; accD = acc[1] + accD; accb = acc[2] + accb; }
+                last = ci == gm.nchunks - 1;
+                if (!last) { acc[0] = accA; acc[1] = accD; acc[2] = accb; }
+              }
+            }
+            if (last) {
+              float* dst = p.part + ((int64_t)b * p.dim + d) * 3;
+              dst[0] = accA; dst[1] = accD; dst[2] = accb;
+            }
+          }
+        }
+      }
+      // ---- dB / dC of this chunk over the rows the CTA walked: sum over the row lanes through shared memory ----
+      if (gm.rt == 1) {
+        if (nj > 0) {
+          n1_emit<true, REV>(dBrow, l0, L, dBv, plain);
+          n1_emit<true, REV>(dCrow, l0, L, dCv, plain);
+        }
+      } else {      // single-chunk rows: the ring is idle by now and doubles as the slab; chunked rows have their own slab
+        __syncthreads();                                   // also orders this chunk's slab writes after the previous chunk's reads
+        float* slab0 = s_ring + (gm.nchunks > 1 ? (size_t)gm.rt * 6 * lr : 0);
+        float* slabB = slab0 + (size_t)q.r * gm.lc + lq;
+        float* slabC = slabB + (size_t)gm.rt * gm.lc;
+        *reinterpret_cast<float4*>(slabB) = make_float4(dBv[0], dBv[1], dBv[2], dBv[3]);
+        *reinterpret_cast<float4*>(slabB + 4) = make_float4(dBv[4], dBv[5], dBv[6], dBv[7]);
+        *reinterpret_cast<float4*>(slabC) = make_float4(dCv[0], dCv[1], dCv[2], dCv[3]);
+        *reinterpret_cast<float4*>(slabC + 4) = make_float4(dCv[4], dCv[5], dCv[6], dCv[7]);
+        __syncthreads();
+        const int c8 = gm.lc / N1_P;
+        for (int i = threadIdx.x; i < 2 * c8; i += blockDim.x) {
+          const int which = i / c8, pos = (i - which * c8) * N1_P;
+          if (c * gm.lc + pos >= L) continue;
+          float acc[N1_P];
+#pragma unroll
+          for (int e = 0; e < N1_P; ++e) acc[e] = 0.f;
+          const float* col = slab0 + (size_t)which * gm.rt * gm.lc + pos;
+          for (int rr = 0; rr < gm.rt; ++rr) {
+            const float4 v0 = *reinterpret_cast<const float4*>(col + (size_t)rr * gm.lc);
+            const float4 v1 = *reinterpret_cast<const float4*>(col + (size_t)rr * gm.lc + 4);
+            acc[0] += v0.x; acc[1] += v0.y; acc[2] += v0.z; acc[3] += v0.w;
+            acc[4] += v1.x; acc[5] += v1.y; acc[6] += v1.z; acc[7] += v1.w;
+          }
+          n1_emit<true, REV>(which == 0 ? dBrow : dCrow, c * gm.lc + pos, L, acc, plain);
+        }
+      }
+    }
+  };
+  if (p.layout == SS2D_LAYOUT_NATURAL && p.dirs[g] == 3) body(std::true_type{}); else body(std::false_type{});
 }
 
 // ------------------------------------------------------------------------------------------------- host side
@@ -511,23 +758,14 @@ static cudaError_t n1_bwd_rows_launch(const ScanParams& p, const ScanState& st, 
                                       float* dbias, int grads_zeroed, cudaStream_t stream) {
   const bool sp = p.softplus != 0;
   static PerDeviceOnce once_sp, once_nosp;
-  const void* kern_sp = STATE ? reinterpret_cast<const void*>(scan_n1_bwd_rows_state_kernel<true, DET>)
-                              : reinterpret_cast<const void*>(scan_n1_bwd_rows_kernel<true, DET>);
-  const void* kern_nosp = STATE ? reinterpret_cast<const void*>(scan_n1_bwd_rows_state_kernel<false, DET>)
-                                : reinterpret_cast<const void*>(scan_n1_bwd_rows_kernel<false, DET>);
-  cudaError_t e = sp ? func_attr_once(once_sp, kern_sp, cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024)
-                     : func_attr_once(once_nosp, kern_nosp, cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024);
+  const auto kern = sp ? scan_n1_bwd_rows_kernel<true, STATE, DET> : scan_n1_bwd_rows_kernel<false, STATE, DET>;
+  cudaError_t e = func_attr_once(sp ? once_sp : once_nosp, reinterpret_cast<const void*>(kern),
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 136 * 1024);
   if (e != cudaSuccess) return e;
   const int rows_cta = gr.rt * gr.rseq;
   dim3 grid((p.dpg + rows_cta - 1) / rows_cta, p.G, p.batch);
   const int nt = gr.rt * gr.wpr * 32;
-  if constexpr (STATE) {
-    if (sp) scan_n1_bwd_rows_state_kernel<true, DET><<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed, st);
-    else scan_n1_bwd_rows_state_kernel<false, DET><<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed, st);
-  } else {
-    if (sp) scan_n1_bwd_rows_kernel<true, DET><<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed);
-    else scan_n1_bwd_rows_kernel<false, DET><<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed);
-  }
+  kern<<<grid, nt, smem, stream>>>(p, gr, dA, dD, dbias, grads_zeroed, st);
   return cudaGetLastError();
 }
 
@@ -538,15 +776,9 @@ static cudaError_t n1_bwd_launch(const ScanParams& p, const ScanState& st, const
   dim3 grid((p.dpg + gm.rt - 1) / gm.rt, p.G, p.batch);
   const size_t smem = n1_one_row_smem(gm);
   const int nt = n1_threads(gm);
-  if constexpr (STATE) {
-    auto kern = vec ? (sp ? scan_n1_bwd_state_kernel<true, true, DET> : scan_n1_bwd_state_kernel<true, false, DET>)
-                    : (sp ? scan_n1_bwd_state_kernel<false, true, DET> : scan_n1_bwd_state_kernel<false, false, DET>);
-    kern<<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed, st);
-  } else {
-    auto kern = vec ? (sp ? scan_n1_bwd_kernel<true, true, DET> : scan_n1_bwd_kernel<true, false, DET>)
-                    : (sp ? scan_n1_bwd_kernel<false, true, DET> : scan_n1_bwd_kernel<false, false, DET>);
-    kern<<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed);
-  }
+  auto kern = vec ? (sp ? scan_n1_bwd_kernel<true, true, STATE, DET> : scan_n1_bwd_kernel<true, false, STATE, DET>)
+                  : (sp ? scan_n1_bwd_kernel<false, true, STATE, DET> : scan_n1_bwd_kernel<false, false, STATE, DET>);
+  kern<<<grid, nt, smem, stream>>>(p, gm, dA, dD, dbias, grads_zeroed, st);
   return cudaGetLastError();
 }
 

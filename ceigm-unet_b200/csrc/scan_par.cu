@@ -232,16 +232,195 @@ __global__ void __launch_bounds__(kParThreads) scan_par_fwd_kernel(const ScanPar
 // ------------------------------------------------------------------------------------------------- backward
 // DET: dB / dC go to partial slab blockIdx.x with plain stores (summed in slab order by scan_bwd_fold_kernel)
 // STATE: chunk 0 starts from st.h0, the reverse carry from st.dlast, and st.dh0 receives the adjoint of h0 (each may be null)
-template <int T, bool DET>
-__global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_kernel(const ScanParams p) {
-  constexpr bool STATE = false;
-  const ScanState st{};
-#include "scan_par_bwd_body.inc"
-}
-template <int T, bool DET>
-__global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_state_kernel(const ScanParams p, const ScanState st) {
-  constexpr bool STATE = true;
-#include "scan_par_bwd_body.inc"
+template <int T, bool STATE, bool DET>
+__global__ void __launch_bounds__(kParThreads, 2) scan_par_bwd_kernel(const ScanParams p, const ScanState st) {
+  using S = ParShape<T>;
+  constexpr int P = 8, LC = T * P;
+  __shared__ float s_agg[2][S::RT * S::WPR][2];
+  __shared__ __align__(16) float s_slab[2][S::RT][LC];     // per-row dB / dC of the current chunk
+  __shared__ float s_red[S::RT * S::WPR][3];
+  const int tid = threadIdx.x, r = tid / T, t = tid % T;
+  const int b = blockIdx.z, g = blockIdx.y;
+  const int row = blockIdx.x * S::RT + r;
+  const bool valid = row < p.dpg;
+  const int d = g * p.dpg + (valid ? row : 0);
+  const int L = p.L;
+  ScanOrder so;
+  so.dir = p.layout == SS2D_LAYOUT_NATURAL ? p.dirs[g] : 0;
+  so.H = p.H; so.W = p.W; so.L = L;
+  const int l_end = valid ? L : 0;
+  const bool single_cta_group = DET || gridDim.x == 1;
+
+  const float A1 = valid ? p.A[(int64_t)d * p.A_ld] : 0.f;
+  const float A2 = A1 * kLog2e;
+  const float bias = (valid && p.bias) ? p.bias[d] : 0.f;
+  const float Dd = (valid && p.Dv && !p.accum) ? p.Dv[d] : 0.f;
+  const int du_ch = d, u_ch = p.u_mod > 0 ? d % p.u_mod : d;
+  const int64_t u_ro = (int64_t)b * p.u_bs + (int64_t)u_ch * p.u_ds;
+  const int64_t du_ro = p.u_mod > 0 ? ((int64_t)b * p.dim + du_ch) * (int64_t)L : (int64_t)b * p.u_bs + (int64_t)d * p.u_ds;
+  const int64_t dl_ro = (int64_t)b * p.dl_bs + (int64_t)d * p.dl_ds;
+  const int64_t dy_ro = (int64_t)b * p.out_bs + (int64_t)u_ch * p.out_ds;
+  const int64_t B_ro = (int64_t)b * p.B_bs + (int64_t)g * p.B_gs;
+  const int64_t C_ro = (int64_t)b * p.C_bs + (int64_t)g * p.C_gs;
+  float* dBrow = (DET ? det_slab(p, 0, blockIdx.x) : p.dB) + (int64_t)(b * p.G + g) * p.A_ld * L;
+  float* dCrow = (DET ? det_slab(p, 1, blockIdx.x) : p.dC) + (int64_t)(b * p.G + g) * p.A_ld * L;
+
+  const bool rev = so.reversed();
+  const bool fast_io = valid && p.io_dtype == SS2D_F32 && p.out_dtype == SS2D_F32 && so.contiguous() && (L & 3) == 0 &&
+                       !p.accum && row_fast(p.u, u_ro) && row_fast(p.delta, dl_ro) && row_fast(p.dout, dy_ro) &&
+                       row_fast(p.Bm, B_ro) && row_fast(p.Cm, C_ro) && row_fast(p.du, du_ro) && row_fast(p.ddelta, dl_ro);
+  const float* fu = reinterpret_cast<const float*>(p.u) + u_ro;
+  const float* fd = reinterpret_cast<const float*>(p.delta) + dl_ro;
+  const float* fy = reinterpret_cast<const float*>(p.dout) + dy_ro;
+  const float* fB = reinterpret_cast<const float*>(p.Bm) + B_ro;
+  const float* fC = reinterpret_cast<const float*>(p.Cm) + C_ro;
+
+  float t_carry = (STATE && st.dlast && valid) ? st.dlast[state_slot(p, b, d, 0)] : 0.f;   // a_l g_l of the first position of the chunk after this one
+  float accA = 0.f, accD = 0.f, accb = 0.f;
+  const int nchunks = (L + LC - 1) / LC;
+  for (int c = nchunks - 1; c >= 0; --c) {
+    const int l0 = c * LC + t * P;
+    const bool full = l0 + P <= l_end;
+    float dl[P], uu[P], bb[P], cc[P], dy[P];
+    if (fast_io && full) {
+      load_seg_fast<P>(fd, l0, L, rev, dl);
+      load_seg_fast<P>(fu, l0, L, rev, uu);
+      load_seg_fast<P>(fy, l0, L, rev, dy);
+      load_seg_fast<P>(fB, l0, L, rev, bb);
+      load_seg_fast<P>(fC, l0, L, rev, cc);
+    } else {
+      load_seg<P>(p.delta, p.io_dtype, dl_ro, l0, l_end, so, dl);
+      load_seg<P>(p.u, p.io_dtype, u_ro, l0, l_end, so, uu);
+      load_seg<P>(p.dout, p.out_dtype, dy_ro, l0, l_end, so, dy);
+      load_seg<P>(p.Bm, p.io_dtype, B_ro, l0, l_end, so, bb);
+      load_seg<P>(p.Cm, p.io_dtype, C_ro, l0, l_end, so, cc);
+    }
+    // state entering the chunk: checkpoint written by the forward at the end of the previous SS2D_CHUNK block
+    const float h_chunk = (c > 0 && valid)
+                              ? __ldg(p.ckpt_in + (((int64_t)b * p.dim + d) * p.nck + (c * LC) / SS2D_CHUNK - 1) * p.N)
+                              : (STATE && st.h0 && valid) ? __ldg(st.h0 + state_slot(p, b, d, 0)) : 0.f;
+    // ---- forward recompute: a, local h, decay products ----
+    float a[P], hh[P];
+    float h = 0.f, pm = 1.f;
+#pragma unroll
+    for (int i = 0; i < P; ++i) {
+      float x = dl[i] + bias;
+      if (p.softplus) x = softplus20(x);
+      if (l0 + i >= l_end) x = 0.f;
+      dl[i] = x;
+      a[i] = ex2f(x * A2);
+      h = fmaf(a[i], h, x * uu[i] * bb[i]);
+      pm *= a[i];
+      hh[i] = h;
+      cc[i] *= dy[i];                                        // c_l = C_l dy_l
+    }
+    float Pex, Hex, Ptot, Htot;
+    row_exclusive<T, true>(pm, h, t, r, s_agg[0], Pex, Hex, Ptot, Htot);
+    const float h_in = fmaf(Pex, h_chunk, Hex);              // true state before this thread's first position
+    {                                                        // true states: h_i = local_i + (prod a_0..i) h_in
+      float pc = 1.f;
+#pragma unroll
+      for (int i = 0; i < P; ++i) { pc *= a[i]; hh[i] = fmaf(pc, h_in, hh[i]); }
+    }
+    // ---- reverse: t_l = a_l (c_l + t_(l+1)); g_l = c_l + t_(l+1) ----
+    float tl[P];
+    float tq = 0.f, qm = 1.f;
+#pragma unroll
+    for (int i = P - 1; i >= 0; --i) { tq = a[i] * (cc[i] + tq); qm *= a[i]; tl[i] = tq; }
+    float Qex, Tex, Qtot, Ttot;
+    row_exclusive<T, false>(qm, tq, t, r, s_agg[1], Qex, Tex, Qtot, Ttot);
+    const float t_in = fmaf(Qex, t_carry, Tex);              // t of the position right after this thread's last one
+    float dub[P], ddl[P], dBv[P], dCv[P];
+    {
+      float qc = 1.f, t_next = t_in;
+#pragma unroll
+      for (int i = P - 1; i >= 0; --i) {
+        qc *= a[i];
+        const float ti = fmaf(qc, t_in, tl[i]);              // true t_i
+        const float gi = cc[i] + t_next;                     // true g_i
+        t_next = ti;
+        const float hprev = i > 0 ? hh[i - 1] : h_in;
+        const float sB = gi * bb[i];
+        const float w = ti * hprev;
+        float dd = fmaf(uu[i], sB, w * A1);
+        if (p.softplus) {
+          const float de = dl[i];
+          dd *= de < 0.015625f ? de * (1.f - de * (0.5f - de * 0.16666667f)) : 1.f - ex2f(-de * kLog2e);
+        }
+        if (l0 + i >= l_end) dd = 0.f;
+        dub[i] = fmaf(Dd, dy[i], dl[i] * sB);
+        ddl[i] = dd;
+        dBv[i] = gi * dl[i] * uu[i];
+        dCv[i] = dy[i] * hh[i];
+        accA = fmaf(w, dl[i], accA);
+        accD = fmaf(dy[i], uu[i], accD);
+        accb += dd;
+      }
+    }
+    if (fast_io && full) {
+      store_seg_fast<P>(reinterpret_cast<float*>(p.du) + du_ro, l0, L, rev, dub);
+      store_seg_fast<P>(reinterpret_cast<float*>(p.ddelta) + dl_ro, l0, L, rev, ddl);
+    } else {
+      store_seg<P>(p.du, p.io_dtype, du_ro, l0, l_end, so, dub, p.accum != 0);
+      store_seg<P>(p.ddelta, p.io_dtype, dl_ro, l0, l_end, so, ddl, p.accum != 0);
+    }
+    t_carry = fmaf(Qtot, t_carry, Ttot);
+    // ---- dB / dC: sum over the rows of this CTA, then one (vector) reduction per 4 positions to global memory ----
+#pragma unroll
+    for (int i = 0; i < P; i += 4) {
+      *reinterpret_cast<float4*>(&s_slab[0][r][t * P + i]) = make_float4(dBv[i], dBv[i + 1], dBv[i + 2], dBv[i + 3]);
+      *reinterpret_cast<float4*>(&s_slab[1][r][t * P + i]) = make_float4(dCv[i], dCv[i + 1], dCv[i + 2], dCv[i + 3]);
+    }
+    __syncthreads();
+    for (int i = tid; i < 2 * (LC / 4); i += kParThreads) {
+      const int which = i / (LC / 4), pos = (i - which * (LC / 4)) * 4;
+      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 4
+      for (int rr = 0; rr < S::RT; ++rr) {
+        const float4 v = *reinterpret_cast<const float4*>(&s_slab[which][rr][pos]);
+        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+      }
+      const int l = c * LC + pos;
+      if (l < L) {
+        float* dst = which == 0 ? dBrow : dCrow;
+        if (so.dir <= 1 && l + 3 < L && (L & 3) == 0) {
+          float4* q4 = reinterpret_cast<float4*>(dst + l);
+          if (single_cta_group) *q4 = acc;
+          else asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(q4), "f"(acc.x), "f"(acc.y), "f"(acc.z), "f"(acc.w) : "memory");
+        } else {
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            if (l + e < L) {
+              float* q1 = dst + so.natural(l + e);
+              if (single_cta_group) *q1 = f4_at(acc, e);
+              else atomicAdd(q1, f4_at(acc, e));
+            }
+          }
+        }
+      }
+    }
+    __syncthreads();
+  }
+  if (STATE && st.dh0 && t == 0 && valid) st.dh0[state_slot(p, b, d, 0)] = t_carry;      // a_0 g_0
+  // ---- dA, dD, d(delta_bias): sum over the T threads of the row -> per-(batch, channel) partials ----
+#pragma unroll
+  for (int off = S::SEG / 2; off >= 1; off >>= 1) {
+    accA += __shfl_xor_sync(0xffffffffu, accA, off);
+    accD += __shfl_xor_sync(0xffffffffu, accD, off);
+    accb += __shfl_xor_sync(0xffffffffu, accb, off);
+  }
+  if constexpr (S::WPR > 1) {
+    if ((t & 31) == 0) { s_red[r * S::WPR + t / 32][0] = accA; s_red[r * S::WPR + t / 32][1] = accD; s_red[r * S::WPR + t / 32][2] = accb; }
+    __syncthreads();
+    if (t == 0) {
+      accA = accD = accb = 0.f;
+      for (int w = 0; w < S::WPR; ++w) { accA += s_red[r * S::WPR + w][0]; accD += s_red[r * S::WPR + w][1]; accb += s_red[r * S::WPR + w][2]; }
+    }
+  }
+  if (t == 0 && valid) {
+    float* dst = p.part + ((int64_t)b * p.dim + d) * (p.N + 2);
+    dst[0] = accA; dst[1] = accD; dst[2] = accb;
+  }
 }
 
 // threads per row: the smallest power of two whose T*P positions cover the row, at most 128 (longer rows are chunked)
@@ -261,13 +440,8 @@ template <int T, bool DET, bool STATE>
 static cudaError_t launch_par_bwd(const ScanParams& p, const ScanState& st, cudaStream_t stream) {
   dim3 grid((p.dpg + ParShape<T>::RT - 1) / ParShape<T>::RT, p.G, p.batch);
   static PerDeviceOnce once;   // 16.6 KB of static shared memory per CTA: ask for a carve-out that fits several CTAs per SM
-  if constexpr (STATE) {
-    func_attr_once(once, reinterpret_cast<const void*>(scan_par_bwd_state_kernel<T, DET>), cudaFuncAttributePreferredSharedMemoryCarveout, 50);
-    scan_par_bwd_state_kernel<T, DET><<<grid, kParThreads, 0, stream>>>(p, st);
-  } else {
-    func_attr_once(once, reinterpret_cast<const void*>(scan_par_bwd_kernel<T, DET>), cudaFuncAttributePreferredSharedMemoryCarveout, 50);
-    scan_par_bwd_kernel<T, DET><<<grid, kParThreads, 0, stream>>>(p);
-  }
+  func_attr_once(once, reinterpret_cast<const void*>(scan_par_bwd_kernel<T, STATE, DET>), cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+  scan_par_bwd_kernel<T, STATE, DET><<<grid, kParThreads, 0, stream>>>(p, st);
   return cudaGetLastError();
 }
 template <bool DET, bool STATE>

@@ -47,10 +47,11 @@ struct ScanParams {
   int64_t slab_stride;
 };
 
-// State passing, a separate kernel argument of the STATE instantiations (ScanParams keeps its layout, so the default kernels
-// keep their instructions). Rows of A_ld floats like A; this pass's states start at element 0. Forward: the state before a
-// row's first position is h0 (non-null whenever STATE). Backward: h0 starts the recompute of chunk 0, dlast is the adjoint
-// entering the row's last position, dh0 receives the adjoint of h0; each may be null.
+// State passing, the last kernel argument of every scan kernel template with a STATE flag (a separate argument, so ScanParams
+// keeps its layout and the STATE = false instantiations keep their instructions; they are passed zeros and never read it).
+// Rows of A_ld floats like A; this pass's states start at element 0. Forward: the state before a row's first position is h0
+// (non-null whenever STATE). Backward: h0 starts the recompute of chunk 0, dlast is the adjoint entering the row's last
+// position, dh0 receives the adjoint of h0; each may be null.
 struct ScanState {
   const float* h0;
   const float* dlast;

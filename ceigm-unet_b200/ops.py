@@ -161,10 +161,6 @@ class ScanProblem:
                 rc = _lib.lib().ss2d_scan_fwd_gated(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
                                                     _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(z), _ptr(out),
                                                     _ptr(out_z), _ptr(ckpt), _ptr(last), _stream(dev))
-            elif h0 is None:
-                rc = _lib.lib().ss2d_scan_fwd(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
-                                              _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(out), _ptr(ckpt),
-                                              _ptr(last), _stream(dev))
             else:
                 rc = _lib.lib().ss2d_scan_fwd_state(ctypes.byref(d), _ptr(self.u), _ptr(self.delta), _ptr(self.A), _ptr(self.B),
                                                     _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(out), _ptr(ckpt),
@@ -264,11 +260,6 @@ class ScanProblem:
                                            _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(z), _ptr(out), _ptr(dout), _ptr(dlast),
                                            _ptr(ckpt), _ptr(du), _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD),
                                            _ptr(dbias), _ptr(dz), _ptr(dh0), _ptr(ws), ctypes.c_size_t(ws_bytes), _stream(dev))
-            elif not stateful:
-                rc = L.ss2d_scan_bwd(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B),
-                                     _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(dout), _ptr(ckpt), _ptr(du),
-                                     _ptr(ddelta), _ptr(dA), _ptr(dB), _ptr(dC), _ptr(dD), _ptr(dbias), _ptr(ws),
-                                     ctypes.c_size_t(ws_bytes), _stream(dev))
             else:
                 rc = L.ss2d_scan_bwd_state(ctypes.byref(d), _ptr(u), _ptr(delta), _ptr(self.A), _ptr(self.B),
                                            _ptr(self.C), _ptr(self.D), _ptr(self.bias), _ptr(h0), _ptr(dout), _ptr(dlast),

@@ -98,12 +98,12 @@ def _det_launchable(name):
     return any(k in name for k in ("scan_bwd_fold_kernel", "scan_bwd_finalize_kernel", "scan_fwd", "scan_n1_fwd", "scan_par_fwd"))
 
 
-def test_deterministic_kernels_issue_no_global_atomics():
+def test_det_instantiations_with_and_without_state_issue_no_global_atomics():
     funcs = _sass_functions()
     launchable = [n for n in funcs if _det_launchable(n)]
     det_instances = [n for n in launchable if any(t in n for t in _DET_TEMPLATES)]
-    # 7 generic + 2 fast + 4 one-row + 2 rows-walking + 6 parallel-along-L instantiations
-    assert len(det_instances) == 21, det_instances
+    # 7 generic + 2 fast + 4 one-row + 2 rows-walking + 6 parallel-along-L instantiations, each with STATE = 0 and 1
+    assert len(det_instances) == 42, det_instances
     assert any("scan_bwd_fold_kernel" in n for n in launchable)
     offenders = {n: sorted(set(m.group(0) for m in _GLOBAL_ATOMIC.finditer(funcs[n]))) for n in launchable}
     offenders = {n: v for n, v in offenders.items() if v}

@@ -77,9 +77,9 @@ def test_workspace_query_does_not_depend_on_states(shape, det):
     assert _bwd(d, ws_bytes=_ws(d, 0) - 16) == ERR_WORKSPACE
 
 
-# backward kernel templates whose STATE instantiations carry their own entry names; the last template flag is DET
-_STATE_BWD = {"scan_bwd_state_kernel": 7, "scan_bwd2_state_kernel": 2, "scan_n1_bwd_state_kernel": 4,
-              "scan_n1_bwd_rows_state_kernel": 2, "scan_par_bwd_state_kernel": 6}
+# backward kernel templates whose last two template flags are STATE, DET
+_STATE_BWD = {"scan_bwd_kernel": 7, "scan_bwd2_kernel": 2, "scan_n1_bwd_kernel": 4, "scan_n1_bwd_rows_kernel": 2,
+              "scan_par_bwd_kernel": 6}
 # forward kernel templates whose last template flag is STATE
 _STATE_FWD = {"scan_fwd_kernel": 6, "scan_fwdr_kernel": 4, "scan_fwd_carry_kernel": 2, "scan_fwd_fixup_kernel": 2,
               "scan_n1_fwd_kernel": 4, "scan_par_fwd_kernel": 6}
@@ -90,9 +90,14 @@ def _split(name):
     return (m.group(1), m.group(2)) if m else (None, None)
 
 
-def test_every_state_instantiation_exists():
+def _bwd_state(name):
+    """STATE flag (second-to-last template flag) of a backward instantiation."""
+    return re.findall(r"L[a-z]+\d+E", _split(name)[1])[-2] == "Lb1E"
+
+
+def test_every_backward_template_has_its_state_instantiations():
     funcs = _sass_functions()
-    bwd = {k: [n for n in funcs if _split(n)[0] == k] for k in _STATE_BWD}
+    bwd = {k: [n for n in funcs if _split(n)[0] == k and _bwd_state(n)] for k in _STATE_BWD}
     for k, per_det in _STATE_BWD.items():
         assert len(bwd[k]) == 2 * per_det, (k, bwd[k])          # DET = 0 and 1
     for k, count in _STATE_FWD.items():
@@ -100,9 +105,9 @@ def test_every_state_instantiation_exists():
         assert len(on) == count, (k, on)
 
 
-def test_deterministic_state_kernels_issue_no_global_atomics():
+def test_state_det_instantiations_issue_no_global_atomics():
     funcs = _sass_functions()
-    det_state = [n for n in funcs if _split(n)[0] in _STATE_BWD and _split(n)[1].endswith("Lb1E")]
+    det_state = [n for n in funcs if _split(n)[0] in _STATE_BWD and _bwd_state(n) and _split(n)[1].endswith("Lb1E")]
     fwd_state = [n for n in funcs if _split(n)[0] in _STATE_FWD and _split(n)[1].endswith("Lb1E")]
     assert len(det_state) == sum(_STATE_BWD.values())
     offenders = {n: sorted(set(m.group(0) for m in _GLOBAL_ATOMIC.finditer(funcs[n]))) for n in det_state + fwd_state}
@@ -110,8 +115,8 @@ def test_deterministic_state_kernels_issue_no_global_atomics():
     assert not offenders, offenders
 
 
-def test_default_state_bwd2_still_reduces_in_l2():
+def test_state_instantiation_of_default_bwd2_still_reduces_in_l2():
     """The check above would pass vacuously if the pattern never matched: the non-deterministic STATE scan_bwd2 uses RED."""
     funcs = _sass_functions()
-    plain = [n for n in funcs if _split(n)[0] == "scan_bwd2_state_kernel" and _split(n)[1].endswith("Lb0E")]
+    plain = [n for n in funcs if _split(n)[0] == "scan_bwd2_kernel" and _bwd_state(n) and _split(n)[1].endswith("Lb0E")]
     assert plain and all(_GLOBAL_ATOMIC.search(funcs[n]) for n in plain)
