@@ -576,6 +576,8 @@ int ss2d_dwconv3_wgrad(const float* x, const float* dy, float* dweight, float* d
                        int32_t W, void* workspace, size_t workspace_bytes, ss2d_stream_t stream) {
   if (!x || !dy || !dweight) return SS2D_ERR_NULL_POINTER;
   if (batch <= 0 || C <= 0 || H <= 0 || W <= 0 || C > 65535) return SS2D_ERR_BAD_SHAPE;
+  const size_t va = (W & 3) == 0 ? 16 : 4;      // W % 4 == 0: the kernel reads x and dy as float4 pixel quads
+  if (!aligned(x, va) || !aligned(dy, va) || !aligned(dweight, 4) || !aligned(dbias, 4)) return SS2D_ERR_ALIGNMENT;
   if (!workspace || workspace_bytes < ss2d_dwconv3_wgrad_workspace_bytes(batch, C, H, W) || !aligned(workspace, 4))
     return SS2D_ERR_WORKSPACE;
   cudaError_t e = dwconv3_wgrad_launch(x, dy, dweight, dbias, static_cast<float*>(workspace), batch, C, H, W,

@@ -605,6 +605,9 @@ def dwconv3_wgrad(x: torch.Tensor, dy: torch.Tensor, want_bias: bool):
     _require(x.is_cuda and dy.is_cuda and x.dtype == torch.float32 and dy.dtype == torch.float32 and x.shape == dy.shape
              and x.dim() == 4 and x.is_contiguous() and dy.is_contiguous(), "dwconv3_wgrad: contiguous fp32 (B, C, H, W) tensors")
     Bn, C, H, W = x.shape
+    va = 16 if W % 4 == 0 else 4          # the C ABI's alignment rule; a fresh copy of a misaligned view satisfies it
+    x = x if x.data_ptr() % va == 0 else x.clone()
+    dy = dy if dy.data_ptr() % va == 0 else dy.clone()
     L = _lib.lib()
     ws_bytes = int(L.ss2d_dwconv3_wgrad_workspace_bytes(Bn, C, H, W))
     ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=x.device)

@@ -256,7 +256,8 @@ int ss2d_group_gate_bwd(const float* ys, int32_t G, const int32_t* plane_of, uin
  * dweight[c][ky][kx] = sum_(b,h,w) dy[b,c,h,w] * x[b,c,h+ky-1,w+kx-1] (zero padding 1), dbias[c] = sum dy[b,c,h,w]:
  * the backward of nn.Conv2d(D, D, groups=D, kernel_size=3, padding=1, bias=True) w.r.t. its parameters
  * (model/gm/ss2d.py:316-325, 512). x, dy: fp32 (batch, C, H, W) contiguous; dweight: (C, 1, 3, 3) fp32; dbias: (C) fp32
- * or NULL. Fully overwritten, deterministic. workspace: ss2d_dwconv3_wgrad_workspace_bytes(batch, C, H, W) bytes. */
+ * or NULL. Fully overwritten, deterministic. workspace: ss2d_dwconv3_wgrad_workspace_bytes(batch, C, H, W) bytes.
+ * x and dy 16-byte aligned when W % 4 == 0 (else 4), dweight / dbias 4-byte aligned, else SS2D_ERR_ALIGNMENT. */
 int ss2d_dwconv3_wgrad(const float* x, const float* dy, float* dweight, float* dbias, int32_t batch, int32_t C, int32_t H,
                        int32_t W, void* workspace, size_t workspace_bytes, ss2d_stream_t stream);
 size_t ss2d_dwconv3_wgrad_workspace_bytes(int32_t batch, int32_t C, int32_t H, int32_t W);
