@@ -13,7 +13,7 @@ from . import _lib, dist, functional, modules, ops                 # noqa: F401
 from ._lib import build, launch_count, version                    # noqa: F401
 from .functional import (CrossMerge, CrossMerge_1, CrossMerge_2, CrossMerge_3, CrossMerge_4, CrossScan,   # noqa: F401
                          CrossScan_1, CrossScan_2, CrossScan_3, CrossScan_4, SelectiveScanCore, SelectiveScanOflex,
-                         selective_scan)
+                         selective_scan, selective_state_update)
 from .modules import SS2D, GroupMambaLayer, LayerNormRows, PVT2FFN, custom_ffn, mamba_init             # noqa: F401
 
 

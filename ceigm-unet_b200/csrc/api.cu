@@ -19,6 +19,8 @@ bool scan_fwdr_try(const ScanParams& p, const ScanState& st, const ScanGate& gt,
 cudaError_t scan_gate_fwd_launch(const ss2d_scan_desc* d, const void* y, const void* z, void* out_z, cudaStream_t s);
 cudaError_t scan_gate_bwd_launch(const ss2d_scan_desc* d, const void* dout_z, const void* z, const void* y, float* dy, void* dz,
                                  cudaStream_t s);
+// one recurrent step (state_update.cu)
+cudaError_t ssm_step_launch(const StepParams& p, int io_dtype, cudaStream_t stream);
 constexpr int kDwnMaxSeg = 4;
 struct DwnSegs { int nseg; int cbeg[kDwnMaxSeg + 1]; int k[kDwnMaxSeg]; const float* w[kDwnMaxSeg]; const float* b[kDwnMaxSeg]; };
 cudaError_t dwnhwc_stencil_launch(const void* x, const void* aux, void* y, const DwnSegs& sg, int flip, int epi, int B, int H,
@@ -445,6 +447,31 @@ int ss2d_scan_bwd_state(const ss2d_scan_desc* d, const void* u, const void* delt
       ++g_launches;
     }
   }
+  return SS2D_OK;
+}
+
+int ss2d_state_update(const ss2d_step_desc* d, float* state, const void* x, const void* dt, const float* A, const void* Bmat,
+                      const void* Cmat, const float* Dvec, const float* dt_bias, const void* z, void* out, ss2d_stream_t stream) {
+  if (!d) return SS2D_ERR_NULL_POINTER;
+  if (d->batch <= 0 || d->dim <= 0 || d->dstate <= 0 || d->n_groups <= 0 || d->dim % d->n_groups != 0) return SS2D_ERR_BAD_SHAPE;
+  if (d->dstate > SS2D_MAX_DSTATE) return SS2D_ERR_DSTATE;
+  if (!dtype_ok(d->io_dtype) || (d->dt_softplus != 0 && d->dt_softplus != 1)) return SS2D_ERR_BAD_DTYPE;
+  if (!state || !x || !dt || !A || !Bmat || !Cmat || !out) return SS2D_ERR_NULL_POINTER;
+  const size_t es = esize(d->io_dtype);
+  if (!aligned(state, 16) || !aligned(x, es) || !aligned(dt, es) || !aligned(Bmat, es) || !aligned(Cmat, es) || !aligned(z, es) ||
+      !aligned(out, es) || !aligned(A, 4) || !aligned(Dvec, 4) || !aligned(dt_bias, 4))
+    return SS2D_ERR_ALIGNMENT;
+  StepParams p;
+  p.state = state; p.x = x; p.dt = dt; p.B = Bmat; p.C = Cmat; p.z = z;
+  p.A = A; p.D = Dvec; p.bias = dt_bias; p.out = out;
+  p.rows = (int64_t)d->batch * d->dim;
+  p.dim = d->dim; p.dstate = d->dstate; p.dpg = d->dim / d->n_groups; p.softplus = d->dt_softplus;
+  p.io_bs = d->io_batch_stride;
+  p.B_bs = d->B_batch_stride; p.B_gs = d->B_group_stride;
+  p.C_bs = d->C_batch_stride; p.C_gs = d->C_group_stride;
+  const cudaError_t e = ssm_step_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  ++g_launches;
   return SS2D_OK;
 }
 

@@ -63,6 +63,17 @@ struct ScanGate {
   const void* z;
   void* out_z;
 };
+// One recurrent step (ss2d_state_update, csrc/state_update.cu); strides in elements, innermost stride 1.
+struct StepParams {
+  float* state;                      // [batch][dim][dstate]
+  const void *x, *dt, *B, *C, *z;    // z may be null
+  const float *A, *D, *bias;         // D, bias may be null
+  void* out;
+  int64_t rows;                      // batch * dim
+  int dim, dstate, dpg, softplus;    // dpg = dim / n_groups
+  int64_t io_bs, B_bs, B_gs, C_bs, C_gs;
+};
+
 // backward: the STATE instantiation runs when any of the three pointers is set
 inline bool has_state(const ScanState& st) { return st.h0 || st.dlast || st.dh0; }
 

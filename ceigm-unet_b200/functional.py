@@ -107,6 +107,23 @@ def selective_scan(u, delta, A, B, C, D=None, delta_bias=None, delta_softplus=Fa
     return (out, last) if return_last_state else out
 
 
+def selective_state_update(state, x, dt, A, B, C, D=None, z=None, dt_bias=None, dt_softplus=False):
+    """One recurrent step of the selective scan with mamba_ssm's `selective_state_update` arguments; `state` is updated in place.
+
+        t = dt + dt_bias (softplus(t) when dt_softplus),  state = exp(t A) * state + t x B,  out = C . state + D x  (* silu(z))
+
+    state: fp32 (batch, dim, dstate), contiguous (the layout of `selective_scan`'s final state: a prefill's `last_state` is
+    stepped from directly). x, dt, z: (batch, dim); B, C: (batch, dstate) or (batch, n_groups, dstate), all of one dtype (fp32 /
+    fp16 / bf16); A: fp32 (dim, dstate); D, dt_bias: fp32 (dim) or None. Returns out (batch, dim) in x's dtype.
+    Inference only, like mamba_ssm's function: with grad mode on, no input may require grad (train with `selective_scan`)."""
+    if torch.is_grad_enabled():
+        for name, t in (("state", state), ("x", x), ("dt", dt), ("A", A), ("B", B), ("C", C), ("D", D), ("z", z),
+                        ("dt_bias", dt_bias)):
+            if t is not None and t.requires_grad:
+                raise RuntimeError(f"selective_state_update has no backward, but {name} requires grad: run it under torch.no_grad()")
+    return ops.state_update(state, x, dt, A, B, C, D, z, dt_bias, dt_softplus)
+
+
 # ---- cross scan / merge ---------------------------------------------------------------------------
 def _make_cross_pair(dirs, suffix):
     dirs = tuple(dirs)

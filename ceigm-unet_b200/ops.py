@@ -274,6 +274,51 @@ class ScanProblem:
         return grads + [dh0] if stateful else grads
 
 
+# ---- recurrent step ----------------------------------------------------------------------------
+def state_update(state, x, dt, A, B, C, D=None, z=None, dt_bias=None, dt_softplus=False) -> torch.Tensor:
+    """One step of the selective scan, `state` updated in place (ss2d_state_update) -> out (batch, dim) in x's dtype.
+    state: fp32 (batch, dim, dstate) contiguous, 16-byte aligned; x, dt, z: (batch, dim); B, C: (batch, dstate) or
+    (batch, n_groups, dstate), all of x's dtype; A: fp32 (dim, dstate) contiguous; D, dt_bias: fp32 (dim) or None.
+    x, dt and z are made contiguous unless they already are (the C ABI gives them one shared row stride)."""
+    _require(x.dtype in _DT, "x must be float32, float16 or bfloat16")
+    for name, t in (("state", state), ("x", x), ("dt", dt), ("A", A), ("B", B), ("C", C), ("D", D), ("z", z), ("dt_bias", dt_bias)):
+        if t is not None:
+            _require(t.is_cuda, f"Expected {name}.is_cuda() to be true")
+            _require(t.device == state.device, f"{name} must be on the device of state")
+    _require(state.dtype == torch.float32 and state.dim() == 3, "state must be a float32 (batch, dim, dstate) tensor")
+    batch, dim, N = state.shape
+    _require(state.is_contiguous() and state.data_ptr() % 16 == 0, "state must be contiguous and 16-byte aligned (it is updated in place)")
+    _require(N <= _lib.MAX_DSTATE, "selective_state_update only supports state dimension <= 256")
+    _require(A.dtype == torch.float32 and tuple(A.shape) == (dim, N) and A.is_contiguous(), "A must be a contiguous float32 (dim, dstate) tensor")
+    for name, t in (("x", x), ("dt", dt), ("z", z)):
+        if t is not None:
+            _require(t.dtype == x.dtype and tuple(t.shape) == (batch, dim), f"{name} must be (batch, dim) of x's dtype")
+    if B.dim() == 2:
+        B, C = B.unsqueeze(1), C.unsqueeze(1)
+    _require(B.dim() == 3 and tuple(C.shape) == tuple(B.shape), "B and C must both be (batch, dstate) or (batch, n_groups, dstate)")
+    G = B.shape[1]
+    _require(tuple(B.shape) == (batch, G, N) and G > 0 and dim % G == 0, "B and C must be (batch, n_groups, dstate), dim % n_groups == 0")
+    _require(B.dtype == x.dtype and C.dtype == x.dtype, "B and C must have x's dtype")
+    for name, t in (("D", D), ("dt_bias", dt_bias)):
+        if t is not None:
+            _require(t.dtype == torch.float32 and tuple(t.shape) == (dim,) and t.is_contiguous(), f"{name} must be a contiguous float32 (dim,) tensor")
+    B = B if B.stride(-1) == 1 else B.contiguous()
+    C = C if C.stride(-1) == 1 else C.contiguous()
+    x, dt = x.contiguous(), dt.contiguous()
+    z = None if z is None else z.contiguous()
+    out = torch.empty((batch, dim), dtype=x.dtype, device=x.device)
+    d = _lib.StepDesc()
+    d.batch, d.dim, d.dstate, d.n_groups = batch, dim, N, G
+    d.io_dtype, d.dt_softplus, d.io_batch_stride = _DT[x.dtype], int(bool(dt_softplus)), dim
+    d.B_batch_stride, d.B_group_stride = B.stride(0), B.stride(1)
+    d.C_batch_stride, d.C_group_stride = C.stride(0), C.stride(1)
+    with torch.cuda.device(state.device):
+        rc = _lib.lib().ss2d_state_update(ctypes.byref(d), _ptr(state), _ptr(x), _ptr(dt), _ptr(A), _ptr(B), _ptr(C), _ptr(D),
+                                          _ptr(dt_bias), _ptr(z), _ptr(out), _stream(state.device))
+    _lib.check(rc, "ss2d_state_update")
+    return out
+
+
 # ---- stand-alone permutations ------------------------------------------------------------------
 def cross_scan(x: torch.Tensor, dirs: Sequence[int]) -> torch.Tensor:
     """x (B, C, H, W) -> (B, K, C, H*W), plane k traversed in direction dirs[k] (csms6s.py:11-206)."""

@@ -179,6 +179,35 @@ int ss2d_scan_bwd_gated(const ss2d_scan_desc* desc, const void* u, const void* d
                         float* ddelta_bias, void* dz, float* dh0, void* workspace, size_t workspace_bytes,
                         ss2d_stream_t stream);
 
+/* ---- recurrent step: advance a saved state by one position (mamba_ssm's selective_state_update) ------------------
+ * Per (b, d, n), g = d / (dim / n_groups), all in fp32:
+ *   t = dt[b,d] + dt_bias[d], then t = softplus(t) (threshold 20) when dt_softplus;
+ *   state[b,d,n] = exp(t A[d,n]) state[b,d,n] + t x[b,d] B[b,g,n]      (in place);
+ *   out[b,d] = sum_n C[b,g,n] state[b,d,n] + D[d] x[b,d], times silu(z[b,d]) when z != NULL; rounded once to the io dtype.
+ * state: fp32 (batch, dim, dstate), contiguous, 16-byte aligned: the layout of last_state / h0 / dh0 above, so a scan's final
+ *   state is a step's input and the other way round. A: fp32 (dim, dstate) contiguous. Dvec, dt_bias: fp32 (dim) or NULL.
+ * x, dt, z, out: (batch, dim) of io_dtype, element (b, d) at b * io_batch_stride + d. B, C: (batch, n_groups, dstate) of
+ *   io_dtype, element (b, g, n) at b * X_batch_stride + g * X_group_stride + n. z may be NULL.
+ * Errors, returned before any launch: SS2D_ERR_NULL_POINTER (desc, state, x, dt, A, B, C or out NULL), SS2D_ERR_BAD_SHAPE
+ * (a size <= 0, dim % n_groups != 0), SS2D_ERR_DSTATE (dstate > SS2D_MAX_DSTATE), SS2D_ERR_BAD_DTYPE (io_dtype, or
+ * dt_softplus not 0 / 1), SS2D_ERR_ALIGNMENT (state not 16-byte aligned, an io pointer not aligned to its element size, A / D /
+ * dt_bias not 4-byte aligned). One kernel, no atomics: the results are bit-identical across calls and CUDA-graph replays. */
+typedef struct ss2d_step_desc {
+  int32_t batch;
+  int32_t dim;
+  int32_t dstate;
+  int32_t n_groups;
+  int32_t io_dtype;        /* ss2d_dtype of x, dt, B, C, z, out */
+  int32_t dt_softplus;     /* 1: t = softplus(dt + dt_bias), threshold 20 */
+  /* element strides */
+  int64_t io_batch_stride; /* x, dt, z, out */
+  int64_t B_batch_stride, B_group_stride;
+  int64_t C_batch_stride, C_group_stride;
+} ss2d_step_desc;
+int ss2d_state_update(const ss2d_step_desc* desc, float* state, const void* x, const void* dt, const float* A,
+                      const void* Bmat, const void* Cmat, const float* Dvec, const float* dt_bias, const void* z,
+                      void* out, ss2d_stream_t stream);
+
 /* ---- stand-alone cross-scan / cross-merge (exact permutations; model/gm/csms6s.py:11-206) ----
  * cross_scan : x (batch, channels, H, W) -> xs (batch, K, channels, L), xs[:,k] in direction dirs[k].
  * cross_merge: ys (batch, K, channels, L) in scan order -> y (batch, channels, L) natural order,
