@@ -448,6 +448,8 @@ int gate_proj_tc_launch(const float* ys, int K, unsigned tmask, const float* lnw
   if (!ys || (C > 0 && (!W || !out)) || (C == 0 && !g_out)) return SS2D_ERR_NULL_POINTER;
   if (batch <= 0 || L <= 0 || H <= 0 || Wd <= 0 || (int64_t)H * Wd != L) return SS2D_ERR_BAD_SHAPE;
   if (!gate_proj_tc_supported(D, C, K, dtype) || (lnb && !lnw)) return SS2D_ERR_UNSUPPORTED;
+  if ((H & 3) || (Wd & 3)) return SS2D_ERR_UNSUPPORTED;          // the plane boxes' tensor maps need 16-byte row strides
+  if ((C > 0 && out_rs < C) || (z && z_rs < D) || (g_out && g_rs < D)) return SS2D_ERR_BAD_LAYOUT;   // overlapping rows
   const int esize = dtype == SS2D_F32 ? 4 : 2;
   auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
   if ((C > 0 && (!al16(out) || ((out_rs * esize) & 15))) || (z && (!al16(z) || ((z_rs * esize) & 15))) || (g_out && (!al16(g_out) || ((g_rs * esize) & 15))) ||

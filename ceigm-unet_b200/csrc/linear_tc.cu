@@ -285,6 +285,7 @@ int linear_tc_launch(const void* A, int64_t lda, const void* W, int64_t ldw, con
   if (!A || !W || !parts) return SS2D_ERR_NULL_POINTER;
   if (M <= 0 || N <= 0 || K <= 0 || n_parts <= 0 || n_parts > TC_MAX_PARTS) return SS2D_ERR_BAD_SHAPE;
   if (dtype != SS2D_F32 && dtype != SS2D_BF16) return SS2D_ERR_BAD_DTYPE;
+  if (lda < K || ldw < K) return SS2D_ERR_BAD_LAYOUT;            // rows of A / W would overlap
   const int esize = dtype == SS2D_F32 ? 4 : 2;
   TcParams p;
   memset(&p, 0, sizeof(p));
@@ -299,15 +300,20 @@ int linear_tc_launch(const void* A, int64_t lda, const void* W, int64_t ldw, con
     if (!q.out) return SS2D_ERR_NULL_POINTER;
     if (!linear_tc_supported(q.n_cols, K, dtype)) return SS2D_ERR_UNSUPPORTED;
     if (q.planes_L < 0 || (q.planes_L > 0 && M % q.planes_L != 0)) return SS2D_ERR_BAD_SHAPE;
+    if (q.planes_L == 0 && q.ld < q.n_cols) return SS2D_ERR_BAD_LAYOUT;     // output rows would overlap
     if (q.planes_L == 0 && ((q.ld * esize) & 15 || (reinterpret_cast<uintptr_t>(q.out) & 15))) return SS2D_ERR_ALIGNMENT;
     p.part[i].out = q.out; p.part[i].ld = q.ld; p.part[i].n0 = n0; p.part[i].n = q.n_cols;
     p.part[i].planes_L = q.planes_L; p.part[i].act = q.act;
-    if (!tc_make_map(&maps.w[i], static_cast<const char*>(W) + (size_t)n0 * ldw * esize, esize, K, q.n_cols, ldw, q.n_cols))
-      return SS2D_ERR_ALIGNMENT;
     n0 += q.n_cols;
     nmax = q.n_cols > nmax ? q.n_cols : nmax;
   }
   if (n0 != N) return SS2D_ERR_BAD_SHAPE;
+  // tensor maps only once every argument has been validated: their creation is the one check whose outcome depends on the driver
+  for (int i = 0; i < n_parts; ++i) {
+    const TcPart& q = p.part[i];
+    if (!tc_make_map(&maps.w[i], static_cast<const char*>(W) + (size_t)q.n0 * ldw * esize, esize, K, q.n, ldw, q.n))
+      return SS2D_ERR_ALIGNMENT;
+  }
   if (!tc_make_map(&maps.a, A, esize, K, M, lda, TC_BM)) return SS2D_ERR_ALIGNMENT;
   p.acc_stride = nmax <= 16 ? 16 : nmax <= 32 ? 32 : nmax <= 64 ? 64 : nmax <= 128 ? 128 : 256;
   const size_t w_bytes = ((size_t)p.kblocks * nmax * 128 + 1023) & ~(size_t)1023;

@@ -581,9 +581,10 @@ def linear_tc(x: torch.Tensor, W: torch.Tensor, bias, parts):
     K = x.shape[-1]
     N = W.shape[0]
     x2 = x.reshape(-1, K)
-    if x2.stride(1) != 1:
+    if x2.stride(1) != 1 or x2.stride(0) < K:         # the kernel rejects overlapping rows (e.g. a broadcast x)
         x2 = x2.contiguous()
-    _require(W.dim() == 2 and W.shape[1] == K and W.stride(1) == 1, "linear_tc: W must be (N, K) with unit inner stride")
+    _require(W.dim() == 2 and W.shape[1] == K and W.stride(1) == 1 and W.stride(0) >= K,
+             "linear_tc: W must be (N, K) with unit inner stride and non-overlapping rows")
     M = x2.shape[0]
     _require(sum(p[0] for p in parts) == N, "linear_tc: the parts must cover the N columns")
     arr = (_lib.LinearPart * len(parts))()

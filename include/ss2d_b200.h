@@ -368,7 +368,8 @@ size_t ss2d_wgrad_ts_workspace_bytes(int32_t batch, int32_t rows, int32_t M, int
  * accumulation in tensor memory), A streamed once by TMA, W resident in shared memory.
  * A: (M, K) rows lda elements apart; W: (N, K) rows ldw elements apart (nn.Linear's weight layout); bias: (N) fp32 or NULL.
  * dtype: SS2D_F32 or SS2D_BF16, the type of A, W and every output. A, W and row-major outputs 16-byte aligned with
- * row strides that are multiples of 16 bytes, else SS2D_ERR_ALIGNMENT.
+ * row strides that are multiples of 16 bytes, else SS2D_ERR_ALIGNMENT. Rows must not overlap: lda < K, ldw < K or a
+ * row-major part with ld < n_cols is SS2D_ERR_BAD_LAYOUT.
  * The N columns are cut into n_parts <= 4 consecutive parts of n_cols columns each (16 <= n_cols <= 256, multiple of 16;
  * ss2d_linear_tc_supported(n_cols, K, dtype) tells whether W's part fits next to the A ring in shared memory):
  *   planes_L == 0: row-major part, out[m * ld + c];
@@ -397,8 +398,9 @@ int32_t ss2d_linear_tc_supported(int32_t n_cols, int32_t K, int32_t dtype);
  * g_out: optional (batch * L, D) rows: the gated tensor (what out_proj's weight gradient needs); mean_rstd: optional
  * (batch * L, 2) fp32 for ss2d_out_gate_bwd. ln_weight / ln_bias as for ss2d_out_gate_fwd (a bias without a weight:
  * SS2D_ERR_UNSUPPORTED). D % 64 == 0, C % 16 == 0, C <= 256, operand tile + weight within shared memory
- * (ss2d_gate_proj_supported); H % 4 == 0 and Wd % 4 == 0 (the planes are read as TMA boxes); all row pointers / strides
- * 16-byte aligned.
+ * (ss2d_gate_proj_supported); H % 4 == 0 and Wd % 4 == 0 (the planes are read as TMA boxes), else SS2D_ERR_UNSUPPORTED;
+ * all row pointers / strides 16-byte aligned. Rows must not overlap: out_row_stride < C (C > 0), z_row_stride < D (z given)
+ * or g_row_stride < D (g_out given) is SS2D_ERR_BAD_LAYOUT.
  * C == 0 (W = NULL, out = NULL): epilogue only — the kernel stops after the gate and g_out (required) receives what
  * ss2d_out_gate_fwd would write; the TMA-fed alternative to that kernel for 4-aligned images. */
 int ss2d_gate_proj_fwd(const float* ys, int32_t K, uint32_t transposed_mask, const float* ln_weight, const float* ln_bias, float eps,
