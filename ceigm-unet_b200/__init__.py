@@ -3,7 +3,8 @@
 Layers (SURVEY.md §8b):
   b1  dropin/selective_scan_cuda_core.py, dropin/selective_scan_cuda_oflex.py, dropin/selective_scan_cuda.py (mamba_ssm's
       module, with the z gate) — the reference extension modules' `fwd` / `bwd` functions; `install_dropin()` registers them
-      in sys.modules so that the reference's own `model/gm/csms6s.py` picks them up unchanged.
+      in sys.modules so that the reference's own `model/gm/csms6s.py` picks them up unchanged. dropin/causal_conv1d_cuda.py and
+      dropin/causal_conv1d.py serve causal-conv1d 1.1.x, the convolution in front of every Mamba block's scan.
   b2  functional.py — SelectiveScanCore/Oflex, CrossScan[_k], CrossMerge[_k] autograd Functions.
   b3  modules.py — SS2D, GroupMambaLayer (and the FFNs next to them: PVT2FFN, custom_ffn) with the reference's state_dict.
 Underneath: ops.py -> _lib.py (ctypes) -> libss2d_b200.so (csrc/*.cu, C ABI in include/ss2d_b200.h).
@@ -13,7 +14,7 @@ from . import _lib, dist, functional, modules, ops                 # noqa: F401
 from ._lib import build, launch_count, version                    # noqa: F401
 from .functional import (CrossMerge, CrossMerge_1, CrossMerge_2, CrossMerge_3, CrossMerge_4, CrossScan,   # noqa: F401
                          CrossScan_1, CrossScan_2, CrossScan_3, CrossScan_4, SelectiveScanCore, SelectiveScanOflex,
-                         selective_scan, selective_state_update)
+                         causal_conv1d_fn, causal_conv1d_update, selective_scan, selective_state_update)
 from .modules import SS2D, GroupMambaLayer, LayerNormRows, PVT2FFN, custom_ffn, mamba_init             # noqa: F401
 
 
@@ -40,10 +41,13 @@ def graphed(module, sample_args, num_warmup_iters: int = 3):
 def install_dropin() -> None:
     """Make `import selective_scan_cuda_core` / `selective_scan_cuda_oflex` / `selective_scan_cuda` (mamba_ssm's module)
     resolve to this package's modules (the reference imports them at module import time inside try/except:
-    model/gm/csms6s.py:209-220)."""
+    model/gm/csms6s.py:209-220), and `import causal_conv1d_cuda` / `from causal_conv1d import causal_conv1d_fn,
+    causal_conv1d_update` (mamba_ssm's convolution) too."""
     import sys
 
-    from .dropin import selective_scan_cuda, selective_scan_cuda_core, selective_scan_cuda_oflex
+    from .dropin import causal_conv1d, causal_conv1d_cuda, selective_scan_cuda, selective_scan_cuda_core, selective_scan_cuda_oflex
     sys.modules["selective_scan_cuda_core"] = selective_scan_cuda_core
     sys.modules["selective_scan_cuda_oflex"] = selective_scan_cuda_oflex
     sys.modules["selective_scan_cuda"] = selective_scan_cuda
+    sys.modules["causal_conv1d_cuda"] = causal_conv1d_cuda
+    sys.modules["causal_conv1d"] = causal_conv1d

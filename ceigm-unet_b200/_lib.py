@@ -23,6 +23,7 @@ EXPORTS = [
     "ss2d_scan_fwd", "ss2d_scan_ckpt_floats", "ss2d_scan_bwd", "ss2d_scan_bwd_workspace_bytes",
     "ss2d_scan_fwd_state", "ss2d_scan_bwd_state",
     "ss2d_scan_fwd_gated", "ss2d_scan_bwd_gated", "ss2d_scan_bwd_gated_workspace_bytes", "ss2d_state_update",
+    "ss2d_conv1d_fwd", "ss2d_conv1d_bwd", "ss2d_conv1d_bwd_workspace_bytes", "ss2d_conv1d_update",
     "ss2d_cross_scan", "ss2d_cross_merge", "ss2d_out_gate_fwd", "ss2d_out_gate_bwd",
     "ss2d_out_gate_bwd_partials", "ss2d_group_gate_fwd", "ss2d_group_gate_bwd", "ss2d_out_gate_max_width", "ss2d_wgrad_ts", "ss2d_wgrad_ts_workspace_bytes",
     "ss2d_layernorm_fwd", "ss2d_layernorm_bwd", "ss2d_layernorm_bwd_partials",
@@ -54,6 +55,16 @@ class StepDesc(ctypes.Structure):
         ("io_dtype", ctypes.c_int32), ("dt_softplus", ctypes.c_int32), ("io_batch_stride", ctypes.c_int64),
         ("B_batch_stride", ctypes.c_int64), ("B_group_stride", ctypes.c_int64),
         ("C_batch_stride", ctypes.c_int64), ("C_group_stride", ctypes.c_int64),
+    ]
+
+
+class Conv1dDesc(ctypes.Structure):
+    """Mirror of `ss2d_conv1d_desc` (include/ss2d_b200.h)."""
+    _fields_ = [
+        ("batch", ctypes.c_int32), ("dim", ctypes.c_int32), ("seqlen", ctypes.c_int32), ("width", ctypes.c_int32),
+        ("io_dtype", ctypes.c_int32), ("silu", ctypes.c_int32),
+        ("x_batch_stride", ctypes.c_int64), ("x_dim_stride", ctypes.c_int64),
+        ("out_batch_stride", ctypes.c_int64), ("out_dim_stride", ctypes.c_int64),
     ]
 
 
@@ -111,6 +122,15 @@ def lib() -> ctypes.CDLL:
     L.ss2d_scan_bwd_workspace_bytes.restype = sz
     L.ss2d_state_update.argtypes = [ctypes.POINTER(StepDesc), fp, vp, vp, fp, vp, vp, fp, fp, vp, vp, vp]
     L.ss2d_state_update.restype = ctypes.c_int
+    cd = ctypes.POINTER(Conv1dDesc)
+    L.ss2d_conv1d_fwd.argtypes = [cd, vp, fp, fp, vp, vp]
+    L.ss2d_conv1d_fwd.restype = ctypes.c_int
+    L.ss2d_conv1d_bwd_workspace_bytes.argtypes = [cd]
+    L.ss2d_conv1d_bwd_workspace_bytes.restype = sz
+    L.ss2d_conv1d_bwd.argtypes = [cd, vp, fp, fp, vp, vp, fp, fp, vp, sz, vp]
+    L.ss2d_conv1d_bwd.restype = ctypes.c_int
+    L.ss2d_conv1d_update.argtypes = [cd, vp, vp, fp, fp, vp, vp]
+    L.ss2d_conv1d_update.restype = ctypes.c_int
     ip = ctypes.POINTER(ctypes.c_int32)
     L.ss2d_cross_scan.argtypes = [vp, vp, i32, i32, i32, i32, i32, ip, i32, vp]
     L.ss2d_cross_scan.restype = ctypes.c_int

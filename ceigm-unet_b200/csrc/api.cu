@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstring>
 
+#include "conv1d_params.h"
 #include "scan_params.h"
 #include "ss2d_b200.h"
 
@@ -21,6 +22,11 @@ cudaError_t scan_gate_bwd_launch(const ss2d_scan_desc* d, const void* dout_z, co
                                  cudaStream_t s);
 // one recurrent step (state_update.cu)
 cudaError_t ssm_step_launch(const StepParams& p, int io_dtype, cudaStream_t stream);
+// causal depthwise conv1d (causal_conv1d.cu)
+int conv1d_bwd_slabs(int batch, int dim, int64_t L);
+cudaError_t conv1d_fwd_launch(const Conv1dParams& p, int io_dtype, cudaStream_t stream);
+cudaError_t conv1d_bwd_launch(const Conv1dParams& p, int io_dtype, cudaStream_t stream);
+cudaError_t conv1d_update_launch(const Conv1dParams& p, int io_dtype, cudaStream_t stream);
 constexpr int kDwnMaxSeg = 4;
 struct DwnSegs { int nseg; int cbeg[kDwnMaxSeg + 1]; int k[kDwnMaxSeg]; const float* w[kDwnMaxSeg]; const float* b[kDwnMaxSeg]; };
 cudaError_t dwnhwc_stencil_launch(const void* x, const void* aux, void* y, const DwnSegs& sg, int flip, int epi, int B, int H,
@@ -470,6 +476,83 @@ int ss2d_state_update(const ss2d_step_desc* d, float* state, const void* x, cons
   p.B_bs = d->B_batch_stride; p.B_gs = d->B_group_stride;
   p.C_bs = d->C_batch_stride; p.C_gs = d->C_group_stride;
   const cudaError_t e = ssm_step_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  ++g_launches;
+  return SS2D_OK;
+}
+
+static int conv1d_validate(const ss2d_conv1d_desc* d, bool update) {
+  if (!d) return SS2D_ERR_NULL_POINTER;
+  if (d->batch <= 0 || d->dim <= 0 || d->seqlen <= 0 || d->width < 2 || d->width > 4 || (update && d->seqlen != 1))
+    return SS2D_ERR_BAD_SHAPE;
+  if (!dtype_ok(d->io_dtype) || (d->silu != 0 && d->silu != 1)) return SS2D_ERR_BAD_DTYPE;
+  if (d->x_batch_stride < 0 || d->x_dim_stride < 0 || d->out_dim_stride < (update ? 1 : d->seqlen) ||
+      d->out_batch_stride < (int64_t)d->dim * d->out_dim_stride)
+    return SS2D_ERR_BAD_LAYOUT;
+  return SS2D_OK;
+}
+
+static Conv1dParams conv1d_params(const ss2d_conv1d_desc* d, const void* x, const float* weight, const float* bias) {
+  Conv1dParams p = {};
+  p.x = x; p.w = weight; p.bias = bias;
+  p.x_bs = d->x_batch_stride; p.x_ds = d->x_dim_stride;
+  p.o_bs = d->out_batch_stride; p.o_ds = d->out_dim_stride;
+  p.L = d->seqlen; p.batch = d->batch; p.dim = d->dim; p.width = d->width; p.silu = d->silu;
+  return p;
+}
+
+int ss2d_conv1d_fwd(const ss2d_conv1d_desc* d, const void* x, const float* weight, const float* bias, void* out,
+                    ss2d_stream_t stream) {
+  const int v = conv1d_validate(d, false);
+  if (v != SS2D_OK) return v;
+  if (!x || !weight || !out) return SS2D_ERR_NULL_POINTER;
+  const size_t es = esize(d->io_dtype);
+  if (!aligned(x, es) || !aligned(out, es) || !aligned(weight, 4) || !aligned(bias, 4)) return SS2D_ERR_ALIGNMENT;
+  Conv1dParams p = conv1d_params(d, x, weight, bias);
+  p.out = out;
+  const cudaError_t e = conv1d_fwd_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  ++g_launches;
+  return SS2D_OK;
+}
+
+size_t ss2d_conv1d_bwd_workspace_bytes(const ss2d_conv1d_desc* d) {
+  if (conv1d_validate(d, false) != SS2D_OK) return 0;
+  const int slabs = conv1d_bwd_slabs(d->batch, d->dim, d->seqlen);
+  return slabs > 1 ? (size_t)d->dim * slabs * (d->width + 1) * sizeof(float) : 0;
+}
+
+int ss2d_conv1d_bwd(const ss2d_conv1d_desc* d, const void* x, const float* weight, const float* bias, const void* dout,
+                    void* dx, float* dweight, float* dbias, void* workspace, size_t workspace_bytes, ss2d_stream_t stream) {
+  const int v = conv1d_validate(d, false);
+  if (v != SS2D_OK) return v;
+  if (!x || !weight || !dout || !dx || !dweight) return SS2D_ERR_NULL_POINTER;
+  const size_t es = esize(d->io_dtype);
+  if (!aligned(x, es) || !aligned(dout, es) || !aligned(dx, es) || !aligned(weight, 4) || !aligned(bias, 4) ||
+      !aligned(dweight, 4) || !aligned(dbias, 4) || !aligned(workspace, 4))
+    return SS2D_ERR_ALIGNMENT;
+  const size_t need = ss2d_conv1d_bwd_workspace_bytes(d);
+  if (need > 0 && (!workspace || workspace_bytes < need)) return SS2D_ERR_WORKSPACE;
+  Conv1dParams p = conv1d_params(d, x, weight, bias);
+  p.dout = dout; p.out = dx; p.dw = dweight; p.db = dbias; p.part = static_cast<float*>(workspace);
+  p.slabs = conv1d_bwd_slabs(d->batch, d->dim, d->seqlen);
+  const cudaError_t e = conv1d_bwd_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  g_launches += p.slabs > 1 ? 2 : 1;
+  return SS2D_OK;
+}
+
+int ss2d_conv1d_update(const ss2d_conv1d_desc* d, const void* x, void* conv_state, const float* weight, const float* bias,
+                       void* out, ss2d_stream_t stream) {
+  const int v = conv1d_validate(d, true);
+  if (v != SS2D_OK) return v;
+  if (!x || !conv_state || !weight || !out) return SS2D_ERR_NULL_POINTER;
+  const size_t es = esize(d->io_dtype);
+  if (!aligned(x, es) || !aligned(conv_state, es) || !aligned(out, es) || !aligned(weight, 4) || !aligned(bias, 4))
+    return SS2D_ERR_ALIGNMENT;
+  Conv1dParams p = conv1d_params(d, x, weight, bias);
+  p.state = conv_state; p.out = out;
+  const cudaError_t e = conv1d_update_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e);
   ++g_launches;
   return SS2D_OK;

@@ -124,6 +124,53 @@ def selective_state_update(state, x, dt, A, B, C, D=None, z=None, dt_bias=None, 
     return ops.state_update(state, x, dt, A, B, C, D, z, dt_bias, dt_softplus)
 
 
+# ---- causal depthwise conv1d (the causal-conv1d 1.1.x interface) ----------------------------------
+def _silu_flag(activation):
+    if activation not in (None, "silu", "swish"):
+        raise NotImplementedError("activation must be None, silu, or swish")      # a RuntimeError, as in causal-conv1d
+    return activation is not None
+
+
+class _CausalConv1d(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, bias, silu):
+        ctx.save_for_backward(x, weight, bias)
+        ctx.silu = silu
+        return ops.conv1d_fwd(x, weight, bias, silu)
+
+    @staticmethod
+    def backward(ctx, dout):
+        x, weight, bias = ctx.saved_tensors
+        dx, dweight, dbias = ops.conv1d_bwd(x, weight, bias, dout, ctx.silu)
+        return dx, dweight, dbias, None
+
+
+def causal_conv1d_fn(x, weight, bias=None, seq_idx=None, activation=None):
+    """Causal depthwise conv1d with causal-conv1d's arguments, differentiable in x, weight and bias:
+
+        out[b,d,l] = act(bias[d] + sum_{k<width} weight[d,k] x[b,d,l-(width-1)+k]),  x = 0 before position 0,
+
+    that is nn.Conv1d(dim, dim, width, groups=dim, padding=width-1)(x)[..., :L] then act: SiLU for "silu" / "swish", none for None.
+    x: (batch, dim, L) fp32 / fp16 / bf16 with stride 1 along L; weight: (dim, width), 2 <= width <= 4; bias: (dim) or None, of
+    weight's dtype (fp32 parameters with a bf16 x, as under autocast, are fine). Math in fp32; out has x's dtype. seq_idx and
+    channel-last x are not supported (RuntimeError)."""
+    if seq_idx is not None:
+        raise RuntimeError("causal_conv1d_fn: seq_idx is not supported")
+    return _CausalConv1d.apply(x, weight, bias, _silu_flag(activation))
+
+
+def causal_conv1d_update(x, conv_state, weight, bias=None, activation=None):
+    """One decode position with causal-conv1d's arguments: conv_state (batch, dim, width) of x's dtype is shifted left by one in
+    place and x (batch, dim) stored in its last slot; returns act(bias + sum_k weight[:, k] conv_state[..., k]) (batch, dim).
+    After a prefill over L positions, conv_state = F.pad(x, (width - L, 0)) holds the last width inputs, and step t returns the
+    forward over L + t + 1 positions at position L + t. Inference only: with grad mode on, no input may require grad."""
+    if torch.is_grad_enabled():
+        for name, t in (("x", x), ("conv_state", conv_state), ("weight", weight), ("bias", bias)):
+            if t is not None and t.requires_grad:
+                raise RuntimeError(f"causal_conv1d_update has no backward, but {name} requires grad: run it under torch.no_grad()")
+    return ops.conv1d_update(x, conv_state, weight, bias, _silu_flag(activation))
+
+
 # ---- cross scan / merge ---------------------------------------------------------------------------
 def _make_cross_pair(dirs, suffix):
     dirs = tuple(dirs)

@@ -319,6 +319,101 @@ def state_update(state, x, dt, A, B, C, D=None, z=None, dt_bias=None, dt_softplu
     return out
 
 
+# ---- causal depthwise conv1d (causal-conv1d 1.1.x) ----------------------------------------------
+def _conv1d_checks(x, weight, bias, x_rank, tensors=()):
+    """The metadata checks of every conv1d call, then the device checks; returns weight and bias as contiguous fp32 (the C ABI
+    takes fp32 parameters whatever x's dtype)."""
+    _require(x.dtype in _DT, "x must be float32, float16 or bfloat16")
+    _require(weight.dtype in _DT, "weight must be float32, float16 or bfloat16")
+    _require(weight.dim() == 2 and 2 <= weight.shape[1] <= 4, "weight must be (dim, width) with 2 <= width <= 4")
+    _require(x.dim() == x_rank and x.shape[1] == weight.shape[0],
+             "x must be (batch, dim, seqlen)" if x_rank == 3 else "x must be (batch, dim)")
+    if bias is not None:
+        _require(bias.dtype == weight.dtype and tuple(bias.shape) == (weight.shape[0],), "bias must be (dim,) of weight's dtype")
+    if x_rank == 3:
+        _require(x.stride(2) == 1 or x.stride(1) != 1, "channel-last x (stride 1 along dim) is not supported")
+    for name, t in (("x", x), ("weight", weight), ("bias", bias)) + tuple(tensors):
+        if t is not None:
+            _require(t.is_cuda, f"Expected {name}.is_cuda() to be true")
+            _require(t.device == x.device, f"{name} must be on the device of x")
+    return weight.float().contiguous(), None if bias is None else bias.float().contiguous()
+
+
+def _conv1d_rows(x):
+    """x with stride 1 along seqlen (a stride other than channel-last's is copied away, as causal-conv1d does)."""
+    return x if x.stride(2) == 1 else x.contiguous()
+
+
+def _conv1d_desc(x, width, silu, out):
+    d = _lib.Conv1dDesc()
+    d.batch, d.dim = x.shape[0], x.shape[1]
+    d.seqlen = x.shape[2] if x.dim() == 3 else 1
+    d.width, d.io_dtype, d.silu = width, _DT[x.dtype], int(bool(silu))
+    d.x_batch_stride, d.x_dim_stride = x.stride(0), x.stride(1)
+    d.out_batch_stride, d.out_dim_stride = out.stride(0), out.stride(1)
+    return d
+
+
+def conv1d_fwd(x, weight, bias=None, silu=False) -> torch.Tensor:
+    """out = act(causal depthwise conv1d of x) (ss2d_conv1d_fwd). x (batch, dim, seqlen) fp32 / fp16 / bf16 with stride 1 along
+    seqlen (other batch / dim strides, such as a view of mamba's xz.chunk, are read in place); weight (dim, width), bias (dim) or
+    None, of one dtype. -> out (batch, dim, seqlen), dense, in x's dtype."""
+    w, b = _conv1d_checks(x, weight, bias, 3)
+    x = _conv1d_rows(x)
+    out = torch.empty(x.shape, dtype=x.dtype, device=x.device)
+    d = _conv1d_desc(x, w.shape[1], silu, out)
+    with torch.cuda.device(x.device):
+        rc = _lib.lib().ss2d_conv1d_fwd(ctypes.byref(d), _ptr(x), _ptr(w), _ptr(b), _ptr(out), _stream(x.device))
+    _lib.check(rc, "ss2d_conv1d_fwd")
+    return out
+
+
+def conv1d_bwd(x, weight, bias, dout, silu=False, dx=None):
+    """Gradients of conv1d_fwd (ss2d_conv1d_bwd) -> (dx, dweight, dbias). dx has x's dtype and is written into `dx` when given;
+    dweight / dbias are accumulated in fp32 and returned in weight's dtype; dbias is None without a bias. Bit-identical from call
+    to call."""
+    _require(tuple(dout.shape) == tuple(x.shape), "dout must have x's shape")
+    if dx is not None:
+        _require(tuple(dx.shape) == tuple(x.shape) and dx.dtype == x.dtype, "dx must have x's shape and dtype")
+    w, b = _conv1d_checks(x, weight, bias, 3, (("dout", dout), ("dx", dx)))
+    x = _conv1d_rows(x)
+    dout = dout.to(x.dtype).contiguous()
+    # dout and dx share one stride pair: dx is written in place when its strides are dout's, else through a dense buffer
+    buf = dx if dx is not None and dx.stride() == dout.stride() else torch.empty(x.shape, dtype=x.dtype, device=x.device)
+    dim, width = w.shape
+    dw = torch.empty((dim, width), dtype=torch.float32, device=x.device)
+    db = None if bias is None else torch.empty(dim, dtype=torch.float32, device=x.device)
+    d = _conv1d_desc(x, width, silu, buf)
+    L = _lib.lib()
+    ws_bytes = L.ss2d_conv1d_bwd_workspace_bytes(ctypes.byref(d))
+    ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=x.device) if ws_bytes else None
+    with torch.cuda.device(x.device):
+        rc = L.ss2d_conv1d_bwd(ctypes.byref(d), _ptr(x), _ptr(w), _ptr(b), _ptr(dout), _ptr(buf), _ptr(dw), _ptr(db), _ptr(ws),
+                               ws_bytes, _stream(x.device))
+    _lib.check(rc, "ss2d_conv1d_bwd")
+    if dx is not None and buf is not dx:
+        dx.copy_(buf)
+        buf = dx
+    return buf, dw.to(weight.dtype), None if db is None else db.to(bias.dtype)
+
+
+def conv1d_update(x, conv_state, weight, bias=None, silu=False) -> torch.Tensor:
+    """One decode position (ss2d_conv1d_update): conv_state (batch, dim, width), contiguous, of x's dtype, is shifted left by one
+    in place with x (batch, dim) in its last slot; -> out = act(bias + weight . conv_state), (batch, dim) in x's dtype."""
+    _require(x.dim() == 2, "x must be (batch, dim)")
+    _require(conv_state.dtype == x.dtype and tuple(conv_state.shape) == (x.shape[0], x.shape[1], weight.shape[-1]),
+             "conv_state must be (batch, dim, width) of x's dtype")
+    _require(conv_state.is_contiguous(), "conv_state must be contiguous (it is updated in place)")
+    w, b = _conv1d_checks(x, weight, bias, 2, (("conv_state", conv_state),))
+    out = torch.empty(x.shape, dtype=x.dtype, device=x.device)
+    d = _conv1d_desc(x, w.shape[1], silu, out)
+    with torch.cuda.device(x.device):
+        rc = _lib.lib().ss2d_conv1d_update(ctypes.byref(d), _ptr(x), _ptr(conv_state), _ptr(w), _ptr(b), _ptr(out),
+                                           _stream(x.device))
+    _lib.check(rc, "ss2d_conv1d_update")
+    return out
+
+
 # ---- stand-alone permutations ------------------------------------------------------------------
 def cross_scan(x: torch.Tensor, dirs: Sequence[int]) -> torch.Tensor:
     """x (B, C, H, W) -> (B, K, C, H*W), plane k traversed in direction dirs[k] (csms6s.py:11-206)."""

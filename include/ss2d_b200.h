@@ -208,6 +208,44 @@ int ss2d_state_update(const ss2d_step_desc* desc, float* state, const void* x, c
                       const void* Bmat, const void* Cmat, const float* Dvec, const float* dt_bias, const void* z,
                       void* out, ss2d_stream_t stream);
 
+/* ---- causal depthwise 1-D convolution of Mamba blocks (the contract of causal-conv1d 1.1.x, channel-first x) -----------
+ * x (batch, dim, seqlen) of io_dtype, element (b, d, l) at b * x_batch_stride + d * x_dim_stride + l. weight: fp32 (dim, width)
+ * contiguous, 2 <= width <= 4. bias: fp32 (dim) or NULL (zero). act: SiLU when silu == 1, else the identity. All math in fp32.
+ *   fwd:    out[b,d,l] = act(bias[d] + sum_{k<width} weight[d,k] x[b,d,l-(width-1)+k]), x = 0 at negative positions;
+ *           out is rounded once to io_dtype.
+ *   bwd:    g = dout act'(pre), pre recomputed from x; dx[b,d,l] = sum_k weight[d,k] g[b,d,l+(width-1)-k] (g = 0 past seqlen - 1);
+ *           dweight[d,k] = sum_{b,l} g[b,d,l] x[b,d,l-(width-1)+k] and dbias[d] = sum_{b,l} g[b,d,l], fp32, fully overwritten
+ *           (dbias NULL: not computed). No atomics: bit-identical from call to call. workspace:
+ *           ss2d_conv1d_bwd_workspace_bytes(desc) bytes (0 when one slab covers a channel: workspace may then be NULL).
+ *   update: one decode position, seqlen == 1. conv_state (batch, dim, width) of io_dtype, contiguous, is shifted left by one in
+ *           place and x[b,d] is stored in its last slot; then out[b,d] = act(bias[d] + sum_k weight[d,k] conv_state[b,d,k]).
+ *           x (batch, dim) at b * x_batch_stride + d * x_dim_stride.
+ * out / dout / dx share one stride pair: (b, d, l) at b * out_batch_stride + d * out_dim_stride + l; for update out (b, d) at
+ * b * out_batch_stride + d * out_dim_stride. Written rows must not overlap: out_dim_stride >= seqlen and
+ * out_batch_stride >= dim * out_dim_stride, else SS2D_ERR_BAD_LAYOUT, as is a negative x stride.
+ * Errors, returned before any launch: SS2D_ERR_NULL_POINTER (desc, x, weight, out / dout / dx / dweight / conv_state NULL),
+ * SS2D_ERR_BAD_SHAPE (a size <= 0, width outside 2..4, seqlen != 1 in update), SS2D_ERR_BAD_DTYPE (io_dtype, or silu not 0 / 1),
+ * SS2D_ERR_BAD_LAYOUT (strides, above), SS2D_ERR_ALIGNMENT (an io pointer not aligned to its element size, weight / bias /
+ * dweight / dbias / workspace not 4-byte aligned), SS2D_ERR_WORKSPACE (workspace NULL or smaller than required). */
+typedef struct ss2d_conv1d_desc {
+  int32_t batch;
+  int32_t dim;
+  int32_t seqlen;
+  int32_t width;
+  int32_t io_dtype;          /* ss2d_dtype of x, out, dout, dx, conv_state */
+  int32_t silu;              /* 1: SiLU activation, 0: none */
+  /* element strides */
+  int64_t x_batch_stride, x_dim_stride;
+  int64_t out_batch_stride, out_dim_stride;   /* out, dout, dx */
+} ss2d_conv1d_desc;
+int ss2d_conv1d_fwd(const ss2d_conv1d_desc* desc, const void* x, const float* weight, const float* bias, void* out,
+                    ss2d_stream_t stream);
+size_t ss2d_conv1d_bwd_workspace_bytes(const ss2d_conv1d_desc* desc);
+int ss2d_conv1d_bwd(const ss2d_conv1d_desc* desc, const void* x, const float* weight, const float* bias, const void* dout,
+                    void* dx, float* dweight, float* dbias, void* workspace, size_t workspace_bytes, ss2d_stream_t stream);
+int ss2d_conv1d_update(const ss2d_conv1d_desc* desc, const void* x, void* conv_state, const float* weight, const float* bias,
+                       void* out, ss2d_stream_t stream);
+
 /* ---- stand-alone cross-scan / cross-merge (exact permutations; model/gm/csms6s.py:11-206) ----
  * cross_scan : x (batch, channels, H, W) -> xs (batch, K, channels, L), xs[:,k] in direction dirs[k].
  * cross_merge: ys (batch, K, channels, L) in scan order -> y (batch, channels, L) natural order,
