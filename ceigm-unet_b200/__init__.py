@@ -5,7 +5,9 @@ Layers (SURVEY.md §8b):
       module, with the z gate) — the reference extension modules' `fwd` / `bwd` functions; `install_dropin()` registers them
       in sys.modules so that the reference's own `model/gm/csms6s.py` picks them up unchanged. dropin/causal_conv1d_cuda.py and
       dropin/causal_conv1d.py serve causal-conv1d 1.1.x, the convolution in front of every Mamba block's scan.
-  b2  functional.py — SelectiveScanCore/Oflex, CrossScan[_k], CrossMerge[_k] autograd Functions.
+  b2  functional.py — SelectiveScanCore/Oflex, CrossScan[_k], CrossMerge[_k] autograd Functions; the Mamba functions
+      selective_scan, selective_state_update, causal_conv1d_fn / _update, and mamba_chunk_scan_combined (Mamba-2's chunked
+      scan, mamba_ssm 2.x's arguments, differentiable).
   b3  modules.py — SS2D, GroupMambaLayer (and the FFNs next to them: PVT2FFN, custom_ffn) with the reference's state_dict.
 Underneath: ops.py -> _lib.py (ctypes) -> libss2d_b200.so (csrc/*.cu, C ABI in include/ss2d_b200.h).
 There is no CPU or PyTorch fallback: without the built library every operator raises RuntimeError.
@@ -14,7 +16,8 @@ from . import _lib, dist, functional, modules, ops                 # noqa: F401
 from ._lib import build, launch_count, version                    # noqa: F401
 from .functional import (CrossMerge, CrossMerge_1, CrossMerge_2, CrossMerge_3, CrossMerge_4, CrossScan,   # noqa: F401
                          CrossScan_1, CrossScan_2, CrossScan_3, CrossScan_4, SelectiveScanCore, SelectiveScanOflex,
-                         causal_conv1d_fn, causal_conv1d_update, selective_scan, selective_state_update)
+                         causal_conv1d_fn, causal_conv1d_update, mamba_chunk_scan_combined, selective_scan,
+                         selective_state_update)
 from .modules import SS2D, GroupMambaLayer, LayerNormRows, PVT2FFN, custom_ffn, mamba_init             # noqa: F401
 
 

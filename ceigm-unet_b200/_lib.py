@@ -24,6 +24,7 @@ EXPORTS = [
     "ss2d_scan_fwd_state", "ss2d_scan_bwd_state",
     "ss2d_scan_fwd_gated", "ss2d_scan_bwd_gated", "ss2d_scan_bwd_gated_workspace_bytes", "ss2d_state_update",
     "ss2d_conv1d_fwd", "ss2d_conv1d_bwd", "ss2d_conv1d_bwd_workspace_bytes", "ss2d_conv1d_update",
+    "ss2d_ssd_fwd", "ss2d_ssd_fwd_workspace_bytes", "ss2d_ssd_bwd", "ss2d_ssd_bwd_workspace_bytes",
     "ss2d_cross_scan", "ss2d_cross_merge", "ss2d_out_gate_fwd", "ss2d_out_gate_bwd",
     "ss2d_out_gate_bwd_partials", "ss2d_group_gate_fwd", "ss2d_group_gate_bwd", "ss2d_out_gate_max_width", "ss2d_wgrad_ts", "ss2d_wgrad_ts_workspace_bytes",
     "ss2d_layernorm_fwd", "ss2d_layernorm_bwd", "ss2d_layernorm_bwd_partials",
@@ -65,6 +66,17 @@ class Conv1dDesc(ctypes.Structure):
         ("io_dtype", ctypes.c_int32), ("silu", ctypes.c_int32),
         ("x_batch_stride", ctypes.c_int64), ("x_dim_stride", ctypes.c_int64),
         ("out_batch_stride", ctypes.c_int64), ("out_dim_stride", ctypes.c_int64),
+    ]
+
+
+class SsdDesc(ctypes.Structure):
+    """Mirror of `ss2d_ssd_desc` (include/ss2d_b200.h)."""
+    _fields_ = [
+        ("batch", ctypes.c_int32), ("seqlen", ctypes.c_int32), ("heads", ctypes.c_int32), ("headdim", ctypes.c_int32),
+        ("n_groups", ctypes.c_int32), ("dstate", ctypes.c_int32), ("chunk_size", ctypes.c_int32), ("io_dtype", ctypes.c_int32),
+        ("dt_softplus", ctypes.c_int32), ("d_mode", ctypes.c_int32), ("dt_min", ctypes.c_float), ("dt_max", ctypes.c_float),
+    ] + [(f"{t}_{s}_stride", ctypes.c_int64) for t in ("x", "z", "out", "dt") for s in ("batch", "seq", "head")] + [
+        ("bc_batch_stride", ctypes.c_int64), ("bc_seq_stride", ctypes.c_int64), ("bc_group_stride", ctypes.c_int64),
     ]
 
 
@@ -131,6 +143,15 @@ def lib() -> ctypes.CDLL:
     L.ss2d_conv1d_bwd.restype = ctypes.c_int
     L.ss2d_conv1d_update.argtypes = [cd, vp, vp, fp, fp, vp, vp]
     L.ss2d_conv1d_update.restype = ctypes.c_int
+    sd = ctypes.POINTER(SsdDesc)
+    L.ss2d_ssd_fwd_workspace_bytes.argtypes = [sd]
+    L.ss2d_ssd_fwd_workspace_bytes.restype = sz
+    L.ss2d_ssd_fwd.argtypes = [sd, vp, vp, fp, vp, vp, fp, fp, vp, fp, vp, fp, vp, sz, vp]
+    L.ss2d_ssd_fwd.restype = ctypes.c_int
+    L.ss2d_ssd_bwd_workspace_bytes.argtypes = [sd]
+    L.ss2d_ssd_bwd_workspace_bytes.restype = sz
+    L.ss2d_ssd_bwd.argtypes = [sd, vp, vp, fp, vp, vp, fp, fp, vp, fp, vp, fp, vp, vp, fp, vp, vp, fp, fp, vp, fp, vp, sz, vp]
+    L.ss2d_ssd_bwd.restype = ctypes.c_int
     ip = ctypes.POINTER(ctypes.c_int32)
     L.ss2d_cross_scan.argtypes = [vp, vp, i32, i32, i32, i32, i32, ip, i32, vp]
     L.ss2d_cross_scan.restype = ctypes.c_int

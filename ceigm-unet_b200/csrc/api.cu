@@ -11,6 +11,7 @@
 #include "conv1d_params.h"
 #include "scan_params.h"
 #include "ss2d_b200.h"
+#include "ssd_params.h"
 
 namespace ss2d {
 cudaError_t scan_fwd_dispatch(const ScanParams& p, const ScanState& st, cudaStream_t stream);
@@ -27,6 +28,9 @@ int conv1d_bwd_slabs(int batch, int dim, int64_t L);
 cudaError_t conv1d_fwd_launch(const Conv1dParams& p, int io_dtype, cudaStream_t stream);
 cudaError_t conv1d_bwd_launch(const Conv1dParams& p, int io_dtype, cudaStream_t stream);
 cudaError_t conv1d_update_launch(const Conv1dParams& p, int io_dtype, cudaStream_t stream);
+// Mamba-2 chunked scan (ssd.cu)
+cudaError_t ssd_fwd_launch(const SsdParams& p, int io_dtype, cudaStream_t stream);
+cudaError_t ssd_bwd_launch(const SsdParams& p, int io_dtype, cudaStream_t stream);
 constexpr int kDwnMaxSeg = 4;
 struct DwnSegs { int nseg; int cbeg[kDwnMaxSeg + 1]; int k[kDwnMaxSeg]; const float* w[kDwnMaxSeg]; const float* b[kDwnMaxSeg]; };
 cudaError_t dwnhwc_stencil_launch(const void* x, const void* aux, void* y, const DwnSegs& sg, int flip, int epi, int B, int H,
@@ -555,6 +559,158 @@ int ss2d_conv1d_update(const ss2d_conv1d_desc* d, const void* x, void* conv_stat
   const cudaError_t e = conv1d_update_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e);
   ++g_launches;
+  return SS2D_OK;
+}
+
+// true when rows of `inner` elements placed at the strides of the three (stride, extent) pairs never overlap
+static bool rows_disjoint(int64_t inner, int64_t s0, int64_t n0, int64_t s1, int64_t n1, int64_t s2, int64_t n2) {
+  int64_t st[3] = {s0, s1, s2}, ex[3] = {n0, n1, n2};
+  for (int i = 0; i < 3; ++i)
+    for (int j = i + 1; j < 3; ++j)
+      if (st[j] < st[i]) { std::swap(st[i], st[j]); std::swap(ex[i], ex[j]); }
+  int64_t span = inner;
+  for (int i = 0; i < 3; ++i) {
+    if (ex[i] <= 1) continue;
+    if (st[i] < span) return false;
+    span += st[i] * (ex[i] - 1);
+  }
+  return true;
+}
+
+static int ssd_validate(const ss2d_ssd_desc* d) {
+  if (!d) return SS2D_ERR_NULL_POINTER;
+  if (d->batch <= 0 || d->seqlen <= 0 || d->heads <= 0 || d->headdim <= 0 || d->n_groups <= 0 || d->dstate <= 0 ||
+      d->chunk_size <= 0 || d->batch > 65535 || d->heads > 65535 || d->heads % d->n_groups != 0 || !(d->dt_min <= d->dt_max))
+    return SS2D_ERR_BAD_SHAPE;
+  if (d->dstate % 16 != 0 || d->dstate > SS2D_MAX_DSTATE) return SS2D_ERR_DSTATE;
+  if ((d->headdim != 32 && d->headdim != 64 && d->headdim != 128) ||
+      (d->chunk_size != 64 && d->chunk_size != 128 && d->chunk_size != 256))
+    return SS2D_ERR_UNSUPPORTED;
+  if (!dtype_ok(d->io_dtype) || (d->dt_softplus != 0 && d->dt_softplus != 1) || d->d_mode < 0 || d->d_mode > 2)
+    return SS2D_ERR_BAD_DTYPE;
+  const int64_t strides[] = {d->x_batch_stride, d->x_seq_stride, d->x_head_stride, d->z_batch_stride, d->z_seq_stride,
+                             d->z_head_stride, d->out_batch_stride, d->out_seq_stride, d->out_head_stride,
+                             d->dt_batch_stride, d->dt_seq_stride, d->dt_head_stride, d->bc_batch_stride, d->bc_seq_stride,
+                             d->bc_group_stride};
+  for (int64_t s : strides)
+    if (s < 0) return SS2D_ERR_BAD_LAYOUT;
+  if (!rows_disjoint(d->headdim, d->out_batch_stride, d->batch, d->out_seq_stride, d->seqlen, d->out_head_stride, d->heads))
+    return SS2D_ERR_BAD_LAYOUT;
+  return SS2D_OK;
+}
+
+static int64_t ssd_chunks(const ss2d_ssd_desc* d) { return ((int64_t)d->seqlen + d->chunk_size - 1) / d->chunk_size; }
+
+size_t ss2d_ssd_fwd_workspace_bytes(const ss2d_ssd_desc* d) {
+  if (ssd_validate(d) != SS2D_OK) return 0;
+  const int64_t bhc = (int64_t)d->batch * d->heads * ssd_chunks(d);
+  return sizeof(float) * (size_t)bhc * (2 * (size_t)d->chunk_size + (size_t)d->headdim * d->dstate);
+}
+
+static int ssd_inputs_check(const ss2d_ssd_desc* d, const void* x, const void* dt, const float* A, const void* Bmat,
+                            const void* Cmat, const float* D, const float* dt_bias, const void* z, const float* h0, const void* out,
+                            const float* hT, const void* workspace) {
+  if (!x || !dt || !A || !Bmat || !Cmat || !out || (d->d_mode != 0 && !D)) return SS2D_ERR_NULL_POINTER;
+  const size_t es = esize(d->io_dtype);
+  if (!aligned(x, es) || !aligned(dt, es) || !aligned(Bmat, es) || !aligned(Cmat, es) || !aligned(z, es) ||
+      !aligned(out, es) || !aligned(A, 4) || !aligned(D, 4) || !aligned(dt_bias, 4) || !aligned(h0, 4) || !aligned(hT, 4) ||
+      !aligned(workspace, 4))
+    return SS2D_ERR_ALIGNMENT;
+  return SS2D_OK;
+}
+
+static SsdParams ssd_params(const ss2d_ssd_desc* d, const void* x, const void* dt, const float* A, const void* Bmat,
+                            const void* Cmat, const float* D, const float* dt_bias, const void* z, const float* h0,
+                            void* workspace) {
+  SsdParams p = {};
+  p.x = x; p.dt = dt; p.B = Bmat; p.C = Cmat; p.z = z; p.A = A; p.D = d->d_mode ? D : nullptr; p.dt_bias = dt_bias;
+  p.h0 = h0;
+  p.batch = d->batch; p.heads = d->heads; p.groups = d->n_groups; p.P = d->headdim; p.N = d->dstate; p.Q = d->chunk_size;
+  p.nchunks = (int)ssd_chunks(d); p.L = d->seqlen; p.d_mode = d->d_mode; p.softplus = d->dt_softplus;
+  p.dt_min = d->dt_min; p.dt_max = d->dt_max;
+  p.x_b = d->x_batch_stride; p.x_l = d->x_seq_stride; p.x_h = d->x_head_stride;
+  p.z_b = d->z_batch_stride; p.z_l = d->z_seq_stride; p.z_h = d->z_head_stride;
+  p.o_b = d->out_batch_stride; p.o_l = d->out_seq_stride; p.o_h = d->out_head_stride;
+  p.dt_b = d->dt_batch_stride; p.dt_l = d->dt_seq_stride; p.dt_h = d->dt_head_stride;
+  p.bc_b = d->bc_batch_stride; p.bc_l = d->bc_seq_stride; p.bc_g = d->bc_group_stride;
+  p.npass = (int)(((int64_t)p.P * p.N + 255) / 256);
+  const int64_t bhq = (int64_t)d->batch * d->heads * p.nchunks * d->chunk_size;
+  p.t = static_cast<float*>(workspace);
+  p.cum = p.t + bhq;
+  p.states = p.cum + bhq;
+  return p;
+}
+
+int ss2d_ssd_fwd(const ss2d_ssd_desc* d, const void* x, const void* dt, const float* A, const void* Bmat, const void* Cmat,
+                 const float* D, const float* dt_bias, const void* z, const float* h0, void* out, float* hT, void* workspace,
+                 size_t workspace_bytes, ss2d_stream_t stream) {
+  const int v = ssd_validate(d);
+  if (v != SS2D_OK) return v;
+  const int c = ssd_inputs_check(d, x, dt, A, Bmat, Cmat, D, dt_bias, z, h0, out, hT, workspace);
+  if (c != SS2D_OK) return c;
+  const size_t need = ss2d_ssd_fwd_workspace_bytes(d);
+  if (!workspace || workspace_bytes < need) return SS2D_ERR_WORKSPACE;
+  SsdParams p = ssd_params(d, x, dt, A, Bmat, Cmat, D, dt_bias, z, h0, workspace);
+  p.out = out; p.hT = hT;
+  const cudaError_t e = ssd_fwd_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  g_launches += 3;
+  return SS2D_OK;
+}
+
+// backward workspace, in floats after the forward's: hfin, R (like the states), dotp, dcum1, ddtd, ddts, colM, dBh, dCh, partD,
+// partA, partBias
+static size_t ssd_bwd_extra_floats(const ss2d_ssd_desc* d) {
+  const size_t bh = (size_t)d->batch * d->heads, nc = (size_t)ssd_chunks(d), Q = d->chunk_size, PN = (size_t)d->headdim * d->dstate;
+  const size_t npass = (PN + 255) / 256, nblk = nc * (Q / 64);
+  return bh * PN + bh * nc * PN + bh * nc * npass + 3 * bh * nc * Q + bh * nc * (Q / 64) * (Q / 64) * 64 +
+         2 * bh * nc * Q * d->dstate +
+         (size_t)d->batch * nblk * d->heads * d->headdim + 2 * bh * nc;
+}
+
+size_t ss2d_ssd_bwd_workspace_bytes(const ss2d_ssd_desc* d) {
+  if (ssd_validate(d) != SS2D_OK) return 0;
+  return ss2d_ssd_fwd_workspace_bytes(d) + sizeof(float) * ssd_bwd_extra_floats(d);
+}
+
+int ss2d_ssd_bwd(const ss2d_ssd_desc* d, const void* x, const void* dt, const float* A, const void* Bmat, const void* Cmat,
+                 const float* D, const float* dt_bias, const void* z, const float* h0, const void* dout, const float* dhT,
+                 void* dx, void* ddt, float* dA, void* dB, void* dC, float* dD, float* ddt_bias, void* dz, float* dh0,
+                 void* workspace, size_t workspace_bytes, ss2d_stream_t stream) {
+  const int v = ssd_validate(d);
+  if (v != SS2D_OK) return v;
+  const int c = ssd_inputs_check(d, x, dt, A, Bmat, Cmat, D, dt_bias, z, h0, dout, dhT, workspace);
+  if (c != SS2D_OK) return c;
+  if (!dx || !ddt || !dA || !dB || !dC || (d->d_mode != 0 && !dD)) return SS2D_ERR_NULL_POINTER;
+  const size_t es = esize(d->io_dtype);
+  if (!aligned(dx, es) || !aligned(ddt, es) || !aligned(dB, es) || !aligned(dC, es) || !aligned(dz, es) || !aligned(dA, 4) ||
+      !aligned(dD, 4) || !aligned(ddt_bias, 4) || !aligned(dh0, 4))
+    return SS2D_ERR_ALIGNMENT;
+  const size_t need = ss2d_ssd_bwd_workspace_bytes(d);
+  if (!workspace || workspace_bytes < need) return SS2D_ERR_WORKSPACE;
+  SsdParams p = ssd_params(d, x, dt, A, Bmat, Cmat, D, dt_bias, z, h0, workspace);
+  p.dout = dout; p.dhT = dhT; p.dx = dx; p.ddt = ddt; p.dA = dA; p.dB = dB; p.dC = dC; p.dD = d->d_mode ? dD : nullptr;
+  p.ddt_bias = dt_bias ? ddt_bias : nullptr; p.dh0 = dh0;
+  // without z there is no dz; with z a scratch dz is not needed: dz NULL keeps z out of the output (dy still gated)
+  p.dz = z ? dz : nullptr;
+  const size_t bh = (size_t)d->batch * d->heads, nc = (size_t)p.nchunks, Q = d->chunk_size, PN = (size_t)d->headdim * d->dstate;
+  float* w = static_cast<float*>(workspace) + ss2d_ssd_fwd_workspace_bytes(d) / sizeof(float);
+  p.hfin = w; w += bh * PN;
+  p.R = w; w += bh * nc * PN;
+  p.dotp = w; w += bh * nc * p.npass;
+  p.dcum1 = w; w += bh * nc * Q;
+  p.ddtd = w; w += bh * nc * Q;
+  p.ddts = w; w += bh * nc * Q;
+  p.colM = w; w += bh * nc * (Q / 64) * (Q / 64) * 64;
+  p.dBh = w; w += bh * nc * Q * d->dstate;
+  p.dCh = w; w += bh * nc * Q * d->dstate;
+  p.partD = w; w += (size_t)d->batch * nc * (Q / 64) * d->heads * d->headdim;
+  p.partA = w; w += bh * nc;
+  p.partBias = w;
+  p.hT = p.hfin;
+  const cudaError_t e = ssd_bwd_launch(p, d->io_dtype, static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e);
+  g_launches += 9;
   return SS2D_OK;
 }
 

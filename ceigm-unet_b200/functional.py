@@ -171,6 +171,54 @@ def causal_conv1d_update(x, conv_state, weight, bias=None, activation=None):
     return ops.conv1d_update(x, conv_state, weight, bias, _silu_flag(activation))
 
 
+# ---- Mamba-2 chunked selective scan (the mamba_ssm 2.x interface) -----------------------------------
+class _ChunkScan(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, dt, A, B, C, D, z, dt_bias, initial_states, chunk_size, dt_softplus, dt_limit):
+        ops_in = ops.ssd_prepare(x, dt, A, B, C, chunk_size, D, z, dt_bias, initial_states, dt_limit)
+        out, final = ops.ssd_fwd(*ops_in[:5], chunk_size, *ops_in[5:], dt_softplus, dt_limit, True)
+        ctx.save_for_backward(*ops_in)      # the inputs only: the backward recomputes the chunk states
+        ctx.cfg = (chunk_size, dt_softplus, dt_limit)
+        ctx.dtypes = tuple(None if t is None else t.dtype for t in (dt, A, D, dt_bias))
+        return out, final
+
+    @staticmethod
+    def backward(ctx, dout, dfinal):
+        x, dt, A, B, C, D, z, dt_bias, h0 = ctx.saved_tensors
+        chunk_size, dt_softplus, dt_limit = ctx.cfg
+        if dout is None:
+            dout = torch.zeros_like(x)
+        dx, ddt, dA, dB, dC, dD, dz, ddt_bias, dh0 = ops.ssd_bwd(x, dt, A, B, C, chunk_size, D, z, dt_bias, h0, dt_softplus,
+                                                                 dt_limit, dout, dfinal)
+        dt_t, A_t, D_t, bias_t = ctx.dtypes
+        cast = lambda g, t: None if g is None else g.to(t)   # noqa: E731
+        return (dx, cast(ddt, dt_t), cast(dA, A_t), dB, dC, cast(dD, D_t), dz, cast(ddt_bias, bias_t), dh0, None, None, None)
+
+
+def mamba_chunk_scan_combined(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bias=None, initial_states=None, seq_idx=None,
+                              cu_seqlens=None, dt_softplus=False, dt_limit=(0.0, float("inf")), return_final_states=False,
+                              return_varlen_states=False):
+    """Mamba-2's scan (SSD) with mamba_ssm's arguments, computed in chunks of chunk_size positions on the tensor cores:
+
+        t_l = clamp(softplus?(dt_l + dt_bias), dt_limit),  H_l = exp(t_l A) H_{l-1} + t_l x_l (x) B_l,  H_{-1} = initial_states,
+        y_l = C_l . H_l + D x_l,  out_l = y_l * silu(z_l) (with z).
+
+    x, z (batch, seqlen, heads, headdim), dt (batch, seqlen, heads), A (heads), B, C (batch, seqlen, n_groups, dstate), D (heads)
+    or (heads, headdim), dt_bias (heads), initial_states (batch, heads, headdim, dstate). x, z, B and C share one dtype (fp32 /
+    fp16 / bf16); math in fp32; out has x's dtype. headdim in {32, 64, 128}, dstate a multiple of 16 up to 256, chunk_size in
+    {64, 128, 256}. The default dt_limit (0, inf) does not clamp, as in mamba_ssm. Returns out, or (out, final_states) with
+    final_states = H_{seqlen-1} fp32 (batch, heads, headdim, dstate): the (batch, heads * headdim, dstate) state that
+    selective_scan(..., initial_state=) and selective_state_update take.
+    Differentiable in x, dt, A, B, C, D, z, dt_bias and initial_states, and through final_states; the gradients are
+    bit-identical from call to call, and autograd keeps only the inputs. seq_idx, cu_seqlens and return_varlen_states are not
+    supported (RuntimeError)."""
+    if seq_idx is not None or cu_seqlens is not None or return_varlen_states:
+        raise RuntimeError("mamba_chunk_scan_combined: seq_idx, cu_seqlens and return_varlen_states are not supported")
+    out, final = _ChunkScan.apply(x, dt, A, B, C, D, z, dt_bias, initial_states, chunk_size, bool(dt_softplus),
+                                  tuple(dt_limit))
+    return (out, final) if return_final_states else out
+
+
 # ---- cross scan / merge ---------------------------------------------------------------------------
 def _make_cross_pair(dirs, suffix):
     dirs = tuple(dirs)

@@ -414,6 +414,122 @@ def conv1d_update(x, conv_state, weight, bias=None, silu=False) -> torch.Tensor:
     return out
 
 
+# ---- Mamba-2 chunked selective scan (mamba_ssm 2.x's mamba_chunk_scan_combined) ------------------------
+SSD_HEADDIMS = (32, 64, 128)
+SSD_CHUNKS = (64, 128, 256)
+
+
+def ssd_prepare(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bias=None, initial_states=None, dt_limit=(0.0, float("inf"))):
+    """The checks of every chunked-scan call, then the operands as the C ABI takes them: x, z, B, C with stride 1 along their
+    last axis (copied when not), B and C with one stride set, dt in x's dtype, A, D, dt_bias and initial_states as contiguous
+    fp32. Returns (x, dt, A, B, C, D, z, dt_bias, initial_states)."""
+    _require(x.dtype in _DT, "x must be float32, float16 or bfloat16")
+    _require(x.dim() == 4, "x must be (batch, seqlen, heads, headdim)")
+    b, L, h, P = x.shape
+    _require(B.dim() == 4 and tuple(B.shape[:2]) == (b, L), "B must be (batch, seqlen, n_groups, dstate)")
+    _require(tuple(C.shape) == tuple(B.shape), "C must have B's shape")
+    g, N = B.shape[2], B.shape[3]
+    _require(g > 0 and h % g == 0, "heads must be a multiple of n_groups")
+    _require(tuple(dt.shape) == (b, L, h), "dt must be (batch, seqlen, heads)")
+    _require(tuple(A.shape) == (h,), "A must be (heads,)")
+    _require(B.dtype == x.dtype and C.dtype == x.dtype, "B and C must have x's dtype")
+    if z is not None:
+        _require(tuple(z.shape) == tuple(x.shape) and z.dtype == x.dtype, "z must have x's shape and dtype")
+    if D is not None:
+        _require(tuple(D.shape) in ((h,), (h, P)), "D must be (heads,) or (heads, headdim)")
+    if dt_bias is not None:
+        _require(tuple(dt_bias.shape) == (h,), "dt_bias must be (heads,)")
+    if initial_states is not None:
+        _require(tuple(initial_states.shape) == (b, h, P, N), "initial_states must be (batch, heads, headdim, dstate)")
+    _require(chunk_size in SSD_CHUNKS, f"chunk_size must be one of {SSD_CHUNKS}")
+    _require(P in SSD_HEADDIMS, f"headdim must be one of {SSD_HEADDIMS}")
+    _require(N % 16 == 0 and 0 < N <= _lib.MAX_DSTATE, "dstate must be a multiple of 16 up to 256")
+    _require(len(dt_limit) == 2 and dt_limit[0] <= dt_limit[1], "dt_limit must be (min, max) with min <= max")
+    for name, t in (("x", x), ("dt", dt), ("A", A), ("B", B), ("C", C), ("D", D), ("z", z), ("dt_bias", dt_bias),
+                    ("initial_states", initial_states)):
+        if t is not None:
+            _require(t.is_cuda, f"Expected {name}.is_cuda() to be true")
+            _require(t.device == x.device, f"{name} must be on the device of x")
+    last1 = lambda t: t if t is None or t.stride(-1) == 1 or t.shape[-1] == 1 else t.contiguous()   # noqa: E731
+    x, z, B, C = last1(x), last1(z), last1(B), last1(C)
+    if B.stride() != C.stride():
+        B, C = B.contiguous(), C.contiguous()
+    f32 = lambda t: None if t is None else t.detach().float().contiguous()   # noqa: E731
+    return (x.detach(), dt.detach().to(x.dtype), f32(A), B.detach(), C.detach(), f32(D), None if z is None else z.detach(),
+            f32(dt_bias), f32(initial_states))
+
+
+def _ssd_desc(x, dt, B, D, z, out, chunk_size, dt_softplus, dt_limit):
+    b, L, h, P = x.shape
+    d = _lib.SsdDesc()
+    d.batch, d.seqlen, d.heads, d.headdim, d.n_groups, d.dstate = b, L, h, P, B.shape[2], B.shape[3]
+    d.chunk_size, d.io_dtype, d.dt_softplus = chunk_size, _DT[x.dtype], int(bool(dt_softplus))
+    d.d_mode = 0 if D is None else (1 if D.dim() == 1 else 2)
+    # mamba_ssm clamps only when dt_limit is not its default (0, inf): a default limit leaves a negative t unclamped
+    lo, hi = (-float("inf"), float("inf")) if tuple(dt_limit) == (0.0, float("inf")) else dt_limit
+    d.dt_min, d.dt_max = float(lo), float(hi)
+    d.x_batch_stride, d.x_seq_stride, d.x_head_stride = x.stride(0), x.stride(1), x.stride(2)
+    if z is not None:
+        d.z_batch_stride, d.z_seq_stride, d.z_head_stride = z.stride(0), z.stride(1), z.stride(2)
+    d.out_batch_stride, d.out_seq_stride, d.out_head_stride = out.stride(0), out.stride(1), out.stride(2)
+    d.dt_batch_stride, d.dt_seq_stride, d.dt_head_stride = dt.stride(0), dt.stride(1), dt.stride(2)
+    d.bc_batch_stride, d.bc_seq_stride, d.bc_group_stride = B.stride(0), B.stride(1), B.stride(2)
+    return d
+
+
+def ssd_fwd(x, dt, A, B, C, chunk_size, D=None, z=None, dt_bias=None, initial_states=None, dt_softplus=False,
+            dt_limit=(0.0, float("inf")), return_final_states=False):
+    """Mamba-2's chunked scan, forward (ss2d_ssd_fwd). x (batch, seqlen, heads, headdim) and z (like x, or None), B and C
+    (batch, seqlen, n_groups, dstate), all of one dtype (fp32 / fp16 / bf16); dt (batch, seqlen, heads) is cast to it; A (heads),
+    D (heads) / (heads, headdim) / None and dt_bias (heads) / None are cast to fp32; initial_states (batch, heads, headdim,
+    dstate) / None is cast to fp32. Strides other than the last are read in place (column slices of a projection output); a
+    last stride other than 1 is copied away. -> (out in x's dtype, dense; final_states fp32 (batch, heads, headdim, dstate) or
+    None)."""
+    x, dt, A, B, C, D, z, dt_bias, h0 = ssd_prepare(x, dt, A, B, C, chunk_size, D, z, dt_bias, initial_states, dt_limit)
+    b, L, h, P = x.shape
+    out = torch.empty(x.shape, dtype=x.dtype, device=x.device)
+    hT = torch.empty((b, h, P, B.shape[3]), dtype=torch.float32, device=x.device) if return_final_states else None
+    d = _ssd_desc(x, dt, B, D, z, out, chunk_size, dt_softplus, dt_limit)
+    lib = _lib.lib()
+    ws_bytes = lib.ss2d_ssd_fwd_workspace_bytes(ctypes.byref(d))
+    ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        rc = lib.ss2d_ssd_fwd(ctypes.byref(d), _ptr(x), _ptr(dt), _ptr(A), _ptr(B), _ptr(C), _ptr(D), _ptr(dt_bias), _ptr(z),
+                              _ptr(h0), _ptr(out), _ptr(hT), _ptr(ws), ws_bytes, _stream(x.device))
+    _lib.check(rc, "ss2d_ssd_fwd")
+    return out, hT
+
+
+def ssd_bwd(x, dt, A, B, C, chunk_size, D, z, dt_bias, initial_states, dt_softplus, dt_limit, dout, dfinal=None):
+    """Gradients of ssd_fwd (ss2d_ssd_bwd), with the operands as ssd_prepare returns them, dout (like x) and dfinal (the
+    gradient of final_states, or None). -> (dx, ddt, dA, dB, dC, dD, dz, ddt_bias, dinitial_states): dx, dz, dB, dC and ddt in
+    x's dtype, dense; dA, dD, ddt_bias and dinitial_states fp32; None for the absent inputs. Bit-identical from call to call."""
+    b, L, h, P = x.shape
+    g, N = B.shape[2], B.shape[3]
+    dout = dout.to(x.dtype).contiguous()
+    dhT = None if dfinal is None else dfinal.float().contiguous()
+    dev = x.device
+    dx = torch.empty(x.shape, dtype=x.dtype, device=dev)
+    dz = None if z is None else torch.empty(x.shape, dtype=x.dtype, device=dev)
+    ddt = torch.empty((b, L, h), dtype=x.dtype, device=dev)
+    dB = torch.empty((b, L, g, N), dtype=x.dtype, device=dev)
+    dC = torch.empty((b, L, g, N), dtype=x.dtype, device=dev)
+    dA = torch.empty(h, dtype=torch.float32, device=dev)
+    dD = None if D is None else torch.empty(D.shape, dtype=torch.float32, device=dev)
+    ddt_bias = None if dt_bias is None else torch.empty(h, dtype=torch.float32, device=dev)
+    dh0 = None if initial_states is None else torch.empty((b, h, P, N), dtype=torch.float32, device=dev)
+    d = _ssd_desc(x, dt, B, D, z, dout, chunk_size, dt_softplus, dt_limit)
+    lib = _lib.lib()
+    ws_bytes = lib.ss2d_ssd_bwd_workspace_bytes(ctypes.byref(d))
+    ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.ss2d_ssd_bwd(ctypes.byref(d), _ptr(x), _ptr(dt), _ptr(A), _ptr(B), _ptr(C), _ptr(D), _ptr(dt_bias), _ptr(z),
+                              _ptr(initial_states), _ptr(dout), _ptr(dhT), _ptr(dx), _ptr(ddt), _ptr(dA), _ptr(dB), _ptr(dC),
+                              _ptr(dD), _ptr(ddt_bias), _ptr(dz), _ptr(dh0), _ptr(ws), ws_bytes, _stream(dev))
+    _lib.check(rc, "ss2d_ssd_bwd")
+    return dx, ddt, dA, dB, dC, dD, dz, ddt_bias, dh0
+
+
 # ---- stand-alone permutations ------------------------------------------------------------------
 def cross_scan(x: torch.Tensor, dirs: Sequence[int]) -> torch.Tensor:
     """x (B, C, H, W) -> (B, K, C, H*W), plane k traversed in direction dirs[k] (csms6s.py:11-206)."""

@@ -246,6 +246,66 @@ int ss2d_conv1d_bwd(const ss2d_conv1d_desc* desc, const void* x, const float* we
 int ss2d_conv1d_update(const ss2d_conv1d_desc* desc, const void* x, void* conv_state, const float* weight, const float* bias,
                        void* out, ss2d_stream_t stream);
 
+/* ---- Mamba-2 chunked selective scan, SSD (the contract of mamba_ssm 2.x's mamba_chunk_scan_combined), forward ----------------
+ * x (batch, seqlen, heads, headdim) and z (like x, or NULL), dt (batch, seqlen, heads), B and C (batch, seqlen, n_groups,
+ * dstate), all of io_dtype; A (heads) fp32; D fp32: NULL (d_mode 0), (heads) (d_mode 1) or (heads, headdim) contiguous
+ * (d_mode 2); dt_bias (heads) fp32 or NULL. Head k reads group k / (heads / n_groups). All math in fp32:
+ *   t_l = min(max(softplus?(dt_l + dt_bias_k), dt_min), dt_max)   (softplus when dt_softplus == 1, threshold 20),
+ *   H_l = exp(t_l A_k) H_{l-1} + t_l x_l (x) B_l   (headdim x dstate per (b, k)),   H_{-1} = h0 (zeros when NULL),
+ *   y_l = C_l . H_l + D x_l,   out_l = y_l silu(z_l) with z, else y_l; out is rounded once to io_dtype.
+ * hT, when not NULL, receives H_{seqlen-1}. h0 and hT are fp32 (batch, heads, headdim, dstate) contiguous: the (batch, dim,
+ * dstate) state of ss2d_scan_fwd_state / ss2d_state_update with dim = heads * headdim.
+ * Element (b, l, k, p) of x is at b * x_batch_stride + l * x_seq_stride + k * x_head_stride + p (z, out alike with their
+ * strides); dt (b, l, k) at b * dt_batch_stride + l * dt_seq_stride + k * dt_head_stride; B, C (b, l, g, n) at
+ * b * bc_batch_stride + l * bc_seq_stride + g * bc_group_stride + n. Strides are free and non-negative (a column slice of a
+ * projection output is read in place); out's rows of headdim elements must not overlap.
+ * The scan runs in chunks of chunk_size positions whose products run on the tensor cores (16-bit I/O: operands in io_dtype,
+ * fp32 accumulation; fp32 I/O: 3xTF32). No atomics: bit-identical from call to call. Three launches.
+ * workspace: ss2d_ssd_fwd_workspace_bytes(desc) bytes (4-byte aligned).
+ * Errors, returned before any launch: SS2D_ERR_NULL_POINTER (desc, x, dt, A, B, C or out NULL; D NULL with d_mode != 0),
+ * SS2D_ERR_BAD_SHAPE (a size <= 0, batch or heads > 65535, heads % n_groups != 0, dt_min > dt_max or NaN),
+ * SS2D_ERR_DSTATE (dstate not a multiple of 16 or > 256), SS2D_ERR_UNSUPPORTED (headdim not 32 / 64 / 128, chunk_size not
+ * 64 / 128 / 256), SS2D_ERR_BAD_DTYPE (io_dtype, dt_softplus not 0 / 1, d_mode not 0 / 1 / 2), SS2D_ERR_BAD_LAYOUT (a negative
+ * stride, overlapping out rows), SS2D_ERR_ALIGNMENT (an io pointer not aligned to its element size, an fp32 pointer or the
+ * workspace not 4-byte aligned), SS2D_ERR_WORKSPACE (workspace NULL or smaller than required). */
+typedef struct ss2d_ssd_desc {
+  int32_t batch;
+  int32_t seqlen;
+  int32_t heads;
+  int32_t headdim;
+  int32_t n_groups;
+  int32_t dstate;
+  int32_t chunk_size;
+  int32_t io_dtype;          /* ss2d_dtype of x, dt, B, C, z, out */
+  int32_t dt_softplus;       /* 1: softplus(dt + dt_bias), 0: dt + dt_bias */
+  int32_t d_mode;            /* 0: no D, 1: D (heads), 2: D (heads, headdim) */
+  float dt_min, dt_max;      /* clamp of t; -inf / inf for none */
+  /* element strides */
+  int64_t x_batch_stride, x_seq_stride, x_head_stride;
+  int64_t z_batch_stride, z_seq_stride, z_head_stride;
+  int64_t out_batch_stride, out_seq_stride, out_head_stride;
+  int64_t dt_batch_stride, dt_seq_stride, dt_head_stride;
+  int64_t bc_batch_stride, bc_seq_stride, bc_group_stride;   /* B and C */
+} ss2d_ssd_desc;
+size_t ss2d_ssd_fwd_workspace_bytes(const ss2d_ssd_desc* desc);
+int ss2d_ssd_fwd(const ss2d_ssd_desc* desc, const void* x, const void* dt, const float* A, const void* Bmat, const void* Cmat,
+                 const float* D, const float* dt_bias, const void* z, const float* h0, void* out, float* hT, void* workspace,
+                 size_t workspace_bytes, ss2d_stream_t stream);
+/* Backward of ss2d_ssd_fwd, with the same descriptor and inputs. dout (and dx, dz) use the out strides; dhT (the gradient of
+ * hT, fp32 (batch, heads, headdim, dstate) contiguous) or NULL (zero). Outputs, all fully overwritten: dx, dz (like dout, of
+ * io_dtype; dz only with z, and may then be NULL when not wanted), ddt dense (batch, seqlen, heads) of io_dtype, dB and dC
+ * dense (batch, seqlen, n_groups, dstate) of io_dtype, dA (heads) fp32, dD (heads) or (heads, headdim) fp32 by d_mode (NULL
+ * with d_mode 0), ddt_bias (heads) fp32 or NULL, dh0 like h0 or NULL. The chunk states are recomputed, not saved; the state
+ * adjoint runs backwards over the chunks, the chunk-local products run on the tensor cores, and every sum over heads,
+ * positions or batch goes through per-block partials added in a fixed order: no atomics, bit-identical from call to call.
+ * Nine launches. workspace: ss2d_ssd_bwd_workspace_bytes(desc) bytes. Errors as for ss2d_ssd_fwd, plus SS2D_ERR_NULL_POINTER
+ * for dout, dx, ddt, dA, dB or dC NULL, or dD NULL with d_mode != 0. */
+size_t ss2d_ssd_bwd_workspace_bytes(const ss2d_ssd_desc* desc);
+int ss2d_ssd_bwd(const ss2d_ssd_desc* desc, const void* x, const void* dt, const float* A, const void* Bmat, const void* Cmat,
+                 const float* D, const float* dt_bias, const void* z, const float* h0, const void* dout, const float* dhT,
+                 void* dx, void* ddt, float* dA, void* dB, void* dC, float* dD, float* ddt_bias, void* dz, float* dh0,
+                 void* workspace, size_t workspace_bytes, ss2d_stream_t stream);
+
 /* ---- stand-alone cross-scan / cross-merge (exact permutations; model/gm/csms6s.py:11-206) ----
  * cross_scan : x (batch, channels, H, W) -> xs (batch, K, channels, L), xs[:,k] in direction dirs[k].
  * cross_merge: ys (batch, K, channels, L) in scan order -> y (batch, channels, L) natural order,
